@@ -65,7 +65,13 @@ def parse_args():
     ap.add_argument("--envs", type=int, default=TOTAL_ENVS)
     ap.add_argument("--envs-per-gpu", type=int, default=ENVS_PER_GPU)
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary kernel measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/play_stats.npy (float64): the reduced statistics "
+                         "block of g2048_play (include/g2048.h), so that two builds can be compared on the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ helpers
@@ -292,7 +298,7 @@ def main():
         """warmup + steps batches; per step: key chain (prefetched on a side stream one batch ahead) + persistent play
         kernel + statistics reduction, device-timed with CUDA events (L2 flushed before each step).  Returns
         (seconds of the timed steps (max over ranks), reduced statistics of the timed steps, launches, seconds inside
-        the play kernel)."""
+        the play kernel, the last timed step's reduced statistics block as the device tensor it returned)."""
         # the inputs of a step (one 8-byte chain key per batch) are resident in HBM before the timed region
         step_keys = [E.words_tensor(list(E.key_words(SEED + i)), dev) for i in range(warmup + steps)]
         side = torch.cuda.Stream(device=dev)
@@ -349,15 +355,21 @@ def main():
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         kernel_s = sum(a.elapsed_time(b) for a, b in kernel_events) * 1e-3
-        return float(t.item()), [E.play_stats_dict(s) for s in stats_all], launches["n"], kernel_s
+        return float(t.item()), [E.play_stats_dict(s) for s in stats_all], launches["n"], kernel_s, stats_all[-1]
 
     # ---- the timed region -----------------------------------------------------------------------------------------
     batch_global, lo, n = batch_shape(args, world, rank)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    elapsed, summaries, gpu_launches, kernel_s = timed_play_loop(batch_global, lo, n, args.warmup, args.steps, sampler)
+    elapsed, summaries, gpu_launches, kernel_s, last_stats = timed_play_loop(batch_global, lo, n, args.warmup, args.steps, sampler)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # the block is reduced over the ranks: every rank holds the same one
+        words = last_stats.cpu().numpy().view(np.uint64)
+        assert int(words.max()) < (1 << 53), "a statistics word does not fit a float64 exactly"
+        dump_dir = Path(args.dump_outputs)
+        dump_dir.mkdir(parents=True, exist_ok=True)
+        np.save(dump_dir / "play_stats.npy", words.astype(np.float64))
     total_env_steps = sum(s["env_steps"] for s in summaries)  # after the reduction: whole-job totals
     assert all(s["episodes"] == batch_global and s["cut_short"] == 0 and s["overflowed"] == 0 for s in summaries), summaries[0]
     value = total_env_steps / elapsed
@@ -497,7 +509,7 @@ def main():
     if not args.no_extras and args.scaling == "strong":
         w_global, w_lo2, w_n = ENVS_PER_GPU * world, ENVS_PER_GPU * rank, ENVS_PER_GPU
         w_steps = min(args.steps, 10)
-        w_elapsed, w_sum, _, w_kernel = timed_play_loop(w_global, w_lo2, w_n, 3, w_steps)
+        w_elapsed, w_sum, _, w_kernel, _ = timed_play_loop(w_global, w_lo2, w_n, 3, w_steps)
         w_env_steps = sum(s_["env_steps"] for s_ in w_sum)
         assert all(s_["episodes"] == w_global and s_["cut_short"] == 0 for s_ in w_sum)
         other = {"scaling": "weak", "envs_per_gpu": ENVS_PER_GPU, "global_batch": w_global, "steps": w_steps,
