@@ -5,7 +5,7 @@
 // Replaces the jax.random calls at src/runs/batch_runner.py:32,105-106,118-119,126-127,
 // src/actions/act_randomly.py:48 and src/ppo/torch_action_wrapper.py:91 of the reference, and the
 // key handling inside Pgx's 2048 _init/_step/_add_random_num.  Everything is integer work kept in
-// registers; one Threefry block is ~85 ALU instructions (ADD / SHF.L.W / LOP3).
+// registers; one Threefry block is 40 ALU-pipe instructions (SHF.L.W / LOP3) and ~42 FMA-pipe adds (IMAD).
 #pragma once
 #include <cstdint>
 
@@ -20,31 +20,55 @@ struct Key {
 
 __device__ __forceinline__ uint32_t rotl32(uint32_t x, int r) { return __funnelshift_l(x, x, r); }
 
-// One Threefry-2x32-20 block.  ks2 = k.a ^ k.b ^ 0x1BD11BDA is recomputed per call; callers that
-// hash many counters under one key get it hoisted by the compiler after inlining.
+// The kernels that hash the most (play3_kernel above all) were bound by the ALU pipe, which takes the rotates (SHF.L.W)
+// and XORs (LOP3) of Threefry.  Left to itself ptxas folds every key injection and the round add after it into one
+// IADD3 -- also an ALU-pipe instruction -- and only the plain round adds become IMAD.IADD on the FMA pipe.  add_fma()
+// keeps an add on the FMA pipe: a mad.lo.u32 by a 1 that ptxas cannot see as a constant (it is read from constant
+// memory, so the multiplier is a uniform-register operand and costs no per-thread register).
+// (Host builds of these headers -- the test shim -- get a plain add.)
+#ifdef __CUDACC__
+static __constant__ uint32_t c_fma_one = 1u;
+#endif
+
+__device__ __forceinline__ uint32_t add_fma(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+    uint32_t d;
+    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(c_fma_one), "r"(b));
+    return d;
+#else
+    return a + b;
+#endif
+}
+
+// One Threefry-2x32-20 block.  Every add runs on the FMA pipe (add_fma); the rotates and XORs stay on the ALU pipe.
+// The key schedule (ks2 and the five `ks + c` sums of the injections) depends on the key alone: callers that hash
+// several counters under one key get it computed once, because the asm statements are pure and common
+// subexpressions after inlining.
 __device__ __forceinline__ Key threefry2x32(Key k, uint32_t x0, uint32_t x1) {
     const uint32_t ks0 = k.a, ks1 = k.b, ks2 = k.a ^ k.b ^ 0x1BD11BDAu;
-    x0 += ks0;
-    x1 += ks1;
-#define G2048_TF_ROUND(r) \
-    x0 += x1;             \
-    x1 = rotl32(x1, r);   \
+    const uint32_t ks2p1 = add_fma(ks2, 1u), ks0p2 = add_fma(ks0, 2u), ks1p3 = add_fma(ks1, 3u);
+    const uint32_t ks2p4 = add_fma(ks2, 4u), ks0p5 = add_fma(ks0, 5u);
+    x0 = add_fma(x0, ks0);
+    x1 = add_fma(x1, ks1);
+#define G2048_TF_ROUND(r)   \
+    x0 = add_fma(x0, x1);   \
+    x1 = rotl32(x1, r);     \
     x1 ^= x0;
     G2048_TF_ROUND(13) G2048_TF_ROUND(15) G2048_TF_ROUND(26) G2048_TF_ROUND(6)
-    x0 += ks1;
-    x1 += ks2 + 1u;
+    x0 = add_fma(x0, ks1);
+    x1 = add_fma(x1, ks2p1);
     G2048_TF_ROUND(17) G2048_TF_ROUND(29) G2048_TF_ROUND(16) G2048_TF_ROUND(24)
-    x0 += ks2;
-    x1 += ks0 + 2u;
+    x0 = add_fma(x0, ks2);
+    x1 = add_fma(x1, ks0p2);
     G2048_TF_ROUND(13) G2048_TF_ROUND(15) G2048_TF_ROUND(26) G2048_TF_ROUND(6)
-    x0 += ks0;
-    x1 += ks1 + 3u;
+    x0 = add_fma(x0, ks0);
+    x1 = add_fma(x1, ks1p3);
     G2048_TF_ROUND(17) G2048_TF_ROUND(29) G2048_TF_ROUND(16) G2048_TF_ROUND(24)
-    x0 += ks1;
-    x1 += ks2 + 4u;
+    x0 = add_fma(x0, ks1);
+    x1 = add_fma(x1, ks2p4);
     G2048_TF_ROUND(13) G2048_TF_ROUND(15) G2048_TF_ROUND(26) G2048_TF_ROUND(6)
-    x0 += ks2;
-    x1 += ks0 + 5u;
+    x0 = add_fma(x0, ks2);
+    x1 = add_fma(x1, ks0p5);
 #undef G2048_TF_ROUND
     return Key{x0, x1};
 }
