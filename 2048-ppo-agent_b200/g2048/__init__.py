@@ -8,6 +8,7 @@ from . import _native  # noqa: F401  loads libg2048.so; raises ImportError if it
 from . import engine, keys  # noqa: F401
 from .actions import act_drul, act_randomly
 from .env_definitions import ACTION_DIM, BOARD_DIM, BOARD_FLAT_DIM, OBS_DIM
+from .playouts import MonteCarloPolicy, PlayoutValues, playout_values
 from .ppo import DevicePPOBatches, PPODataset, PPOIterationLoop, RolloutBuffer, TorchActionFunction, compute_gae, create_ppo_dataloader
 from .runs import BatchRunner, FixedHorizonRunner, FixedRollout, FlatRollout, PackedRollout, run_actions_batch, run_actions_max_tile
 from .state import State
@@ -15,7 +16,7 @@ from .stats import RunningStatsVec
 
 __all__ = [
     "ACTION_DIM", "BOARD_DIM", "BOARD_FLAT_DIM", "OBS_DIM", "BatchRunner", "DevicePPOBatches", "FixedHorizonRunner", "FixedRollout", "FlatRollout",
-    "PPODataset", "PPOIterationLoop", "PackedRollout",
+    "MonteCarloPolicy", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
     "RolloutBuffer", "RunningStatsVec", "State", "TorchActionFunction", "act_drul", "act_randomly", "compute_gae",
-    "create_ppo_dataloader", "engine", "keys", "run_actions_batch", "run_actions_max_tile",
+    "create_ppo_dataloader", "engine", "keys", "playout_values", "run_actions_batch", "run_actions_max_tile",
 ]

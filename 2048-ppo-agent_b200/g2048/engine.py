@@ -290,6 +290,34 @@ def play_record_compact(rec: dict, offsets: torch.Tensor, total: int) -> dict:
     return flat
 
 
+PLAYOUT_STATS = np.dtype([("score_sum", "<u8"), ("score_sq_sum", "<u8"), ("steps_sum", "<u8"), ("playouts", "<u4"),
+                          ("cut_short", "<u4")])  # G2048PlayoutStats (include/g2048.h)
+
+
+def playout_values(policy: int, boards: torch.Tensor, subs: torch.Tensor, playouts: int, rng_mode: int,
+                   board_ids: torch.Tensor | None = None, board_lo: int = 0, n_boards_global: int | None = None,
+                   stats: torch.Tensor | None = None) -> dict:
+    """Monte-Carlo playouts of the given bitboards (g2048_playout_values): for every (board, action) ``playouts`` games
+    played to the end with the built-in ``policy`` after that action.  Board i has the global id ``board_ids[i]``
+    (int64) or ``board_lo + i``; ``n_boards_global`` (default: ``board_lo + n``) sizes the batch the playouts' keys are
+    split over.  ``subs``: sub keys as for ``play`` ([1+2t] act, [2+2t] step keys of playout step t).
+    Returns dict(records (n, 4, 4) int64 -- the raw G2048PlayoutStats --, score_sum, score_sq_sum, steps_sum (n, 4)
+    int64, playouts, cut_short (n, 4) int64, stats); ``stats`` (optional) accumulates g2048_play's statistics block."""
+    dev = boards.device
+    n = boards.shape[0]
+    if n_boards_global is None:
+        n_boards_global = max(board_lo + n, 1)
+    if board_ids is not None:
+        assert board_ids.dtype == torch.int64 and board_ids.shape[0] == n
+    work = torch.zeros(2, dtype=torch.int64, device=dev)
+    records = torch.empty((n, 4, 4), dtype=torch.int64, device=dev)
+    call("g2048_playout_values", policy, ptr(boards), n, ptr(board_ids), board_lo, n_boards_global, playouts,
+         ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(work), ptr(records), ptr(stats), stream_ptr())
+    last = records[..., 3]
+    return dict(records=records, score_sum=records[..., 0], score_sq_sum=records[..., 1], steps_sum=records[..., 2],
+                playouts=last & 0xFFFFFFFF, cut_short=last >> 32, stats=stats)
+
+
 def play_host(policy: int, seed: int, batch_global: int, rng_mode: int, env_lo: int = 0, n: int | None = None,
               key: np.ndarray | None = None, per_env: bool = True, pinned: bool = False):
     """The host-buffer C entry point (numpy in / numpy out; copies and syncs inside the call).

@@ -31,6 +31,7 @@ import torch
 from .. import _native as N
 from .. import engine as E
 from ..keys import KeyChain
+from ..playouts import MonteCarloPolicy, best_actions
 from ..state import State
 
 ENV_ID = "2048"
@@ -279,8 +280,10 @@ class BatchRunner:
         return per-episode ``final_boards`` / ``lengths`` / ``scores`` and a ``summary`` like ``run_stats_batch`` -- no
         records are kept (evaluating an agent over many games, run/viz_ppo_agent.py style, needs none), and only the
         envs that are still alive go through the network.  Same trajectories and key chain as ``run_packed_batch``."""
-        self._check(batch_size)
+        self._check(batch_size, eval_batch=True)
         fn = self._act_fn
+        if isinstance(fn, MonteCarloPolicy):
+            return self._run_eval_monte_carlo(batch_size)
         if not hasattr(fn, "forward_logits"):
             raise ValueError("run_eval_batch needs a TorchActionFunction; use run_stats_batch for act_randomly / act_drul")
         lo, n = self._range(batch_size)
@@ -329,10 +332,62 @@ class BatchRunner:
                    "mean_max_tile": float(tiles.mean().item()) if n else 0.0}
         return {"final_boards": boards, "lengths": lengths, "scores": scores.to(torch.int32), "summary": summary}
 
+    def _run_eval_monte_carlo(self, batch_size: int) -> dict:
+        """run_eval_batch with a ``MonteCarloPolicy``: per loop step t one ``g2048_playout_values`` launch over the envs
+        alive at the start of the chunk (global env ids as board ids; sub keys split(act key of step t, 1 + 2 max_steps)),
+        the best action per env, and ``g2048_env_step`` with the step key of step t.  An env that finishes inside a
+        chunk is still listed until the chunk ends: it has no legal action, so none of its playouts is played, and the
+        step leaves a finished env as it is.  The host reads the done count once per NET_SYNC_STEPS steps."""
+        fn = self._act_fn
+        lo, n = self._range(batch_size)
+        dev, mode = self.device, self.rng_mode
+        policy, n_subs = fn.rollout_policy, 1 + 2 * int(fn.max_steps)
+        boards, status = E.env_init(self.chain.peek(1)[0], batch_size, lo, n, mode)
+        lengths = torch.zeros(n, dtype=torch.int32, device=dev)
+        scores = torch.zeros(n, dtype=torch.int64, device=dev)
+        actions = torch.zeros(n, dtype=torch.int32, device=dev)
+        t0 = 0
+        while True:
+            steps = NET_SYNC_STEPS
+            subs = self.chain.peek(1 + 2 * (t0 + steps))
+            live_ids = torch.nonzero((status & N.STATUS_DONE) == 0).flatten()
+            if live_ids.shape[0]:
+                board_ids = live_ids + lo
+                for k in range(steps):
+                    t = t0 + k
+                    psubs = E.split_keys(subs[1 + 2 * t], n_subs, 0, n_subs, mode)
+                    rec = E.playout_values(policy, boards[live_ids], psubs, int(fn.playouts), mode, board_ids=board_ids,
+                                           n_boards_global=batch_size)
+                    actions[live_ids] = best_actions(rec, fn.criterion).to(torch.int32)
+                    alive = (status & N.STATUS_DONE) == 0
+                    rewards = E.env_step(boards, status, actions, subs[2 + 2 * t], batch_size, lo, mode)
+                    lengths += alive.to(torch.int32)
+                    scores += rewards.to(torch.int64)  # a best action is legal: no -1 penalties, finished envs get 0
+            t0 += steps
+            done_now = int(((status & N.STATUS_DONE) != 0).sum().item())
+            if self._all_done(done_now, n):
+                break
+        t = int(lengths.max().item()) if n else 0  # the reference's number of loop steps: the longest episode
+        if self.shard is not None and self.shard[1] > 1:
+            from ..dist import allreduce_max_int
+
+            t = allreduce_max_int(t, self.device)
+        self.chain.consume(1 + 2 * t)
+        exps = torch.stack([(boards >> (4 * c)) & 15 for c in range(16)], dim=1).amax(dim=1)
+        hist = torch.bincount(exps, minlength=16)
+        tiles = (2.0 ** exps.double())
+        summary = {"episodes": n, "env_steps": int(lengths.sum().item()), "score_sum": int(scores.sum().item()),
+                   "longest": int(lengths.max().item()) if n else 0, "loop_steps": t,
+                   "max_tile_hist": {1 << e: int(c) for e, c in enumerate(hist.tolist()) if c},
+                   "mean_max_tile": float(tiles.mean().item()) if n else 0.0}
+        return {"final_boards": boards, "lengths": lengths, "scores": scores.to(torch.int32), "summary": summary}
+
     # -- internals -----------------------------------------------------------------------------
-    def _check(self, batch_size: int) -> None:
+    def _check(self, batch_size: int, eval_batch: bool = False) -> None:
         if self._act_fn is None:
             raise ValueError("The action function is not set.")
+        if isinstance(self._act_fn, MonteCarloPolicy) and not eval_batch:
+            raise ValueError("a MonteCarloPolicy plays through run_eval_batch only (it keeps no records)")
         if not isinstance(batch_size, (int, np.integer)) or batch_size <= 0:
             raise ValueError(f"batch_size must be a positive integer, got {batch_size!r}")
 

@@ -180,6 +180,37 @@ int g2048_play_record_compact(int policy, const uint64_t* d_arena_boards, const 
  * column 0) the row slid/merged toward column 0 and the flags (bit 0: moves left, bit 2: moves right). */
 int g2048_row_table_lookup(const uint16_t* d_rows, int64_t n, uint16_t* d_left, uint8_t* d_flags, void* stream);
 
+/* ---- Monte-Carlo playout values of caller-given boards: for every (board, action) pair, K games played to the end
+ * with a built-in rollout policy after that action (the play kernel of g2048_play_tables started from a given board
+ * with a forced first move).
+ *   d_boards (n): start bitboards.  Board i has the GLOBAL id d_board_ids[i] (int64, each in [0, n_boards_global)),
+ *           or board_lo + i when d_board_ids is NULL (board_lo must be 0 with an id list).
+ *   playouts = K >= 1.  Playout p = (id * 4 + a) * K + k, k < K, belongs to a batch of P = n_boards_global * 4 * K
+ *           playouts (P <= 2^31 - 1, else G2048_ERR_INVALID), and starts from board `id`:
+ *           at t = 0 it plays action a and spawns with split(d_subs[2], P)[p]; at t >= 1 the policy acts with
+ *           split(d_subs[1 + 2t], P)[p] and the step spawns with split(d_subs[2 + 2t], P)[p] -- g2048_play's per-env
+ *           derivations, so the draws do not depend on how the boards are sharded or ordered.
+ *   d_subs: n_subs >= 3 sub keys laid out as for g2048_play ([0] unused, [1+2t] act, [2+2t] step keys);
+ *           max_steps = (n_subs - 1) / 2 steps per playout, a playout still running then is cut short.
+ *   d_work: uint64[2] scratch, zeroed by the caller (queue head).
+ *   d_records (n * 4, 8-byte aligned): record 4 i + a, OVERWRITTEN: sums over the K playouts of (board i, action a) of
+ *           the score (merge rewards from the start board on, the forced move's included), its square and the steps
+ *           (the forced move included); `playouts` = K if a is legal on board i, else 0 (an illegal pair is not
+ *           played); `cut_short` = playouts that reached max_steps.
+ *   d_stats: NULL, or uint64[G2048_PLAY_STATS_WORDS] ACCUMULATED as g2048_play's, playouts counted as episodes.
+ * A start board that holds a 2^15 tile is outside the contract (as for g2048_play); such playouts are counted in
+ * d_stats[4]. */
+typedef struct G2048PlayoutStats {
+    uint64_t score_sum;
+    uint64_t score_sq_sum;
+    uint64_t steps_sum;
+    uint32_t playouts;
+    uint32_t cut_short;
+} G2048PlayoutStats;
+int g2048_playout_values(int policy, const uint64_t* d_boards, int64_t n, const int64_t* d_board_ids, int64_t board_lo,
+                         int64_t n_boards_global, int64_t playouts, const uint32_t* d_subs, int64_t n_subs, int rng_mode,
+                         uint64_t* d_work, G2048PlayoutStats* d_records, uint64_t* d_stats, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.
