@@ -160,8 +160,9 @@ __device__ __forceinline__ void spawn_select(u64 x, uint32_t bits_pos, uint32_t 
     const int k = (int)ceilf(r);
     // a full board (only reachable through the illegal-action path) leaves searchsorted at cell 0
     cell = (n_empty == 0) ? 0 : kth_flag_cell(empties, k);
-    const uint32_t m_val = 0x800000u - (bits_val >> 9);
-    val = (m_val > 7549747u) ? 2ull : 1ull;  // m * 2^-23 > 0.9f = 15099494 * 2^-24
+    // m * 2^-23 > 0.9f = 15099494 * 2^-24  <=>  m = 2^23 - (bits >> 9) > 7549747  <=>  bits >> 9 < 838861
+    //                                      <=>  bits < 838861 * 2^9 = 429496832 (tests/test_step_logic.py)
+    val = (bits_val < 429496832u) ? 2ull : 1ull;
 }
 
 __device__ __forceinline__ u64 spawn_tile(u64 x, uint32_t bits_pos, uint32_t bits_val) {
@@ -171,13 +172,30 @@ __device__ __forceinline__ u64 spawn_tile(u64 x, uint32_t bits_pos, uint32_t bit
     return (x & ~(0xFull << (4 * cell))) | (val << (4 * cell));
 }
 
-// transpose of the 4x4 nibble matrix: cell (r, c) <-> cell (c, r)
+// (a & m) | (b & ~m) as one LOP3 (left to itself, ptxas splits the mirror's select below into two)
+__device__ __forceinline__ uint32_t bit_select(uint32_t a, uint32_t b, uint32_t m) {
+#ifdef __CUDA_ARCH__
+    uint32_t d;
+    asm("lop3.b32 %0, %1, %2, %3, 0xE4;" : "=r"(d) : "r"(a), "r"(b), "r"(m));  // 0xE4 = (0xF0 & 0xAA) | (0xCC & ~0xAA)
+    return d;
+#else
+    return (a & m) | (b & ~m);
+#endif
+}
+
+// transpose of the 4x4 nibble matrix: cell (r, c) <-> cell (c, r), in 32-bit halves (the 64-bit form costs twice the
+// ALU-pipe instructions: every 64-bit shift is two)
 __device__ __forceinline__ u64 transpose_board(u64 x) {
-    u64 t = (x ^ (x >> 12)) & 0x0000F0F00000F0F0ull;
-    x ^= t ^ (t << 12);
-    t = (x ^ (x >> 24)) & 0x00000000FF00FF00ull;
-    x ^= t ^ (t << 24);
-    return x;
+    uint32_t lo = (uint32_t)x, hi = (uint32_t)(x >> 32);
+    // 2x2 blocks of cells: swap the (0, 1) and (1, 0) cells of each, which lie in the same half (rows 0-1 / rows 2-3);
+    // t and t << 12 cannot overlap, so t ^ (t << 12) = t * 4097
+    const uint32_t tl = (lo ^ (lo >> 12)) & 0x0000F0F0u, th = (hi ^ (hi >> 12)) & 0x0000F0F0u;
+    lo ^= mad_fma<4097u>(tl, 0u);
+    hi ^= mad_fma<4097u>(th, 0u);
+    // 2x2 blocks of blocks: the upper right block (bytes 1 and 3 of the low half) and the lower left one (bytes 0 and
+    // 2 of the high half) change places
+    const uint32_t nlo = __byte_perm(lo, hi, 0x6240), nhi = __byte_perm(lo, hi, 0x7351);
+    return ((u64)nhi << 32) | nlo;
 }
 
 // reverse the nibble order inside each 16-bit row (mirror the board left <-> right)
@@ -185,8 +203,10 @@ __device__ __forceinline__ u64 mirror_rows(u64 x) {
     uint32_t lo = (uint32_t)x, hi = (uint32_t)(x >> 32);
     lo = __byte_perm(lo, 0, 0x2301);
     hi = __byte_perm(hi, 0, 0x2301);
-    lo = ((lo & 0x0F0F0F0Fu) << 4) | ((lo >> 4) & 0x0F0F0F0Fu);
-    hi = ((hi & 0x0F0F0F0Fu) << 4) | ((hi >> 4) & 0x0F0F0F0Fu);
+    // the two nibbles of every byte change places: one bit-select between the word shifted up (on the FMA pipe) and
+    // the word shifted down
+    lo = bit_select(mad_fma<16u>(lo, 0u), lo >> 4, 0xF0F0F0F0u);
+    hi = bit_select(mad_fma<16u>(hi, 0u), hi >> 4, 0xF0F0F0F0u);
     return ((u64)hi << 32) | lo;
 }
 

@@ -9,10 +9,10 @@
 //   * the exact legal-action mask is 8 byte loads from a second table (64 KiB): "this row can move
 //     left / right", looked up for the four rows of the board and the four rows of its transpose;
 //   * the lane keeps the board AND its transpose in registers, so a vertical move is a horizontal
-//     move on the transpose and every step pays exactly one 16-instruction transpose.
+//     move on the transpose and every step pays exactly one transpose (8 ALU-pipe instructions).
 // Shared-memory loads issue on the LSU pipe, which the kernel otherwise leaves idle.
-// 192 KiB of tables -> one CTA of 512 threads per SM (16 warps keep the ALU pipe saturated).  Same lane scheduling, init-as-two-
-// iterations trick, score-from-potential and results as g2048_play.cu (bit-identical; tested).
+// 192 KiB of tables -> one CTA per SM, of 768 threads (512 for small batches: play3_block_threads).  Same lane
+// scheduling, init-as-two-iterations trick, score-from-potential and results as g2048_play.cu (bit-identical; tested).
 #include "g2048_play3.cuh"
 
 namespace g2048 {
@@ -42,9 +42,14 @@ struct TailEntry {
 };
 constexpr int PLAY3_STATS_BYTES = G2048_PLAY_STATS_WORDS * 8;
 constexpr int PLAY3_CTL_BYTES = 16;  // tail flag, two alternating live-env counters
-constexpr int PLAY3_POOL_BYTES = PLAY3_THREADS * (int)sizeof(TailEntry);
-constexpr int PLAY3_SPAWN_OFFSET = PLAY3_TABLE_BYTES + PLAY3_STATS_BYTES + PLAY3_CTL_BYTES + PLAY3_POOL_BYTES;
-constexpr int PLAY3_SMEM_BYTES = PLAY3_SPAWN_OFFSET + PLAY3_SPAWN_BYTES;
+// the shared memory of a CTA of THREADS threads: row tables, statistics, tail control, tail pool, spawn masks, action table
+template <int THREADS>
+struct Play3Smem {
+    static constexpr int POOL_BYTES = THREADS * (int)sizeof(TailEntry);
+    static constexpr int SPAWN_OFFSET = PLAY3_TABLE_BYTES + PLAY3_STATS_BYTES + PLAY3_CTL_BYTES + POOL_BYTES;
+    static constexpr int ACT_OFFSET = SPAWN_OFFSET + PLAY3_SPAWN_BYTES;
+    static constexpr int BYTES = ACT_OFFSET + PLAY3_ACT_BYTES;
+};
 
 __device__ __forceinline__ void play3_epilogue(Play3Lane& L, const Play3Ctx& c) {
     if (L.pk_has) {
@@ -150,8 +155,8 @@ __device__ G2048_TAIL_INLINE void play3_tail(Play3Lane& lane_state, const Play3C
     lane_state = L;
 }
 
-template <int MODE, int POLICY, bool REC>
-__global__ void __launch_bounds__(PLAY3_THREADS, 1)
+template <int MODE, int POLICY, bool REC, int THREADS>
+__global__ void __launch_bounds__(THREADS, 1)
 play3_kernel(const uint2* __restrict__ subs, int64_t n_subs, uint32_t batch_global, uint32_t env_lo, uint32_t n,
              unsigned long long* __restrict__ work, u64* __restrict__ final_boards, uint32_t* __restrict__ lengths,
              uint32_t* __restrict__ scores, unsigned long long* __restrict__ stats, uint4* __restrict__ results,
@@ -165,17 +170,18 @@ play3_kernel(const uint2* __restrict__ subs, int64_t n_subs, uint32_t batch_glob
 #endif
 
     {
-        play3_copy_row_tables(smem_raw);
-        for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += PLAY3_THREADS) s_stats[i] = 0ull;
+        play3_copy_row_tables<THREADS>(smem_raw);
+        for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += THREADS) s_stats[i] = 0ull;
         if (threadIdx.x < 4) reinterpret_cast<unsigned*>(smem_raw + PLAY3_TABLE_BYTES + PLAY3_STATS_BYTES)[threadIdx.x] = 0u;
         // the spawn masks, as play3_fill_spawn_masks writes them (spelt out here: through the helper ptxas masks one
         // address differently, and this kernel's code is kept instruction for instruction)
         if (threadIdx.x < 16) {
             const unsigned cell = threadIdx.x, cellT = ((cell & 3u) << 2) | (cell >> 2);
             const u64 m = 1ull << (4 * cell), mT = 1ull << (4 * cellT);
-            reinterpret_cast<uint4*>(smem_raw + PLAY3_SPAWN_OFFSET)[cell] =
+            reinterpret_cast<uint4*>(smem_raw + Play3Smem<THREADS>::SPAWN_OFFSET)[cell] =
                 make_uint4((uint32_t)m, (uint32_t)(m >> 32), (uint32_t)mT, (uint32_t)(mT >> 32));
         }
+        play3_fill_act_table(reinterpret_cast<ActEntry*>(smem_raw + Play3Smem<THREADS>::ACT_OFFSET));
     }
     __syncthreads();
 
@@ -188,7 +194,8 @@ play3_kernel(const uint2* __restrict__ subs, int64_t n_subs, uint32_t batch_glob
     c.env_lo = env_lo;
     c.s_left = reinterpret_cast<const uint16_t*>(smem_raw);
     c.s_flags = smem_raw + 65536 * 2;
-    c.s_spawn = reinterpret_cast<const uint4*>(smem_raw + PLAY3_SPAWN_OFFSET);
+    c.s_spawn = reinterpret_cast<const uint4*>(smem_raw + Play3Smem<THREADS>::SPAWN_OFFSET);
+    c.s_act = reinterpret_cast<const ActEntry*>(smem_raw + Play3Smem<THREADS>::ACT_OFFSET);
     c.s_stats = s_stats;
     c.final_boards = final_boards;
     c.lengths = lengths;
@@ -199,7 +206,7 @@ play3_kernel(const uint2* __restrict__ subs, int64_t n_subs, uint32_t batch_glob
     Play3Lane L = {};
     L.phase = PHASE_NONE;
     if (REC) {
-        L.slot = ((unsigned long long)blockIdx.x * PLAY3_THREADS + threadIdx.x) * rec.cap;
+        L.slot = ((unsigned long long)blockIdx.x * THREADS + threadIdx.x) * rec.cap;
         L.slot_end = L.slot + rec.cap;
     }
     bool exhausted = false;  // warp-uniform
@@ -299,35 +306,54 @@ __global__ void row_table_lookup_kernel(const uint16_t* __restrict__ rows, int64
     flags[i] = g_row_flags[rows[i]];
 }
 
-// CTAs of a table-kernel launch over n envs (one per SM, persistent); the recording form sizes its arena by it
-static int64_t play3_grid(int64_t n, int sms) {
-    const int64_t needed = (n + PLAY3_THREADS - 1) / PLAY3_THREADS;
-    return needed < sms ? needed : sms;
+// CTAs (one per SM, persistent) and threads per CTA of a table-kernel launch over n envs; the recording form sizes its
+// arena by them
+struct Play3Shape {
+    int64_t grid;
+    int threads;
+    int64_t lanes() const { return grid * threads; }
+};
+static Play3Shape play3_shape(int64_t n, int sms) {
+    const int threads = play3_block_threads(n, sms);
+    const int64_t needed = (n + threads - 1) / threads;
+    return Play3Shape{needed < sms ? needed : sms, threads};
+}
+
+template <int MODE, int POLICY, bool REC, int THREADS>
+static int launch_play3_with(int64_t grid, const uint32_t* d_subs, int64_t n_subs, int64_t batch_global, int64_t env_lo,
+                             int64_t n, uint64_t* d_work, uint64_t* d_final_boards, uint32_t* d_lengths, uint32_t* d_scores,
+                             uint64_t* d_stats, cudaStream_t st, void* d_results, PlayRecordArena rec) {
+    static bool configured_on[64] = {false};
+    bool* configured = device_once_flag(configured_on);
+    if (!configured) return fail_arg("no CUDA device");
+    if (!*configured) {
+        const int rc = check_cuda(cudaFuncSetAttribute(play3_kernel<MODE, POLICY, REC, THREADS>,
+                                                       cudaFuncAttributeMaxDynamicSharedMemorySize, Play3Smem<THREADS>::BYTES),
+                                  "play: shared memory attribute");
+        if (rc) return rc;
+        *configured = true;
+    }
+    play3_kernel<MODE, POLICY, REC, THREADS><<<(unsigned)grid, THREADS, Play3Smem<THREADS>::BYTES, st>>>(
+        (const uint2*)d_subs, n_subs, (uint32_t)batch_global, (uint32_t)env_lo, (uint32_t)n,
+        (unsigned long long*)d_work, (u64*)d_final_boards, d_lengths, d_scores, (unsigned long long*)d_stats,
+        (uint4*)d_results, rec);
+    return check_cuda(cudaGetLastError(), "play");
 }
 
 template <int MODE, int POLICY, bool REC>
 static int launch_play3(const uint32_t* d_subs, int64_t n_subs, int64_t batch_global, int64_t env_lo, int64_t n,
                         uint64_t* d_work, uint64_t* d_final_boards, uint32_t* d_lengths, uint32_t* d_scores,
                         uint64_t* d_stats, cudaStream_t st, void* d_results, PlayRecordArena rec = PlayRecordArena{}) {
-    int rc = ensure_row_tables(st);
+    const int rc = ensure_row_tables(st);
     if (rc) return rc;
-    static bool configured_on[64] = {false};
-    bool* configured = device_once_flag(configured_on);
-    if (!configured) return fail_arg("no CUDA device");
-    if (!*configured) {
-        rc = check_cuda(cudaFuncSetAttribute(play3_kernel<MODE, POLICY, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             PLAY3_SMEM_BYTES), "play: shared memory attribute");
-        if (rc) return rc;
-        *configured = true;
-    }
     const int sms = sm_count();
     if (sms <= 0) return fail_arg("play: no device");
-    const int64_t grid = play3_grid(n, sms);  // one CTA per SM, persistent
-    play3_kernel<MODE, POLICY, REC><<<(unsigned)grid, PLAY3_THREADS, PLAY3_SMEM_BYTES, st>>>(
-        (const uint2*)d_subs, n_subs, (uint32_t)batch_global, (uint32_t)env_lo, (uint32_t)n,
-        (unsigned long long*)d_work, (u64*)d_final_boards, d_lengths, d_scores, (unsigned long long*)d_stats,
-        (uint4*)d_results, rec);
-    return check_cuda(cudaGetLastError(), "play");
+    const Play3Shape shape = play3_shape(n, sms);
+    if (shape.threads == PLAY3_THREADS)
+        return launch_play3_with<MODE, POLICY, REC, PLAY3_THREADS>(shape.grid, d_subs, n_subs, batch_global, env_lo, n, d_work,
+                                                                   d_final_boards, d_lengths, d_scores, d_stats, st, d_results, rec);
+    return launch_play3_with<MODE, POLICY, REC, PLAY3_SMALL_THREADS>(shape.grid, d_subs, n_subs, batch_global, env_lo, n, d_work,
+                                                                     d_final_boards, d_lengths, d_scores, d_stats, st, d_results, rec);
 }
 
 // the table kernel with every output form (d_results: one 16-byte G2048EpisodeResult per env, may be NULL)
@@ -356,7 +382,7 @@ int play_tables_impl(int policy, const uint32_t* d_subs, int64_t n_subs, int64_t
 
 // slots per lane: room for one whole episode (max_steps + 1) beyond the lane's expected share of the batch's records
 static int64_t play_record_lane_slots(int64_t n, int64_t max_steps, int64_t mean_steps, int sms) {
-    const int64_t lanes = play3_grid(n, sms) * PLAY3_THREADS;
+    const int64_t lanes = play3_shape(n, sms).lanes();
     const int64_t envs_per_lane = (n + lanes - 1) / lanes;
     // share: mean episode (+1 slot for its final board) x envs per lane, +25 % and two mean episodes of slack for the
     // imbalance between lanes (a lane that runs out retires; the others take its envs)
@@ -377,7 +403,7 @@ int play_record_impl(int policy, const uint32_t* d_subs, int64_t n_subs, int64_t
     G2048_REQUIRE(d_arena_boards && d_arena_meta && d_env_slot && d_lengths, "play_record: record pointers");
     const int sms = sm_count();
     if (sms <= 0) return fail_arg("play_record: no device");
-    const int64_t lanes = play3_grid(n, sms) * PLAY3_THREADS;
+    const int64_t lanes = play3_shape(n, sms).lanes();
     const int64_t max_steps = (n_subs - 1) / 2;
     PlayRecordArena rec;
     rec.boards = (u64*)d_arena_boards;
@@ -535,7 +561,7 @@ extern "C" int64_t g2048_play_record_arena_slots(int64_t n, int64_t n_subs, int6
     if (n <= 0 || n_subs < 3 || mean_steps < 0) return -1;
     const int sms = sm_count();
     if (sms <= 0) return -1;
-    const int64_t lanes = play3_grid(n, sms) * PLAY3_THREADS;
+    const int64_t lanes = play3_shape(n, sms).lanes();
     return lanes * play_record_lane_slots(n, (n_subs - 1) / 2, mean_steps, sms);
 }
 

@@ -9,13 +9,33 @@
 namespace g2048 {
 
 #ifndef G2048_PLAY3_THREADS
-#define G2048_PLAY3_THREADS 512
+#define G2048_PLAY3_THREADS 768
+#endif
+#ifndef G2048_PLAY3_SMALL_THREADS
+#define G2048_PLAY3_SMALL_THREADS 512
+#endif
+#ifndef G2048_PLAY3_BIG_ENVS_PER_LANE
+#define G2048_PLAY3_BIG_ENVS_PER_LANE 16
 #endif
 #ifndef G2048_PLAY3_EPILOGUE_BATCH
 #define G2048_PLAY3_EPILOGUE_BATCH 16
 #endif
 constexpr int PLAY3_EPILOGUE_BATCH = G2048_PLAY3_EPILOGUE_BATCH;  // parked finished episodes per epilogue run
-constexpr int PLAY3_THREADS = G2048_PLAY3_THREADS;  // one CTA per SM; 512 / 768 / 1024 threads measured within 3 % of each other, 512 best (shorter tail)
+// One CTA per SM.  While the kernel was bound by the ALU pipe alone, 512 / 768 / 1024 threads were within 3 % and 512
+// drained fastest.  With fewer ALU instructions per step latency matters more: 768 threads (24 warps, <= 80 registers,
+// no spills) are 2.7 % faster at 2^24 envs, but the drain of the last episodes, longer with more lanes, makes them
+// slower where a lane plays only a few envs (2^18 envs: +7 %; break-even between 2^20 and 2^21 envs on 148 SMs, 9 and
+// 18 envs per lane).  So the kernels are compiled for both sizes, and a launch runs PLAY3_THREADS threads per CTA
+// when every lane gets at least PLAY3_BIG_ENVS_PER_LANE envs on average, else PLAY3_SMALL_THREADS (profiles/README.md,
+// round 5).  (One build for 768 threads launched with 512 where needed is as fast at small sizes, but the block size
+// read at run time changes ptxas's schedule of the whole kernel: 2^24 envs 63.1 -> 63.8 ms.)
+constexpr int PLAY3_THREADS = G2048_PLAY3_THREADS;
+constexpr int PLAY3_SMALL_THREADS = G2048_PLAY3_SMALL_THREADS;
+
+// threads per CTA of a launch over n envs (or playouts) on `sms` SMs
+inline int play3_block_threads(int64_t n, int sms) {
+    return n >= (int64_t)G2048_PLAY3_BIG_ENVS_PER_LANE * sms * PLAY3_THREADS ? PLAY3_THREADS : PLAY3_SMALL_THREADS;
+}
 constexpr int PLAY3_TABLE_BYTES = 65536 * 2 + 65536;
 
 // (static: each translation unit that includes this file has its own tables)
@@ -55,13 +75,14 @@ __device__ __forceinline__ void build_row_table_entry(uint32_t row) {
     g_row_flags[row] = (uint8_t)((left != row ? 1u : 0u) | (right != row ? 4u : 0u));  // bits 0 and 2: see the legal mask below
 }
 
-// tables: global (L2) -> shared (at smem_raw: left moves, then flags), 12 x 16 bytes per thread
+// tables: global (L2) -> shared (at smem_raw: left moves, then flags), by a CTA of THREADS threads
+template <int THREADS>
 __device__ __forceinline__ void play3_copy_row_tables(uint8_t* smem_raw) {
     const uint4* src_left = reinterpret_cast<const uint4*>(g_row_left);
     const uint4* src_flags = reinterpret_cast<const uint4*>(g_row_flags);
     uint4* dst = reinterpret_cast<uint4*>(smem_raw);
-    for (int i = threadIdx.x; i < 65536 * 2 / 16; i += PLAY3_THREADS) dst[i] = __ldg(&src_left[i]);
-    for (int i = threadIdx.x; i < 65536 / 16; i += PLAY3_THREADS) dst[65536 * 2 / 16 + i] = __ldg(&src_flags[i]);
+    for (int i = threadIdx.x; i < 65536 * 2 / 16; i += THREADS) dst[i] = __ldg(&src_left[i]);
+    for (int i = threadIdx.x; i < 65536 / 16; i += THREADS) dst[65536 * 2 / 16 + i] = __ldg(&src_flags[i]);
 }
 
 // spawn masks: for each cell, a 1 in its nibble of the board and in its nibble of the transpose (uint4: lo, hi, lo, hi)
@@ -72,6 +93,12 @@ __device__ __forceinline__ void play3_fill_spawn_masks(uint4* s_spawn) {
         const u64 m = 1ull << (4 * cell), mT = 1ull << (4 * cellT);
         s_spawn[cell] = make_uint4((uint32_t)m, (uint32_t)(m >> 32), (uint32_t)mT, (uint32_t)(mT >> 32));
     }
+}
+
+// the random policy's action table (act_random_table, g2048_play.cuh), one entry per legal mask
+constexpr int PLAY3_ACT_BYTES = 16 * (int)sizeof(ActEntry);
+__device__ __forceinline__ void play3_fill_act_table(ActEntry* s_act) {
+    if (threadIdx.x < 16) s_act[threadIdx.x] = act_entry_of(threadIdx.x);
 }
 
 // Recording form (REC = true; src/runs/batch_runner.py:117-154 + src/ppo/rollout_buffer.py:164-187): the lane also
@@ -120,6 +147,7 @@ struct Play3Ctx {
     const uint16_t* s_left;
     const uint8_t* s_flags;
     const uint4* s_spawn;
+    const ActEntry* s_act;
     unsigned long long* s_stats;
     u64* final_boards;
     uint32_t* lengths;
@@ -156,7 +184,7 @@ __device__ __forceinline__ void play3_step(Play3Lane& L, const Play3Ctx& c) {
         const uint2 sa = __ldg(&c.subs[1 + 2 * (int64_t)L.t]);
         const Key head = playing ? Key{sa.x, sa.y} : Key{c.init_sub.x, c.init_sub.y};
         const KeyBlocks<MODE> kb = key_blocks<MODE>(split_at<MODE>(head, c.batch_global, c.env_lo + L.e));
-        action = argmax_bits_legal(kb.bits, L.lm);
+        action = act_random_table(kb.bits, c.s_act[L.lm]);  // = argmax_bits_legal(kb.bits, L.lm)
         const Key kplay = split_at<MODE>(Key{ss.x, ss.y}, c.batch_global, c.env_lo + L.e);
         const Key kinit = (L.phase == PHASE_INIT0) ? kb.child[0] : kb.child[1];
         kstep = playing ? kplay : kinit;

@@ -9,7 +9,8 @@ namespace g2048 {
 
 constexpr int PLAYOUT_STATS_BYTES = G2048_PLAY_STATS_WORDS * 8;
 constexpr int PLAYOUT_SPAWN_OFFSET = PLAY3_TABLE_BYTES + PLAYOUT_STATS_BYTES;
-constexpr int PLAYOUT_SMEM_BYTES = PLAYOUT_SPAWN_OFFSET + PLAY3_SPAWN_BYTES;
+constexpr int PLAYOUT_ACT_OFFSET = PLAYOUT_SPAWN_OFFSET + PLAY3_SPAWN_BYTES;
+constexpr int PLAYOUT_SMEM_BYTES = PLAYOUT_ACT_OFFSET + PLAY3_ACT_BYTES;
 
 // A playout lane: the game as play3_step sees it (e = the global playout index p, which keys its draws) and what the
 // epilogue needs besides -- the (board, action) record it adds to and the start board's potential -- live and parked.
@@ -67,17 +68,18 @@ __device__ __forceinline__ void playout_park(PlayoutLane& P, const Play3Ctx& c, 
 }
 
 // Work item j < n * 4 * K is playout k = j % K of action a = (j / K) % 4 on board i = j / (4 K); its record is j / K.
-template <int MODE, int POLICY>
-__global__ void __launch_bounds__(PLAY3_THREADS, 1)
+template <int MODE, int POLICY, int THREADS>
+__global__ void __launch_bounds__(THREADS, 1)
 playout_kernel(const u64* __restrict__ boards, const int64_t* __restrict__ board_ids, uint32_t board_lo, uint32_t n_items,
                uint32_t playouts, const uint2* __restrict__ subs, int64_t n_subs, uint32_t batch_global,
                unsigned long long* __restrict__ work, G2048PlayoutStats* __restrict__ records,
                unsigned long long* __restrict__ stats) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     unsigned long long* s_stats = reinterpret_cast<unsigned long long*>(smem_raw + PLAY3_TABLE_BYTES);
-    play3_copy_row_tables(smem_raw);
-    for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += PLAY3_THREADS) s_stats[i] = 0ull;
+    play3_copy_row_tables<THREADS>(smem_raw);
+    for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += THREADS) s_stats[i] = 0ull;
     play3_fill_spawn_masks(reinterpret_cast<uint4*>(smem_raw + PLAYOUT_SPAWN_OFFSET));
+    play3_fill_act_table(reinterpret_cast<ActEntry*>(smem_raw + PLAYOUT_ACT_OFFSET));
     __syncthreads();
 
     const unsigned lane = threadIdx.x & 31u;
@@ -90,6 +92,7 @@ playout_kernel(const u64* __restrict__ boards, const int64_t* __restrict__ board
     c.s_left = reinterpret_cast<const uint16_t*>(smem_raw);
     c.s_flags = smem_raw + 65536 * 2;
     c.s_spawn = reinterpret_cast<const uint4*>(smem_raw + PLAYOUT_SPAWN_OFFSET);
+    c.s_act = reinterpret_cast<const ActEntry*>(smem_raw + PLAYOUT_ACT_OFFSET);
     c.s_stats = s_stats;
 
     PlayoutLane P = {};
@@ -163,29 +166,41 @@ __global__ void build_playout_row_tables_kernel() {
     build_row_table_entry(row);
 }
 
-template <int MODE, int POLICY>
-static int launch_playout(const uint64_t* d_boards, const int64_t* d_board_ids, int64_t board_lo, int64_t n_items,
-                          int64_t playouts, const uint32_t* d_subs, int64_t n_subs, int64_t batch_global, uint64_t* d_work,
-                          G2048PlayoutStats* d_records, uint64_t* d_stats, cudaStream_t st) {
-    int rc = ensure_row_tables_with<build_playout_row_tables_kernel>(st);
-    if (rc) return rc;
+template <int MODE, int POLICY, int THREADS>
+static int launch_playout_with(int64_t grid, const uint64_t* d_boards, const int64_t* d_board_ids, int64_t board_lo,
+                               int64_t n_items, int64_t playouts, const uint32_t* d_subs, int64_t n_subs, int64_t batch_global,
+                               uint64_t* d_work, G2048PlayoutStats* d_records, uint64_t* d_stats, cudaStream_t st) {
     static bool configured_on[64] = {false};
     bool* configured = device_once_flag(configured_on);
     if (!configured) return fail_arg("no CUDA device");
     if (!*configured) {
-        rc = check_cuda(cudaFuncSetAttribute(playout_kernel<MODE, POLICY>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             PLAYOUT_SMEM_BYTES), "playout_values: shared memory attribute");
+        const int rc = check_cuda(cudaFuncSetAttribute(playout_kernel<MODE, POLICY, THREADS>,
+                                                       cudaFuncAttributeMaxDynamicSharedMemorySize, PLAYOUT_SMEM_BYTES),
+                                  "playout_values: shared memory attribute");
         if (rc) return rc;
         *configured = true;
     }
-    const int sms = sm_count();
-    if (sms <= 0) return fail_arg("playout_values: no device");
-    const int64_t needed = (n_items + PLAY3_THREADS - 1) / PLAY3_THREADS;
-    const int64_t grid = needed < sms ? needed : sms;  // one CTA per SM, persistent
-    playout_kernel<MODE, POLICY><<<(unsigned)grid, PLAY3_THREADS, PLAYOUT_SMEM_BYTES, st>>>(
+    playout_kernel<MODE, POLICY, THREADS><<<(unsigned)grid, THREADS, PLAYOUT_SMEM_BYTES, st>>>(
         (const u64*)d_boards, d_board_ids, (uint32_t)board_lo, (uint32_t)n_items, (uint32_t)playouts, (const uint2*)d_subs,
         n_subs, (uint32_t)batch_global, (unsigned long long*)d_work, d_records, (unsigned long long*)d_stats);
     return check_cuda(cudaGetLastError(), "playout_values");
+}
+
+template <int MODE, int POLICY>
+static int launch_playout(const uint64_t* d_boards, const int64_t* d_board_ids, int64_t board_lo, int64_t n_items,
+                          int64_t playouts, const uint32_t* d_subs, int64_t n_subs, int64_t batch_global, uint64_t* d_work,
+                          G2048PlayoutStats* d_records, uint64_t* d_stats, cudaStream_t st) {
+    const int rc = ensure_row_tables_with<build_playout_row_tables_kernel>(st);
+    if (rc) return rc;
+    const int sms = sm_count();
+    if (sms <= 0) return fail_arg("playout_values: no device");
+    const int threads = play3_block_threads(n_items, sms);
+    const int64_t needed = (n_items + threads - 1) / threads;
+    const int64_t grid = needed < sms ? needed : sms;  // one CTA per SM, persistent
+#define ARGS grid, d_boards, d_board_ids, board_lo, n_items, playouts, d_subs, n_subs, batch_global, d_work, d_records, d_stats, st
+    if (threads == PLAY3_THREADS) return launch_playout_with<MODE, POLICY, PLAY3_THREADS>(ARGS);
+    return launch_playout_with<MODE, POLICY, PLAY3_SMALL_THREADS>(ARGS);
+#undef ARGS
 }
 
 }  // namespace g2048

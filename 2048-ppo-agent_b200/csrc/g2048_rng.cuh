@@ -40,6 +40,20 @@ __device__ __forceinline__ uint32_t add_fma(uint32_t a, uint32_t b) {
 #endif
 }
 
+// a * M + b on the FMA pipe, for constant M (a shift by a constant and an OR or XOR with bits it cannot overlap, in one
+// instruction).  The multiplier is M times the constant-memory 1, so ptxas cannot turn the product back into a shift
+// (SHF / LEA on the ALU pipe); the product of two uniform values is computed once, outside the loops.
+template <uint32_t M>
+__device__ __forceinline__ uint32_t mad_fma(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+    uint32_t d;
+    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(c_fma_one * M), "r"(b));
+    return d;
+#else
+    return a * M + b;
+#endif
+}
+
 // One Threefry-2x32-20 block.  Every add runs on the FMA pipe (add_fma); the rotates and XORs stay on the ALU pipe.
 // The key schedule (ks2 and the five `ks + c` sums of the injections) depends on the key alone: callers that hash
 // several counters under one key get it computed once, because the asm statements are pure and common

@@ -23,7 +23,7 @@ OUT = ROOT / "profiles" / "r03_sass_opcodes.txt"
 # instruction every two cycles per scheduler (VIADD, PRMT and LEA.HI: tools/probes/probe_int.cu, profiles/README.md)
 ALU_PIPE = ("LOP3", "SHF", "IADD3", "SEL", "VIADD", "PRMT", "LEA", "ISETP", "IMNMX", "VIMNMX", "FSEL", "FSETP", "PLOP3",
             "P2R", "R2P", "FLO", "BREV", "IABS", "LOP", "IADD", "MOV")
-STEP_KERNELS = ("play3_kernel<1, 0, false>", "play3_kernel<1, 1, false>")
+STEP_KERNELS = ("play3_kernel<1, 0, false", "play3_kernel<1, 1, false")  # every block size (last template argument)
 KEEP = ("play3_kernel", "play2_kernel", "play_record_compact", "policy_step_obs", "policy_step_kernel", "rollout_steps_kernel",
         "expand_obs_tma_kernel", "pack_samples", "gae_scan_kernel", "gae_scan_fix", "gae_flat4_kernel", "gae_flat3_kernel",
         "gae_time_major_kernel", "gae_time_major_ring_kernel", "gather_samples_tile_kernel", "compact_records_kernel",
@@ -94,10 +94,8 @@ def main():
         out.append(f"## {name[:150]}")
         out.append(f"   {total} instructions; " + ", ".join(f"{k} {v}" for k, v in c.most_common(14)))
         out.append("")
-    for want in STEP_KERNELS:
-        name = next((k for k in kernels if want in k), None)
-        if name is None:
-            continue
+    for name in (k for want in STEP_KERNELS for k in kernels if want in k):
+        want = name[name.index("play3_kernel"):name.index(">") + 1]
         body = step_body("\n".join(listings[name]))
         by_pipe = collections.Counter()
         for op, v in body.items():
