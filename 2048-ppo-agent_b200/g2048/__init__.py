@@ -8,6 +8,7 @@ from . import _native  # noqa: F401  loads libg2048.so; raises ImportError if it
 from . import engine, keys  # noqa: F401
 from .actions import act_drul, act_randomly
 from .env_definitions import ACTION_DIM, BOARD_DIM, BOARD_FLAT_DIM, OBS_DIM
+from .expectimax import ExpectimaxPolicy, ExpectimaxValues, default_row_values, expectimax_values
 from .playouts import MonteCarloPolicy, PlayoutValues, playout_values
 from .ppo import DevicePPOBatches, PPODataset, PPOIterationLoop, RolloutBuffer, TorchActionFunction, compute_gae, create_ppo_dataloader
 from .runs import BatchRunner, FixedHorizonRunner, FixedRollout, FlatRollout, PackedRollout, run_actions_batch, run_actions_max_tile
@@ -15,8 +16,8 @@ from .state import State
 from .stats import RunningStatsVec
 
 __all__ = [
-    "ACTION_DIM", "BOARD_DIM", "BOARD_FLAT_DIM", "OBS_DIM", "BatchRunner", "DevicePPOBatches", "FixedHorizonRunner", "FixedRollout", "FlatRollout",
+    "ACTION_DIM", "BOARD_DIM", "BOARD_FLAT_DIM", "OBS_DIM", "BatchRunner", "DevicePPOBatches", "ExpectimaxPolicy", "ExpectimaxValues", "FixedHorizonRunner", "FixedRollout", "FlatRollout",
     "MonteCarloPolicy", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
     "RolloutBuffer", "RunningStatsVec", "State", "TorchActionFunction", "act_drul", "act_randomly", "compute_gae",
-    "create_ppo_dataloader", "engine", "keys", "playout_values", "run_actions_batch", "run_actions_max_tile",
+    "create_ppo_dataloader", "default_row_values", "engine", "expectimax_values", "keys", "playout_values", "run_actions_batch", "run_actions_max_tile",
 ]

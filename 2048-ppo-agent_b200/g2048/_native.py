@@ -43,6 +43,7 @@ _INT = C.c_int
 _DBL = C.c_double
 _U64 = C.c_uint64
 _U32 = C.c_uint32
+_FLT = C.c_float
 
 _SIGNATURES = {
     "g2048_version": (_INT, []),
@@ -68,6 +69,7 @@ _SIGNATURES = {
     "g2048_play_swar": (_INT, [_INT, _P, _I64, _I64, _I64, _I64, _INT, _P, _P, _P, _P, _P, _P]),
     "g2048_row_table_lookup": (_INT, [_P, _I64, _P, _P, _P]),
     "g2048_playout_values": (_INT, [_INT, _P, _I64, _P, _I64, _I64, _I64, _P, _I64, _INT, _P, _P, _P, _P]),
+    "g2048_expectimax_values": (_INT, [_P, _I64, _INT, _P, _FLT, _P, _P, _P]),
     "g2048_play_host": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),
     "g2048_play_host_packed": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P]),
     "g2048_play_packed": (_INT, [_INT, _P, _I64, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),

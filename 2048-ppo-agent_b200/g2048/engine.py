@@ -318,6 +318,18 @@ def playout_values(policy: int, boards: torch.Tensor, subs: torch.Tensor, playou
                 playouts=last & 0xFFFFFFFF, cut_short=last >> 32, stats=stats)
 
 
+def expectimax_values(boards: torch.Tensor, depth: int, row_values: torch.Tensor, reward_weight: float = 0.0,
+                      counters: torch.Tensor | None = None) -> torch.Tensor:
+    """Depth-``depth`` expectimax values of the given bitboards over the row heuristic ``row_values`` (65 536 float32)
+    (g2048_expectimax_values): (n, 4) float32 Q values, NaN where the action is illegal.  ``counters`` (optional, 2
+    int64) accumulates the number of leaves (heuristic evaluations) and of chance nodes."""
+    assert row_values.dtype == torch.float32 and row_values.numel() == 65536
+    q = torch.empty((boards.shape[0], 4), dtype=torch.float32, device=boards.device)
+    call("g2048_expectimax_values", ptr(boards), boards.shape[0], depth, ptr(row_values), float(reward_weight), ptr(q),
+         ptr(counters), stream_ptr())
+    return q
+
+
 def play_host(policy: int, seed: int, batch_global: int, rng_mode: int, env_lo: int = 0, n: int | None = None,
               key: np.ndarray | None = None, per_env: bool = True, pinned: bool = False):
     """The host-buffer C entry point (numpy in / numpy out; copies and syncs inside the call).

@@ -30,6 +30,8 @@ import torch
 
 from .. import _native as N
 from .. import engine as E
+from ..expectimax import ExpectimaxPolicy
+from ..expectimax import best_actions as expectimax_best_actions
 from ..keys import KeyChain
 from ..playouts import MonteCarloPolicy, best_actions
 from ..state import State
@@ -284,6 +286,8 @@ class BatchRunner:
         fn = self._act_fn
         if isinstance(fn, MonteCarloPolicy):
             return self._run_eval_monte_carlo(batch_size)
+        if isinstance(fn, ExpectimaxPolicy):
+            return self._run_eval_expectimax(batch_size)
         if not hasattr(fn, "forward_logits"):
             raise ValueError("run_eval_batch needs a TorchActionFunction; use run_stats_batch for act_randomly / act_drul")
         lo, n = self._range(batch_size)
@@ -339,9 +343,36 @@ class BatchRunner:
         chunk is still listed until the chunk ends: it has no legal action, so none of its playouts is played, and the
         step leaves a finished env as it is.  The host reads the done count once per NET_SYNC_STEPS steps."""
         fn = self._act_fn
+        mode = self.rng_mode
+        policy, n_subs = fn.rollout_policy, 1 + 2 * int(fn.max_steps)
+
+        def choose(live_boards, board_ids, sub_act):
+            psubs = E.split_keys(sub_act, n_subs, 0, n_subs, mode)
+            rec = E.playout_values(policy, live_boards, psubs, int(fn.playouts), mode, board_ids=board_ids,
+                                   n_boards_global=batch_size)
+            return best_actions(rec, fn.criterion)
+
+        return self._run_eval_search(batch_size, choose)
+
+    def _run_eval_expectimax(self, batch_size: int) -> dict:
+        """run_eval_batch with an ``ExpectimaxPolicy``: per loop step one ``g2048_expectimax_values`` launch over the
+        envs alive at the start of the chunk and the best action per env (an env that finished inside the chunk has no
+        legal action and gets action 0, which the step ignores); the act sub key is not used."""
+        fn = self._act_fn
+        table = fn.table(self.device)
+
+        def choose(live_boards, board_ids, sub_act):
+            return expectimax_best_actions(E.expectimax_values(live_boards, int(fn.depth), table, float(fn.reward_weight)))
+
+        return self._run_eval_search(batch_size, choose)
+
+    def _run_eval_search(self, batch_size: int, choose) -> dict:
+        """The per-move loop of the search players: per loop step t, ``choose(boards of the envs alive at the start of
+        the chunk, their global env ids, act sub key of step t)`` gives their actions, and ``g2048_env_step`` steps
+        every env with the step key of step t (a finished env stays as it is).  The live list is built once per
+        chunk of NET_SYNC_STEPS steps, and the host reads the done count once per chunk."""
         lo, n = self._range(batch_size)
         dev, mode = self.device, self.rng_mode
-        policy, n_subs = fn.rollout_policy, 1 + 2 * int(fn.max_steps)
         boards, status = E.env_init(self.chain.peek(1)[0], batch_size, lo, n, mode)
         lengths = torch.zeros(n, dtype=torch.int32, device=dev)
         scores = torch.zeros(n, dtype=torch.int64, device=dev)
@@ -355,10 +386,7 @@ class BatchRunner:
                 board_ids = live_ids + lo
                 for k in range(steps):
                     t = t0 + k
-                    psubs = E.split_keys(subs[1 + 2 * t], n_subs, 0, n_subs, mode)
-                    rec = E.playout_values(policy, boards[live_ids], psubs, int(fn.playouts), mode, board_ids=board_ids,
-                                           n_boards_global=batch_size)
-                    actions[live_ids] = best_actions(rec, fn.criterion).to(torch.int32)
+                    actions[live_ids] = choose(boards[live_ids], board_ids, subs[1 + 2 * t]).to(torch.int32)
                     alive = (status & N.STATUS_DONE) == 0
                     rewards = E.env_step(boards, status, actions, subs[2 + 2 * t], batch_size, lo, mode)
                     lengths += alive.to(torch.int32)
@@ -388,6 +416,8 @@ class BatchRunner:
             raise ValueError("The action function is not set.")
         if isinstance(self._act_fn, MonteCarloPolicy) and not eval_batch:
             raise ValueError("a MonteCarloPolicy plays through run_eval_batch only (it keeps no records)")
+        if isinstance(self._act_fn, ExpectimaxPolicy) and not eval_batch:
+            raise ValueError("an ExpectimaxPolicy plays through run_eval_batch only (it keeps no records)")
         if not isinstance(batch_size, (int, np.integer)) or batch_size <= 0:
             raise ValueError(f"batch_size must be a positive integer, got {batch_size!r}")
 

@@ -211,6 +211,24 @@ int g2048_playout_values(int policy, const uint64_t* d_boards, int64_t n, const 
                          int64_t n_boards_global, int64_t playouts, const uint32_t* d_subs, int64_t n_subs, int rng_mode,
                          uint64_t* d_work, G2048PlayoutStats* d_records, uint64_t* d_stats, void* stream);
 
+/* ---- Depth-limited expectimax values of caller-given boards over a row heuristic (no pruning, no transposition
+ * table; all arithmetic float32 in exactly this order, so the values are bit-exact):
+ *   H(b)      = T[row0] + T[row1] + T[row2] + T[row3] + T[col0] + T[col1] + T[col2] + T[col3], left to right
+ *               (row r = bits [16r, 16r+16); column c = row c of the transpose: nibble k is cell 4k + c);
+ *   Q_1(b, a) = w * r + H(b_a);  Q_k(b, a) = w * r + C_{k-1}(b_a) for k >= 2, where (b_a, r) = move(b, a), a legal,
+ *               and r = potential(b_a) - potential(b) is the merge reward (no spawn);
+ *   C_k(s)    = acc / (float)n_empty, acc = 0 then acc = acc + (0.9f * V_k(s + 2@c) + 0.1f * V_k(s + 4@c)) for the
+ *               empty cells c of s in increasing index;
+ *   V_k(b)    = max over the legal a of Q_k(b, a); 0 for a board without a legal action.
+ *   d_boards (n): bitboards; n >= 0 (n = 0 is a no-op).  depth = d in 1..4 counts moves.
+ *   d_row_values: T, float[65536] (device).  reward_weight: w.
+ *   d_q (n * 4, 4-byte aligned): OVERWRITTEN with Q_d(board i, a) at 4 i + a, NaN where a is illegal on board i.
+ *   d_counters: NULL, or uint64[2] ACCUMULATED: [0] H evaluations (leaves), [1] chance nodes expanded.  Both depend on
+ *           the tree alone.
+ * A board that holds a 2^15 tile is outside the contract (as for g2048_play). */
+int g2048_expectimax_values(const uint64_t* d_boards, int64_t n, int depth, const float* d_row_values, float reward_weight,
+                            float* d_q, uint64_t* d_counters, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.
