@@ -16,7 +16,7 @@
 // depend on the mapping.  Subtree sizes differ by 100x from board to board, so the warps of a CTA claim items through a
 // shared-memory counter, and the CTAs of the persistent grid take interleaved items (item = blockIdx + k * gridDim):
 // no global scratch and no inter-CTA hand-over.
-#include "g2048_play3.cuh"
+#include "g2048_xm.cuh"
 
 namespace g2048 {
 
@@ -30,47 +30,9 @@ constexpr int XM_SLOTS = 15 * 8;  // an afterstate has at most 15 empty cells: (
 constexpr int XM_VALS = 15 * 2;
 constexpr int XM_SMEM_BYTES = PLAY3_TABLE_BYTES + XM_WARPS * (XM_SLOTS + XM_VALS) * 4;
 
-struct XmCtx {
-    const float* T;
-    float w;
-    const uint16_t* s_left;
-    const uint8_t* s_flags;
-};
-
 struct XmCount {
     unsigned long long leaves, chance;
 };
-
-// A board travels with its transpose bT: columns are rows of the transpose.
-__device__ __forceinline__ float xm_heuristic(const XmCtx& c, u64 b, u64 bT) {
-    const uint32_t lo = (uint32_t)b, hi = (uint32_t)(b >> 32), tlo = (uint32_t)bT, thi = (uint32_t)(bT >> 32);
-    float h = __ldg(&c.T[lo & 0xFFFFu]);
-    h = h + __ldg(&c.T[lo >> 16]);
-    h = h + __ldg(&c.T[hi & 0xFFFFu]);
-    h = h + __ldg(&c.T[hi >> 16]);
-    h = h + __ldg(&c.T[tlo & 0xFFFFu]);
-    h = h + __ldg(&c.T[tlo >> 16]);
-    h = h + __ldg(&c.T[thi & 0xFFFFu]);
-    h = h + __ldg(&c.T[thi >> 16]);
-    return h;
-}
-
-// (nb, nbT) = move(b, a); with REWARD also r = potential(nb) - potential(b), the merge reward
-template <bool REWARD>
-__device__ __forceinline__ void xm_move(const XmCtx& c, u64 b, u64 bT, int a, u64& nb, u64& nbT, uint32_t& r) {
-    const bool vertical = (a & 1) != 0, rev = a >= 2;
-    u64 src = vertical ? bT : b;
-    if (rev) src = mirror_rows(src);
-    const uint32_t slo = (uint32_t)src, shi = (uint32_t)(src >> 32);
-    const uint32_t m0 = c.s_left[slo & 0xFFFFu], m1 = c.s_left[slo >> 16];
-    const uint32_t m2 = c.s_left[shi & 0xFFFFu], m3 = c.s_left[shi >> 16];
-    u64 moved = ((u64)(m2 | (m3 << 16)) << 32) | (u64)(m0 | (m1 << 16));
-    if (rev) moved = mirror_rows(moved);
-    const u64 movedT = transpose_board(moved);
-    nb = vertical ? movedT : moved;
-    nbT = vertical ? moved : movedT;
-    if (REWARD) r = board_potential(nb) - board_potential(b);
-}
 
 template <int K, bool REWARD>
 __device__ __forceinline__ float xm_chance(const XmCtx& c, u64 s, u64 sT, XmCount& n);

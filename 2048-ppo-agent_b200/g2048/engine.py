@@ -330,6 +330,25 @@ def expectimax_values(boards: torch.Tensor, depth: int, row_values: torch.Tensor
     return q
 
 
+def td_scratch(device) -> torch.Tensor:
+    """Zeroed scratch of g2048_td_train (every call leaves it zeroed, so one serves a whole training run)."""
+    return torch.zeros(int(N.lib.g2048_td_scratch_bytes()) // 8, dtype=torch.int64, device=device)
+
+
+def td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+             row_values: torch.Tensor, alpha: float, subs: torch.Tensor, rng_mode: int, scratch: torch.Tensor,
+             stats: torch.Tensor | None = None) -> None:
+    """``subs.shape[0]`` synchronous TD(0) steps of the row table (g2048_td_train), in place on the env state (boards /
+    after int64, scores / lengths int32, n of each) and on ``row_values`` (65 536 float32).  ``scratch``: from
+    ``td_scratch``.  ``stats`` (optional, 32 int64) accumulates the finished episodes in g2048_play's layout."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert row_values.dtype == torch.float32 and row_values.numel() == 65536
+    call("g2048_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, ptr(row_values), float(alpha),
+         ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
+
+
 def play_host(policy: int, seed: int, batch_global: int, rng_mode: int, env_lo: int = 0, n: int | None = None,
               key: np.ndarray | None = None, per_env: bool = True, pinned: bool = False):
     """The host-buffer C entry point (numpy in / numpy out; copies and syncs inside the call).

@@ -229,6 +229,39 @@ int g2048_playout_values(int policy, const uint64_t* d_boards, int64_t n, const 
 int g2048_expectimax_values(const uint64_t* d_boards, int64_t n, int depth, const float* d_row_values, float reward_weight,
                             float* d_q, uint64_t* d_counters, void* stream);
 
+/* ---- Batched TD(0) afterstate learning of the row table T that g2048_expectimax_values reads (H as above).
+ * Synchronous: every env of a step reads the same frozen T_t, the TD errors are summed in fixed point with integer
+ * atomics, and T_{t+1} is applied after the whole batch has made the step -- so the result is bit-exact and does not
+ * depend on how the work is spread over the GPU.
+ * State of env e < n: d_boards (uint64), d_after (uint64: the previous afterstate, 0 = none -- no afterstate is the
+ * empty board), d_scores and d_lengths (uint32).  Step t uses k = split(d_subs[t], n)[e] and does for every env:
+ *   1. s = board.  If s has a legal action: q_a = (float)r_a + H_t(s_a) for each legal a in action order,
+ *      (s_a, r_a) = move(s, a); a* = the first legal action, replaced by every strictly larger q; target = q_{a*}
+ *      (Q_1 of g2048_expectimax_values with w = 1, the same tie rule).  Without a legal action target = 0.
+ *   2. If after != 0: delta = target - H_t(after) (float32, no contraction); for each of the 8 lines of after in H's
+ *      order acc[idx] += fx(delta) and cnt[idx] += 1, where fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64,
+ *      rounded to nearest even (clamp(d, lo, hi) = fminf(fmaxf(d, lo), hi)).
+ *   3. Without a legal action the episode ends: it is counted in d_stats, board = init(k) (g2048_env_init with the
+ *      explicit key k) and after = score = length = 0; the env makes no move this step.  Otherwise
+ *      board = step(s, a*, k) (g2048_env_step: the same spawn draws), after = s_{a*}, score += r_{a*}, length += 1.
+ *   4. After all envs: for every i with cnt[i] > 0, T[i] = T[i] + alpha * (float)((double)acc[i] / (4096.0 *
+ *      (double)cnt[i])) (float multiply and add, not fused); then acc[i] = cnt[i] = 0.  The per-entry mean makes the
+ *      learning rate independent of the batch size and of how common a row is: a row seen once gets alpha * delta.
+ *   d_row_values: T, float[65536], updated in place.  d_subs: n_steps sub keys (n_steps >= 0; 0 is a no-op).
+ *   d_scratch: g2048_td_scratch_bytes() bytes (acc int64[65536], then cnt uint32[65536]), zeroed by the caller once;
+ *           every call leaves it zeroed.
+ *   d_stats: NULL, or uint64[G2048_PLAY_STATS_WORDS] ACCUMULATED in g2048_play's layout over the episodes that end
+ *           in the call: [0] episodes, [1] their moves, [2] their scores, [4] those whose final board holds a 2^15
+ *           tile, [5] longest, [6] / [7] sum of max tile / its square, [16 + e] episodes whose max tile is 2^e.
+ * G2048_ERR_INVALID for n outside [1, 2^20], n_steps < 0, a negative or non-finite alpha, NULL or misaligned
+ * pointers (8 bytes for boards, after, subs, scratch and stats; 4 for the others).  The launch is cooperative: it
+ * fails with an error, rather than waiting, if its grid cannot be resident at once.  A board that holds a 2^15 tile
+ * is outside the contract (as for g2048_play). */
+int64_t g2048_td_scratch_bytes(void);
+int g2048_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths, int64_t n,
+                   float* d_row_values, float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
+                   void* d_scratch, uint64_t* d_stats, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.
