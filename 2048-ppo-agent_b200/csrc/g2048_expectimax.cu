@@ -16,6 +16,7 @@
 // depend on the mapping.  Subtree sizes differ by 100x from board to board, so the warps of a CTA claim items through a
 // shared-memory counter, and the CTAs of the persistent grid take interleaved items (item = blockIdx + k * gridDim):
 // no global scratch and no inter-CTA hand-over.
+#include "g2048_ntuple.cuh"
 #include "g2048_xm.cuh"
 
 namespace g2048 {
@@ -34,35 +35,35 @@ struct XmCount {
     unsigned long long leaves, chance;
 };
 
-template <int K, bool REWARD>
-__device__ __forceinline__ float xm_chance(const XmCtx& c, u64 s, u64 sT, XmCount& n);
+template <int K, bool REWARD, class Leaf>
+__device__ __forceinline__ float xm_chance(const XmCtx& c, const typename Leaf::Param& leaf, u64 s, u64 sT, XmCount& n);
 
 // Q_K(b, a) for a legal a
-template <int K, bool REWARD>
-__device__ __forceinline__ float xm_q(const XmCtx& c, u64 b, u64 bT, int a, XmCount& n) {
+template <int K, bool REWARD, class Leaf>
+__device__ __forceinline__ float xm_q(const XmCtx& c, const typename Leaf::Param& leaf, u64 b, u64 bT, int a, XmCount& n) {
     u64 nb, nbT;
     uint32_t r;
     xm_move<REWARD>(c, b, bT, a, nb, nbT, r);
     float tail;
     if constexpr (K == 1) {
         ++n.leaves;
-        tail = xm_heuristic(c, nb, nbT);
+        tail = Leaf::value(c, leaf, nb, nbT);
     } else {
-        tail = xm_chance<K - 1, REWARD>(c, nb, nbT, n);
+        tail = xm_chance<K - 1, REWARD, Leaf>(c, leaf, nb, nbT, n);
     }
     // w r with r = 0 when w == 0: w * r = w exactly (w = +0 or -0, r >= 0), so the reward-free form adds w itself
     return (REWARD ? c.w * (float)r : c.w) + tail;
 }
 
-template <int K, bool REWARD>
-__device__ __forceinline__ float xm_value(const XmCtx& c, u64 b, u64 bT, XmCount& n) {
+template <int K, bool REWARD, class Leaf>
+__device__ __forceinline__ float xm_value(const XmCtx& c, const typename Leaf::Param& leaf, u64 b, u64 bT, XmCount& n) {
     const uint32_t lm = play3_legal(c.s_flags, b, bT);
     float v = 0.0f;
     bool any = false;
 #pragma unroll 1
     for (int a = 0; a < 4; ++a) {
         if ((lm >> a) & 1u) {
-            const float q = xm_q<K, REWARD>(c, b, bT, a, n);
+            const float q = xm_q<K, REWARD, Leaf>(c, leaf, b, bT, a, n);
             if (!any || q > v) v = q;
             any = true;
         }
@@ -77,8 +78,8 @@ __device__ __forceinline__ void xm_spawn(u64 s, u64 sT, int p, uint32_t v, u64& 
     childT = sT + ((u64)v << (4 * cellT));
 }
 
-template <int K, bool REWARD>
-__device__ __forceinline__ float xm_chance(const XmCtx& c, u64 s, u64 sT, XmCount& n) {
+template <int K, bool REWARD, class Leaf>
+__device__ __forceinline__ float xm_chance(const XmCtx& c, const typename Leaf::Param& leaf, u64 s, u64 sT, XmCount& n) {
     ++n.chance;
     u64 e = ~nonzero_lsb(s) & NIB_LSB;
     const int ne = __popcll(e);
@@ -89,18 +90,34 @@ __device__ __forceinline__ float xm_chance(const XmCtx& c, u64 s, u64 sT, XmCoun
         e &= e - 1;
         u64 ch, chT;
         xm_spawn(s, sT, p, 1u, ch, chT);
-        const float v2 = xm_value<K, REWARD>(c, ch, chT, n);
+        const float v2 = xm_value<K, REWARD, Leaf>(c, leaf, ch, chT, n);
         xm_spawn(s, sT, p, 2u, ch, chT);
-        const float v4 = xm_value<K, REWARD>(c, ch, chT, n);
+        const float v4 = xm_value<K, REWARD, Leaf>(c, leaf, ch, chT, n);
         acc = acc + (0.9f * v2 + 0.1f * v4);
     }
     return acc / (float)ne;
 }
 
+// The leaf of the search, a template parameter of the kernel.  Leaf::Param is the kernel parameter that carries it:
+// the table T of the row heuristic H (g2048_expectimax_values), which the kernel puts into the search context ...
+struct XmRowLeaf {
+    using Param = const float* __restrict__;
+    static __device__ __forceinline__ const float* table(const Param& T) { return T; }
+    static __device__ __forceinline__ float value(const XmCtx& c, const Param&, u64 b, u64 bT) { return xm_heuristic(c, b, bT); }
+};
+
+// ... or an n-tuple network (g2048_expectimax_values_ntuple): V at the leaves, its placements read from the parameter's
+// constant bank
+struct XmTupleLeaf {
+    using Param = NtNet;
+    static __device__ __forceinline__ const float* table(const Param&) { return nullptr; }
+    static __device__ __forceinline__ float value(const XmCtx&, const Param& net, u64 b, u64) { return nt_value<false>(net, b); }
+};
+
 // Item j < n * 4 is (board j / 4, first action j % 4), one warp each.
-template <int DEPTH, bool REWARD>
+template <int DEPTH, bool REWARD, class Leaf>
 __global__ void __launch_bounds__(XM_THREADS, 1)
-expectimax_kernel(const u64* __restrict__ boards, uint32_t n_items, const float* __restrict__ T, float w,
+expectimax_kernel(const u64* __restrict__ boards, uint32_t n_items, const typename Leaf::Param leaf, float w,
                   float* __restrict__ q_out, unsigned long long* __restrict__ counters) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     __shared__ unsigned s_next;
@@ -112,7 +129,7 @@ expectimax_kernel(const u64* __restrict__ boards, uint32_t n_items, const float*
     float* slots = reinterpret_cast<float*>(smem_raw + PLAY3_TABLE_BYTES) + warp * (XM_SLOTS + XM_VALS);
     float* vals = slots + XM_SLOTS;
     XmCtx c;
-    c.T = T;
+    c.T = Leaf::table(leaf);
     c.w = w;
     c.s_left = reinterpret_cast<const uint16_t*>(smem_raw);
     c.s_flags = smem_raw + 65536 * 2;
@@ -132,7 +149,7 @@ expectimax_kernel(const u64* __restrict__ boards, uint32_t n_items, const float*
             continue;
         }
         if constexpr (DEPTH == 1) {
-            if (lane == 0) q_out[item] = xm_q<1, REWARD>(c, b, bT, a0, n);
+            if (lane == 0) q_out[item] = xm_q<1, REWARD, Leaf>(c, leaf, b, bT, a0, n);
             continue;
         } else {
             u64 s, sT;
@@ -147,7 +164,7 @@ expectimax_kernel(const u64* __restrict__ boards, uint32_t n_items, const float*
                 xm_spawn(s, sT, p, 1u + ((j >> 2) & 1u), ch, chT);
                 const int a1 = j & 3;
                 slots[j] = ((play3_legal(c.s_flags, ch, chT) >> a1) & 1u)
-                               ? xm_q<DEPTH - 1, REWARD>(c, ch, chT, a1, n)
+                               ? xm_q<DEPTH - 1, REWARD, Leaf>(c, leaf, ch, chT, a1, n)
                                : __int_as_float(0x7FC00000);  // NaN: a1 illegal
             }
             __syncwarp();
@@ -196,10 +213,10 @@ __global__ void build_expectimax_row_tables_kernel() {
     build_row_table_entry(row);
 }
 
-template <int DEPTH, bool REWARD>
-static int launch_expectimax(const uint64_t* d_boards, int64_t n_items, const float* d_T, float w, float* d_q,
+template <int DEPTH, bool REWARD, class Leaf>
+static int launch_expectimax(const uint64_t* d_boards, int64_t n_items, const typename Leaf::Param& leaf, float w, float* d_q,
                              uint64_t* d_counters, cudaStream_t st) {
-    auto kernel = expectimax_kernel<DEPTH, REWARD>;
+    auto kernel = expectimax_kernel<DEPTH, REWARD, Leaf>;
     static bool configured_on[64] = {false};
     bool* configured = device_once_flag(configured_on);
     if (!configured) return fail_arg("no CUDA device");
@@ -215,20 +232,29 @@ static int launch_expectimax(const uint64_t* d_boards, int64_t n_items, const fl
     if (sms <= 0) return fail_arg("expectimax_values: no device");
     const int64_t needed = (n_items + XM_WARPS - 1) / XM_WARPS;
     const int64_t grid = needed < sms ? needed : sms;  // one CTA per SM, persistent
-    kernel<<<(unsigned)grid, XM_THREADS, XM_SMEM_BYTES, st>>>((const u64*)d_boards, (uint32_t)n_items, d_T, w, d_q,
+    kernel<<<(unsigned)grid, XM_THREADS, XM_SMEM_BYTES, st>>>((const u64*)d_boards, (uint32_t)n_items, leaf, w, d_q,
                                                              (unsigned long long*)d_counters);
     return check_cuda(cudaGetLastError(), "expectimax_values");
 }
 
-template <bool REWARD>
-static int launch_expectimax_depth(int depth, const uint64_t* d_boards, int64_t n_items, const float* d_T, float w,
+template <bool REWARD, class Leaf>
+static int launch_expectimax_depth(int depth, const uint64_t* d_boards, int64_t n_items, const typename Leaf::Param& leaf, float w,
                                    float* d_q, uint64_t* d_counters, cudaStream_t st) {
     switch (depth) {
-        case 1: return launch_expectimax<1, REWARD>(d_boards, n_items, d_T, w, d_q, d_counters, st);
-        case 2: return launch_expectimax<2, REWARD>(d_boards, n_items, d_T, w, d_q, d_counters, st);
-        case 3: return launch_expectimax<3, REWARD>(d_boards, n_items, d_T, w, d_q, d_counters, st);
-        default: return launch_expectimax<4, REWARD>(d_boards, n_items, d_T, w, d_q, d_counters, st);
+        case 1: return launch_expectimax<1, REWARD, Leaf>(d_boards, n_items, leaf, w, d_q, d_counters, st);
+        case 2: return launch_expectimax<2, REWARD, Leaf>(d_boards, n_items, leaf, w, d_q, d_counters, st);
+        case 3: return launch_expectimax<3, REWARD, Leaf>(d_boards, n_items, leaf, w, d_q, d_counters, st);
+        default: return launch_expectimax<4, REWARD, Leaf>(d_boards, n_items, leaf, w, d_q, d_counters, st);
     }
+}
+
+// the reward-free form when w == 0 (+0 or -0): no merge reward to compute
+template <class Leaf>
+static int launch_expectimax_leaf(int depth, const uint64_t* d_boards, int64_t n, const typename Leaf::Param& leaf, float w, float* d_q,
+                                  uint64_t* d_counters, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    if (w == 0.0f) return launch_expectimax_depth<false, Leaf>(depth, d_boards, n * 4, leaf, w, d_q, d_counters, st);
+    return launch_expectimax_depth<true, Leaf>(depth, d_boards, n * 4, leaf, w, d_q, d_counters, st);
 }
 
 }  // namespace g2048
@@ -242,8 +268,22 @@ extern "C" int g2048_expectimax_values(const uint64_t* d_boards, int64_t n, int 
     G2048_REQUIRE(((uintptr_t)d_q & 3u) == 0, "expectimax_values: d_q must be 4-byte aligned");
     if (n == 0) return G2048_OK;
     G2048_REQUIRE(d_boards && d_row_values && d_q, "expectimax_values: pointers");
-    cudaStream_t st = (cudaStream_t)stream;
-    // the reward-free form when w == 0 (+0 or -0): no merge reward to compute
-    if (reward_weight == 0.0f) return launch_expectimax_depth<false>(depth, d_boards, n * 4, d_row_values, reward_weight, d_q, d_counters, st);
-    return launch_expectimax_depth<true>(depth, d_boards, n * 4, d_row_values, reward_weight, d_q, d_counters, st);
+    return launch_expectimax_leaf<XmRowLeaf>(depth, d_boards, n, d_row_values, reward_weight, d_q, d_counters, stream);
+}
+
+extern "C" int g2048_expectimax_values_ntuple(const uint64_t* d_boards, int64_t n, int depth,
+                                              const G2048TuplePlacement* h_placements, int n_placements,
+                                              const float* d_weights, int64_t n_weights, float reward_weight,
+                                              float* d_q, uint64_t* d_counters, void* stream) {
+    G2048_REQUIRE(depth >= 1 && depth <= 4, "expectimax_values_ntuple: depth must be in 1..4");
+    G2048_REQUIRE(n >= 0 && n < (1ll << 29), "expectimax_values_ntuple: n must be in [0, 2^29)");
+    G2048_REQUIRE(((uintptr_t)d_q & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0,
+                  "expectimax_values_ntuple: d_q and d_weights must be 4-byte aligned");
+    const int rc = ntuple_check(h_placements, n_placements, n_weights, "expectimax_values_ntuple: invalid network");
+    if (rc) return rc;
+    if (n == 0) return G2048_OK;
+    G2048_REQUIRE(d_boards && d_weights && d_q, "expectimax_values_ntuple: pointers");
+    NtNet net;
+    ntuple_net(net, h_placements, n_placements, d_weights);
+    return launch_expectimax_leaf<XmTupleLeaf>(depth, d_boards, n, net, reward_weight, d_q, d_counters, stream);
 }

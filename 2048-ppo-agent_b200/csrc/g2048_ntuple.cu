@@ -1,0 +1,375 @@
+// Batched TD(0) afterstate learning of an n-tuple network (g2048_ntuple_td_train, include/g2048.h).
+//
+// Step t, for every env e < n with its key k = split(subs[t], n)[e]:
+//   greedy move over q_a = (float)r_a + V_t(s_a) (Q_1 of g2048_expectimax_values_ntuple with w = 1, same tie rule);
+//   if the env holds an afterstate: fx(target - V_t(after)) into acc[i] and 1 into cnt[i] for i = off_p + idx_p(after),
+//   every placement p in order; then a finished episode restarts from init(k), anything else moves and spawns with k.
+// After the whole batch: W[i] += alpha * mean of the fixed-point errors of entry i, and acc / cnt go back to zero.
+//
+// Mapping: the accumulate / grid.sync() / apply / grid.sync() structure of td_train_kernel (g2048_td.cu), one
+// cooperative persistent launch for all the steps.  What differs is the size of W: the 4x6 network has 2^26 weights,
+// so the apply phase cannot sweep the sums as the row learner does (12 bytes an entry, ~0.8 GB a step).  Instead the
+// accumulate phase lists the entries it touches: the atomicAdd on cnt[i] that returns 0 is the entry's first touch of
+// the step, and that lane appends i to a list (one list atomic per warp and placement).  The apply phase walks the
+// list, so its cost follows the entries touched, not n_weights.  The new value of an entry depends only on its integer
+// (sum, count), so neither the grid, the order of the atomics nor the order of the list changes a bit.
+//
+// V evaluations: the 4 candidate afterstates and the previous afterstate are evaluated together (nt_values), so 5
+// gathers per placement are in flight at once; an illegal action's board is the unmoved board, whose value is unused.
+//
+// Hot entries: early boards give most placements index 0 (all cells empty).  Each entry is first aggregated in the warp
+// (__match_any_sync: the group's leader adds the group's sum), and index 0 of every placement is further summed per CTA
+// in shared memory, with one global atomic per CTA, placement and step.
+#include <cooperative_groups.h>
+
+#include "g2048_ntuple.cuh"
+#include "g2048_xm.cuh"
+
+namespace g2048 {
+
+namespace cg = cooperative_groups;
+
+// G2048_NTUPLE_PHASES (A/B builds only: make OUT=... BUILD=... EXTRA=-DG2048_NTUPLE_PHASES, as tools/bench_ntuple.py
+// does) makes CTA 0 time both phases of every step with %globaltimer, each up to the grid.sync() that ends it, and
+// ADD to d_stats[8] the accumulate nanoseconds, [9] the apply nanoseconds and [10] the entries listed (words the
+// statistics layout leaves unused).  The default build has none of it.
+#ifdef G2048_NTUPLE_PHASES
+__device__ __forceinline__ unsigned long long nt_clock() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+#endif
+
+constexpr int NT_THREADS = 512;
+constexpr int NT_SMEM_BYTES = PLAY3_TABLE_BYTES;  // the row tables; the small arrays below are static
+constexpr float NT_FX_CLAMP = 16777216.0f;        // 2^24: 2^20 envs * 64 placements * 2^24 * 4096 = 2^62
+constexpr float NT_FX_ONE = 4096.0f;
+
+// scratch: acc int64[n_weights], cnt uint32[n_weights], list uint32[min(n * P, n_weights)], then list_len uint32[2]
+struct NtScratch {
+    int64_t cnt_off, list_off, len_off, bytes;
+};
+
+static NtScratch nt_scratch_layout(int64_t n, int n_placements, int64_t n_weights) {
+    const int64_t touched = n * n_placements < n_weights ? n * n_placements : n_weights;
+    NtScratch s;
+    s.cnt_off = 8 * n_weights;
+    s.list_off = s.cnt_off + 4 * n_weights;
+    s.len_off = (s.list_off + 4 * touched + 7) & ~7ll;
+    s.bytes = s.len_off + 8;
+    return s;
+}
+
+struct NtTdArgs {
+    u64* boards;
+    u64* after;
+    uint32_t* scores;
+    uint32_t* lengths;
+    uint32_t n;
+    float* W;
+    float alpha;
+    const uint2* subs;
+    int64_t n_steps;
+    unsigned long long* acc;
+    uint32_t* cnt;
+    uint32_t* list;
+    uint32_t* list_len;  // [2]: step t appends through list_len[t & 1]
+    unsigned long long* stats;
+    NtNet net;  // net.W == W
+};
+
+// fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64, to nearest even (the multiply by a power of two is exact)
+__device__ __forceinline__ long long nt_fx(float d) {
+    return __float2ll_rn(fminf(fmaxf(d, -NT_FX_CLAMP), NT_FX_CLAMP) * NT_FX_ONE);
+}
+
+// the lanes with `first` append their entry i to the list: one list atomic per warp (all 32 lanes call this)
+__device__ __forceinline__ void nt_append(bool first, uint32_t i, uint32_t* list, uint32_t* list_len, unsigned lane) {
+    const unsigned firsts = __ballot_sync(0xFFFFFFFFu, first);
+    if (firsts) {
+        uint32_t pos = 0u;
+        if (lane == 0u) pos = atomicAdd(list_len, (uint32_t)__popc((int)firsts));
+        pos = __shfl_sync(0xFFFFFFFFu, pos, 0);
+        if (first) list[pos + (uint32_t)__popc((int)(firsts & ((1u << lane) - 1u)))] = i;
+    }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_constant__ NtTdArgs a) {
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    __shared__ unsigned long long s_stats[G2048_PLAY_STATS_WORDS];
+    __shared__ long long s_fx[NT_THREADS];
+    __shared__ unsigned long long s_acc0[G2048_NTUPLE_MAX_PLACEMENTS];
+    __shared__ unsigned s_cnt0[G2048_NTUPLE_MAX_PLACEMENTS];
+    play3_copy_row_tables<NT_THREADS>(smem_raw);
+    for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += NT_THREADS) s_stats[i] = 0ull;
+    if (threadIdx.x < G2048_NTUPLE_MAX_PLACEMENTS) {
+        s_acc0[threadIdx.x] = 0ull;
+        s_cnt0[threadIdx.x] = 0u;
+    }
+    __syncthreads();
+
+    cg::grid_group grid = cg::this_grid();
+    XmCtx c;
+    c.T = nullptr;
+    c.w = 1.0f;
+    c.s_left = reinterpret_cast<const uint16_t*>(smem_raw);
+    c.s_flags = smem_raw + 65536 * 2;
+    const unsigned lane = threadIdx.x & 31u;
+    long long* warp_fx = s_fx + (threadIdx.x & ~31u);
+    const uint32_t stride = gridDim.x * NT_THREADS;
+    const uint32_t P = a.net.n_placements;
+#ifdef G2048_NTUPLE_PHASES
+    unsigned long long t_mark = nt_clock(), ns_acc = 0ull, ns_apply = 0ull, listed = 0ull;
+#endif
+
+    for (int64_t t = 0; t < a.n_steps; ++t) {
+        const uint2 sub = __ldg(&a.subs[t]);
+        uint32_t* list_len = a.list_len + (t & 1);
+        // ---- accumulate: the whole CTA walks the envs together, so every warp is converged at the matches
+        for (uint32_t base = blockIdx.x * NT_THREADS; base < a.n; base += stride) {
+            const uint32_t e = base + threadIdx.x;
+            const bool active = e < a.n;
+            u64 s = 0ull, aft = 0ull;
+            uint32_t score = 0u, length = 0u;
+            if (active) {
+                s = a.boards[e];
+                aft = a.after[e];
+                score = a.scores[e];
+                length = a.lengths[e];
+            }
+            const u64 sT = transpose_board(s);
+            const uint32_t lm = active ? play3_legal(c.s_flags, s, sT) : 0u;
+            u64 cand[5];
+            uint32_t rew[4];
+#pragma unroll
+            for (int act = 0; act < 4; ++act) {
+                u64 nbT;
+                xm_move<true>(c, s, sT, act, cand[act], nbT, rew[act]);
+            }
+            cand[4] = aft;
+            float v[5];
+            nt_values<true, 5>(a.net, cand, v);
+            float target = 0.0f;
+            u64 best = 0ull;
+            uint32_t best_r = 0u;
+            bool any = false;
+#pragma unroll
+            for (int act = 0; act < 4; ++act) {
+                if ((lm >> act) & 1u) {
+                    const float q = (float)rew[act] + v[act];
+                    if (!any || q > target) {
+                        target = q;
+                        best = cand[act];
+                        best_r = rew[act];
+                    }
+                    any = true;
+                }
+            }
+            const bool update = aft != 0ull;  // inactive lanes hold after = 0
+            warp_fx[lane] = update ? nt_fx(target - v[4]) : 0ll;
+            __syncwarp();
+#pragma unroll 1
+            for (uint32_t p = 0; p < P; ++p) {
+                const uint32_t i = nt_entry(a.net.pl[p], aft);
+                const unsigned group = __match_any_sync(0xFFFFFFFFu, update ? i : 0xFFFFFFFFu);  // i < 2^28
+                bool first = false;
+                if (update && lane == (unsigned)(__ffs((int)group) - 1)) {
+                    long long sum = 0;
+                    for (unsigned m = group; m; m &= m - 1u) sum += warp_fx[__ffs((int)m) - 1];
+                    const unsigned count = (unsigned)__popc((int)group);
+                    if (i == a.net.pl[p].offset) {
+                        atomicAdd(&s_acc0[p], (unsigned long long)sum);
+                        atomicAdd(&s_cnt0[p], count);
+                    } else {
+                        atomicAdd(&a.acc[i], (unsigned long long)sum);
+                        first = atomicAdd(&a.cnt[i], count) == 0u;
+                    }
+                }
+                nt_append(first, i, a.list, list_len, lane);
+            }
+            __syncwarp();  // warp_fx is rewritten by the next env
+
+            if (active) {
+                const Key k = split_at<MODE>(Key{sub.x, sub.y}, a.n, e);
+                if (lm == 0u) {  // the episode ends here: count it and start the next one
+                    const uint32_t me = max_exponent(s);
+                    const unsigned long long tile = 1ull << me;
+                    atomicAdd(&s_stats[0], 1ull);
+                    atomicAdd(&s_stats[1], (unsigned long long)length);
+                    atomicAdd(&s_stats[2], (unsigned long long)score);
+                    if (has_max_nibble(s)) atomicAdd(&s_stats[4], 1ull);
+                    atomicMax(&s_stats[5], (unsigned long long)length);
+                    atomicAdd(&s_stats[6], tile);
+                    atomicAdd(&s_stats[7], tile * tile);
+                    atomicAdd(&s_stats[16 + me], 1ull);
+                    a.boards[e] = env_init<MODE>(k).board;
+                    a.after[e] = 0ull;
+                    a.scores[e] = 0u;
+                    a.lengths[e] = 0u;
+                } else {
+                    Key k1, k2;
+                    split2<MODE>(k, k1, k2);
+                    a.boards[e] = spawn_tile(best, bits_scalar<MODE>(k1), bits_scalar<MODE>(k2));
+                    a.after[e] = best;
+                    a.scores[e] = score + best_r;
+                    a.lengths[e] = length + 1u;
+                }
+            }
+        }
+        __syncthreads();
+        if (threadIdx.x < P && s_cnt0[threadIdx.x]) {  // the CTA's index-0 sums, one placement per thread
+            const uint32_t i = a.net.pl[threadIdx.x].offset;
+            atomicAdd(&a.acc[i], s_acc0[threadIdx.x]);
+            if (atomicAdd(&a.cnt[i], s_cnt0[threadIdx.x]) == 0u) a.list[atomicAdd(list_len, 1u)] = i;
+            s_acc0[threadIdx.x] = 0ull;
+            s_cnt0[threadIdx.x] = 0u;
+        }
+        grid.sync();
+#ifdef G2048_NTUPLE_PHASES
+        {
+            const unsigned long long now = nt_clock();
+            ns_acc += now - t_mark;
+            t_mark = now;
+            listed += __ldcg(list_len);
+        }
+#endif
+        // ---- apply: every listed entry moves by alpha times the mean of its errors; its sums and its list slot go
+        // back to zero, and the other list's length is cleared for the next step
+        const uint32_t len = __ldcg(list_len);
+        for (uint32_t j = blockIdx.x * NT_THREADS + threadIdx.x; j < len; j += stride) {
+            const uint32_t i = __ldcg(&a.list[j]);
+            const uint32_t count = __ldcg(&a.cnt[i]);
+            const long long sum = (long long)__ldcg(&a.acc[i]);
+            const float mean = (float)((double)sum / (4096.0 * (double)count));
+            a.W[i] = a.W[i] + a.alpha * mean;
+            a.acc[i] = 0ull;
+            a.cnt[i] = 0u;
+            a.list[j] = 0u;
+        }
+        if (blockIdx.x == 0 && threadIdx.x == 0) a.list_len[(t + 1) & 1] = 0u;
+        grid.sync();
+#ifdef G2048_NTUPLE_PHASES
+        {
+            const unsigned long long now = nt_clock();
+            ns_apply += now - t_mark;
+            t_mark = now;
+        }
+#endif
+    }
+#ifdef G2048_NTUPLE_PHASES
+    if (blockIdx.x == 0 && threadIdx.x == 0 && a.stats) {
+        atomicAdd(&a.stats[8], ns_acc);
+        atomicAdd(&a.stats[9], ns_apply);
+        atomicAdd(&a.stats[10], listed);
+    }
+#endif
+    if (blockIdx.x == 0 && threadIdx.x == 0 && a.n_steps > 0) a.list_len[(a.n_steps - 1) & 1] = 0u;
+
+    if (a.stats) {
+        __syncthreads();
+        for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += NT_THREADS) {
+            const unsigned long long v = s_stats[i];
+            if (v) {
+                if (i == 5) atomicMax(&a.stats[i], v);
+                else atomicAdd(&a.stats[i], v);
+            }
+        }
+    }
+}
+
+// this translation unit's copy of the row tables
+__global__ void build_ntuple_row_tables_kernel() {
+    const uint32_t row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= 65536u) return;
+    build_row_table_entry(row);
+}
+
+template <int MODE>
+static int launch_ntuple_td(const NtTdArgs& args, cudaStream_t st) {
+    auto kernel = ntuple_td_kernel<MODE>;
+    static bool configured_on[64] = {false};
+    bool* configured = device_once_flag(configured_on);
+    if (!configured) return fail_arg("no CUDA device");
+    int dev = 0;
+    int rc = check_cuda(cudaGetDevice(&dev), "ntuple_td_train: device");
+    if (rc) return rc;
+    if (!*configured) {
+        int coop = 0;
+        rc = check_cuda(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev),
+                        "ntuple_td_train: device attribute");
+        if (rc) return rc;
+        if (!coop) return fail_arg("ntuple_td_train: the device does not support cooperative launches");
+        rc = check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, NT_SMEM_BYTES),
+                        "ntuple_td_train: shared memory attribute");
+        if (rc) return rc;
+        *configured = true;
+    }
+    rc = ensure_row_tables_with<build_ntuple_row_tables_kernel>(st);
+    if (rc) return rc;
+    int per_sm = 0;
+    rc = check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT_THREADS, NT_SMEM_BYTES),
+                    "ntuple_td_train: occupancy");
+    if (rc) return rc;
+    const int sms = sm_count();
+    if (sms <= 0 || per_sm <= 0) return fail_arg("ntuple_td_train: the kernel does not fit on this device");
+    const int64_t needed = ((int64_t)args.n + NT_THREADS - 1) / NT_THREADS;
+    const int64_t resident = (int64_t)per_sm * sms;
+    const unsigned grid = (unsigned)(needed < resident ? needed : resident);
+    void* params[] = {const_cast<NtTdArgs*>(&args)};
+    return check_cuda(cudaLaunchCooperativeKernel((const void*)kernel, dim3(grid), dim3(NT_THREADS), params,
+                                                  (size_t)NT_SMEM_BYTES, st),
+                      "ntuple_td_train");
+}
+
+}  // namespace g2048
+
+using namespace g2048;
+
+extern "C" int64_t g2048_ntuple_td_scratch_bytes(int64_t n, int n_placements, int64_t n_weights) {
+    if (n < 1 || n > (1ll << 20) || n_placements < 1 || n_placements > G2048_NTUPLE_MAX_PLACEMENTS || n_weights < 1 ||
+        n_weights > G2048_NTUPLE_MAX_WEIGHTS)
+        return -1;
+    return nt_scratch_layout(n, n_placements, n_weights).bytes;
+}
+
+extern "C" int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                     int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                     float* d_weights, int64_t n_weights, float alpha, const uint32_t* d_subs,
+                                     int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+    G2048_REQUIRE(n >= 1 && n <= (1ll << 20), "ntuple_td_train: n must be in [1, 2^20]");
+    G2048_REQUIRE(n_steps >= 0, "ntuple_td_train: n_steps must be >= 0");
+    G2048_REQUIRE(alpha >= 0.0f && alpha <= 3.402823466e38f, "ntuple_td_train: alpha must be finite and >= 0");
+    G2048_REQUIRE(rng_mode == G2048_RNG_ORIGINAL || rng_mode == G2048_RNG_PARTITIONABLE, "ntuple_td_train: rng_mode");
+    int rc = ntuple_check(h_placements, n_placements, n_weights, "ntuple_td_train: invalid network");
+    if (rc) return rc;
+    G2048_REQUIRE(d_boards && d_after && d_scores && d_lengths && d_weights && d_scratch, "ntuple_td_train: pointers");
+    G2048_REQUIRE(n_steps == 0 || d_subs, "ntuple_td_train: pointers");
+    G2048_REQUIRE(((uintptr_t)d_boards & 7u) == 0 && ((uintptr_t)d_after & 7u) == 0 && ((uintptr_t)d_scratch & 7u) == 0 &&
+                      ((uintptr_t)d_subs & 7u) == 0 && ((uintptr_t)d_stats & 7u) == 0,
+                  "ntuple_td_train: d_boards, d_after, d_subs, d_scratch and d_stats must be 8-byte aligned");
+    G2048_REQUIRE(((uintptr_t)d_scores & 3u) == 0 && ((uintptr_t)d_lengths & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0,
+                  "ntuple_td_train: d_scores, d_lengths and d_weights must be 4-byte aligned");
+    if (n_steps == 0) return G2048_OK;
+    const NtScratch lay = nt_scratch_layout(n, n_placements, n_weights);
+    NtTdArgs args;
+    args.boards = (u64*)d_boards;
+    args.after = (u64*)d_after;
+    args.scores = d_scores;
+    args.lengths = d_lengths;
+    args.n = (uint32_t)n;
+    args.W = d_weights;
+    args.alpha = alpha;
+    args.subs = (const uint2*)d_subs;
+    args.n_steps = n_steps;
+    args.acc = (unsigned long long*)d_scratch;
+    args.cnt = (uint32_t*)((uint8_t*)d_scratch + lay.cnt_off);
+    args.list = (uint32_t*)((uint8_t*)d_scratch + lay.list_off);
+    args.list_len = (uint32_t*)((uint8_t*)d_scratch + lay.len_off);
+    args.stats = (unsigned long long*)d_stats;
+    ntuple_net(args.net, h_placements, n_placements, d_weights);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE>(args, st);
+    return launch_ntuple_td<G2048_RNG_ORIGINAL>(args, st);
+}

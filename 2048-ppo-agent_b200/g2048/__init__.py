@@ -14,11 +14,12 @@ from .ppo import DevicePPOBatches, PPODataset, PPOIterationLoop, RolloutBuffer, 
 from .runs import BatchRunner, FixedHorizonRunner, FixedRollout, FlatRollout, PackedRollout, run_actions_batch, run_actions_max_tile
 from .state import State
 from .stats import RunningStatsVec
-from .td import TDLearner
+from .ntuple import NTupleNetwork
+from .td import NTupleTDLearner, TDLearner
 
 __all__ = [
     "ACTION_DIM", "BOARD_DIM", "BOARD_FLAT_DIM", "OBS_DIM", "BatchRunner", "DevicePPOBatches", "ExpectimaxPolicy", "ExpectimaxValues", "FixedHorizonRunner", "FixedRollout", "FlatRollout",
-    "MonteCarloPolicy", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
+    "MonteCarloPolicy", "NTupleNetwork", "NTupleTDLearner", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
     "RolloutBuffer", "RunningStatsVec", "State", "TDLearner", "TorchActionFunction", "act_drul", "act_randomly", "compute_gae",
     "create_ppo_dataloader", "default_row_values", "engine", "expectimax_values", "keys", "playout_values", "run_actions_batch", "run_actions_max_tile",
 ]

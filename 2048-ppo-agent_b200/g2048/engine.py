@@ -349,6 +349,50 @@ def td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, le
          ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
 
 
+def _placements_ptr(placements: np.ndarray) -> int:
+    """Host pointer of an n-tuple placement array (G2048TuplePlacement[], 12 bytes each, C-contiguous)."""
+    assert placements.dtype.itemsize == 12 and placements.flags.c_contiguous
+    return placements.ctypes.data
+
+
+def ntuple_td_scratch(n: int, placements: np.ndarray, n_weights: int, device) -> torch.Tensor:
+    """Zeroed scratch of g2048_ntuple_td_train for n envs and this network (every call leaves it zeroed)."""
+    size = int(N.lib.g2048_ntuple_td_scratch_bytes(n, placements.shape[0], n_weights))
+    if size < 0:
+        raise ValueError("ntuple_td_scratch: invalid sizes")
+    return torch.zeros(size // 8, dtype=torch.int64, device=device)
+
+
+def ntuple_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                    placements: np.ndarray, weights: torch.Tensor, alpha: float, subs: torch.Tensor, rng_mode: int,
+                    scratch: torch.Tensor, stats: torch.Tensor | None = None) -> None:
+    """``subs.shape[0]`` synchronous TD(0) steps of an n-tuple network (g2048_ntuple_td_train), in place on the env
+    state (as ``td_train``) and on ``weights`` (float32, the network's n_weights).  ``placements``: the host
+    G2048TuplePlacement array (``g2048.ntuple.PLACEMENT_DTYPE``).  ``scratch``: from ``ntuple_td_scratch``."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    need = int(N.lib.g2048_ntuple_td_scratch_bytes(n, placements.shape[0], weights.numel()))
+    if need < 0 or scratch.numel() * scratch.element_size() < need:
+        raise ValueError(f"ntuple_td_train: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch "
+                         f"and network need {need} (ntuple_td_scratch)")
+    call("g2048_ntuple_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, _placements_ptr(placements),
+         placements.shape[0], ptr(weights), weights.numel(), float(alpha), ptr(_i32(subs)), subs.shape[0], rng_mode,
+         ptr(scratch), ptr(stats), stream_ptr())
+
+
+def expectimax_values_ntuple(boards: torch.Tensor, depth: int, placements: np.ndarray, weights: torch.Tensor,
+                             reward_weight: float = 0.0, counters: torch.Tensor | None = None) -> torch.Tensor:
+    """``expectimax_values`` with V of an n-tuple network at the leaves (g2048_expectimax_values_ntuple): (n, 4)
+    float32 Q values, NaN where the action is illegal."""
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    q = torch.empty((boards.shape[0], 4), dtype=torch.float32, device=boards.device)
+    call("g2048_expectimax_values_ntuple", ptr(boards), boards.shape[0], depth, _placements_ptr(placements),
+         placements.shape[0], ptr(weights), weights.numel(), float(reward_weight), ptr(q), ptr(counters), stream_ptr())
+    return q
+
+
 def play_host(policy: int, seed: int, batch_global: int, rng_mode: int, env_lo: int = 0, n: int | None = None,
               key: np.ndarray | None = None, per_env: bool = True, pinned: bool = False):
     """The host-buffer C entry point (numpy in / numpy out; copies and syncs inside the call).

@@ -10,7 +10,8 @@ The search runs in one launch of ``g2048_expectimax_values``: max nodes over the
 empty cell with a 2 (probability 0.9) or a 4 (0.1), and at depth ``depth`` (counted in moves) the heuristic
 ``H(b) = sum of T[row] over the 4 rows and 4 columns``.  A move's value adds ``reward_weight`` times its merge reward.
 All arithmetic is float32 in a fixed order (include/g2048.h), so the values are bit-exact and a game is deterministic
-given the spawns.
+given the spawns.  With ``network=`` (a ``g2048.NTupleNetwork``) the leaves are the network's value V instead of H
+(``g2048_expectimax_values_ntuple``), with the same tree and float order.
 """
 from __future__ import annotations
 
@@ -63,11 +64,18 @@ def default_row_values(device=None) -> torch.Tensor:
     return t
 
 
-def _check(depth: int, row_values) -> None:
+def _check(depth: int, row_values, network=None) -> None:
     if not 1 <= int(depth) <= 4:
         raise ValueError(f"depth must be in 1..4, got {depth}")
     if row_values is not None and (not isinstance(row_values, torch.Tensor) or row_values.numel() != 65536):
         raise ValueError("row_values must be a tensor of 65536 float32 values")
+    if network is not None:
+        from .ntuple import NTupleNetwork
+
+        if not isinstance(network, NTupleNetwork):
+            raise ValueError("network must be an NTupleNetwork")
+        if row_values is not None:
+            raise ValueError("pass row_values or network, not both")
 
 
 def best_actions(q: torch.Tensor) -> torch.Tensor:
@@ -107,11 +115,13 @@ def _table_on(row_values, device) -> torch.Tensor:
     return row_values.to(device=device, dtype=torch.float32).contiguous()
 
 
-def expectimax_values(boards, depth: int = 2, row_values=None, reward_weight: float = 0.0, device=None) -> ExpectimaxValues:
+def expectimax_values(boards, depth: int = 2, row_values=None, reward_weight: float = 0.0, device=None,
+                      network=None) -> ExpectimaxValues:
     """Depth-``depth`` expectimax (1 <= depth <= 4, counted in moves) of every (board, action).  ``boards``: (n,) int64
     bitboards (a tensor, or anything numpy reads as such); ``row_values``: the row table T (65 536 values, default
-    ``default_row_values()``); ``reward_weight``: w, the weight of a move's merge reward."""
-    _check(depth, row_values)
+    ``default_row_values()``); ``reward_weight``: w, the weight of a move's merge reward; ``network``: an
+    ``NTupleNetwork`` whose V replaces H at the leaves (not together with ``row_values``)."""
+    _check(depth, row_values, network)
     if isinstance(boards, torch.Tensor):
         device = boards.device if device is None else torch.device(device)
         boards = boards.to(device=device, dtype=torch.int64).contiguous()
@@ -119,7 +129,11 @@ def expectimax_values(boards, depth: int = 2, row_values=None, reward_weight: fl
         device = N.require_cuda() if device is None else torch.device(device)
         boards = torch.from_numpy(np.ascontiguousarray(np.asarray(boards, dtype=np.uint64).reshape(-1)).view(np.int64)).to(device)
     counters = torch.zeros(2, dtype=torch.int64, device=device)
-    q = E.expectimax_values(boards, int(depth), _table_on(row_values, device), float(reward_weight), counters)
+    if network is not None:
+        q = E.expectimax_values_ntuple(boards, int(depth), network.placements, network.weights_on(device),
+                                       float(reward_weight), counters)
+    else:
+        q = E.expectimax_values(boards, int(depth), _table_on(row_values, device), float(reward_weight), counters)
     return ExpectimaxValues(q, counters)
 
 
@@ -129,14 +143,16 @@ class ExpectimaxPolicy:
     ``row_values`` (default: ``default_row_values()``) and ``reward_weight``.  An act_fn for
     ``BatchRunner.run_eval_batch``: per move one search over the envs still alive, then ``g2048_env_step`` with that
     move's step sub key.  The act sub key is not used, so a game is a function of (seed, batch size, depth, table,
-    reward_weight, rng_mode)."""
+    reward_weight, rng_mode).  With ``network`` (an ``NTupleNetwork``, not together with ``row_values``) the leaves
+    are the network's V."""
 
     depth: int = 2
     row_values: torch.Tensor | None = None
     reward_weight: float = 0.0
+    network: object | None = None
 
     def __post_init__(self):
-        _check(self.depth, self.row_values)
+        _check(self.depth, self.row_values, self.network)
 
     def table(self, device) -> torch.Tensor:
         return _table_on(self.row_values, device)

@@ -10,6 +10,9 @@ reward_weight=1.0)``), and ``T`` moves toward ``r' + H(s'')`` at the lines of th
 ``batch_size`` envs of a step read the same ``T``, the errors are summed in fixed point, and the update follows the
 whole step, so training is bit-exact and a run is a function of (seed, batch size, alpha, initial table, rng_mode,
 steps).  A call of ``train`` is one launch of ``g2048_td_train`` (include/g2048.h).
+
+``NTupleTDLearner`` learns an n-tuple network (``g2048.NTupleNetwork``) the same way, through
+``g2048_ntuple_td_train``: V in place of H, and the update at every placement of the previous afterstate.
 """
 from __future__ import annotations
 
@@ -21,9 +24,12 @@ import torch
 from . import _native as N
 from . import engine as E
 from .keys import KeyChain
+from .ntuple import NTupleNetwork, check_placements, _check_weights
 
 # the step size of the round-7 sweep on one B200 whose greedy player scored best (profiles/README.md, round 7)
 DEFAULT_ALPHA = 0.1
+# the step size of the round-8 sweep on one B200 whose greedy 4x6 player scored best (profiles/README.md, round 8)
+DEFAULT_NTUPLE_ALPHA = 0.02
 MAX_BATCH = 1 << 20
 _FLT_MAX = float(np.finfo(np.float32).max)
 
@@ -46,38 +52,43 @@ def _check_table(table) -> torch.Tensor:
     return table
 
 
-class TDLearner:
-    """Learns the row table by synchronous batched TD(0) over ``batch_size`` envs (1 .. 2^20).
+def _resolved(device) -> torch.device:
+    """``device`` with the current CUDA device filled in for a bare "cuda"."""
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    return device
 
-    ``table``: the float32 (65536,) device tensor being learned (zeros, or a copy of the given finite table).
-    ``train(n_steps)`` makes ``n_steps`` steps and returns the summary of the episodes that ended in them
-    (``engine.play_stats_dict`` form).  Keys come from the runner's chain of ``init_seed``: sub key 0 initialises the
-    envs, and every step consumes one more.  ``state_dict`` / ``load_state_dict`` resume a run bit for bit."""
 
-    def __init__(self, init_seed: int, batch_size: int, alpha: float = DEFAULT_ALPHA, table=None, rng_mode=None,
-                 device=None):
+class _BatchTDLearner:
+    """What the two learners share: ``batch_size`` envs (1 .. 2^20) with their afterstates, scores and lengths, the key
+    chain of ``init_seed`` (sub key 0 initialises the envs, every step consumes one more), ``train`` and the
+    checkpoint.  A subclass holds the value function and launches the steps (``_launch``); its checkpoint entries
+    come from ``_values_state`` and are checked by ``_check_values_state`` before a load changes anything."""
+
+    def _check_common(self, batch_size, alpha) -> tuple[int, float]:
         batch_size = int(batch_size)
         if not 1 <= batch_size <= MAX_BATCH:
             raise ValueError(f"batch_size must be in [1, 2^20], got {batch_size}")
-        self.alpha = _check_alpha(alpha)
-        if table is not None:
-            table = _check_table(table)
+        return batch_size, _check_alpha(alpha)
+
+    def _start(self, rng_mode, device) -> None:
+        """rng_mode and device, after the arguments are checked and before anything is allocated."""
         self.rng_mode = E.resolve_rng_mode(rng_mode)
         self.device = N.require_cuda() if device is None else torch.device(device)
-        self.batch_size = batch_size
-        if table is None:
-            self.table = torch.zeros(65536, dtype=torch.float32, device=self.device)
-        else:
-            self.table = table.to(self.device).clone()
+
+    def _init_envs(self, init_seed) -> None:
         self.chain = KeyChain(init_seed, self.rng_mode, self.device)
-        n = batch_size
+        n = self.batch_size
         self.boards, _ = E.env_init(self.chain.peek(1)[0], n, 0, n, self.rng_mode)
         self.chain.consume(1)
         self.after = torch.zeros(n, dtype=torch.int64, device=self.device)
         self.scores = torch.zeros(n, dtype=torch.int32, device=self.device)
         self.lengths = torch.zeros(n, dtype=torch.int32, device=self.device)
-        self._scratch = E.td_scratch(self.device)
         self.steps = 0
+
+    def _launch(self, subs: torch.Tensor, stats: torch.Tensor) -> None:
+        raise NotImplementedError
 
     def train(self, n_steps: int) -> dict:
         """``n_steps`` learning steps in one launch; returns the summary of the episodes that ended in them."""
@@ -87,24 +98,34 @@ class TDLearner:
         stats = torch.zeros(N.PLAY_STATS_WORDS, dtype=torch.int64, device=self.device)
         if n_steps:
             subs = self.chain.peek(n_steps)
-            E.td_train(self.boards, self.after, self.scores, self.lengths, self.table, self.alpha, subs, self.rng_mode,
-                       self._scratch, stats)
+            self._launch(subs, stats)
             self.chain.consume(n_steps)
             self.steps += n_steps
         return E.play_stats_dict(stats)
 
-    # -- checkpointing: key chain, env state and table ---------------------------------------------------------
+    # -- checkpointing: key chain, env state and the value function ----------------------------------------------
+    def _values_state(self) -> dict:
+        raise NotImplementedError
+
+    def _check_values_state(self, state: dict):
+        raise NotImplementedError
+
+    def _load_values(self, values) -> None:
+        raise NotImplementedError
+
     def state_dict(self) -> dict:
-        return {"key": [int(w) for w in self.chain.key], "position": int(self.chain.position), "rng_mode": int(self.rng_mode),
-                "batch_size": self.batch_size, "alpha": self.alpha, "steps": self.steps, "table": self.table.cpu().clone(),
-                "boards": self.boards.cpu().clone(), "after": self.after.cpu().clone(),
-                "scores": self.scores.cpu().clone(), "lengths": self.lengths.cpu().clone()}
+        out = {"key": [int(w) for w in self.chain.key], "position": int(self.chain.position), "rng_mode": int(self.rng_mode),
+               "batch_size": self.batch_size, "alpha": self.alpha, "steps": self.steps}
+        out.update(self._values_state())
+        out.update({"boards": self.boards.cpu().clone(), "after": self.after.cpu().clone(),
+                    "scores": self.scores.cpu().clone(), "lengths": self.lengths.cpu().clone()})
+        return out
 
     def load_state_dict(self, state: dict) -> None:
         if int(state["batch_size"]) != self.batch_size or state["boards"].shape[0] != self.batch_size:
             raise ValueError("checkpoint was written for a different batch size")
         alpha = _check_alpha(state["alpha"])
-        table = _check_table(state["table"])
+        values = self._check_values_state(state)
         if int(state["rng_mode"]) not in (E.RNG_ORIGINAL, E.RNG_PARTITIONABLE):
             raise ValueError(f"checkpoint has an unknown rng_mode {state['rng_mode']!r}")
         self.alpha = alpha
@@ -112,6 +133,87 @@ class TDLearner:
         self.chain = KeyChain(np.asarray(state["key"], dtype=np.uint32), self.rng_mode, self.device)
         self.chain._base_pos = int(state["position"])
         self.steps = int(state["steps"])
-        self.table.copy_(table.to(self.device))
+        self._load_values(values)
         for name in ("boards", "after", "scores", "lengths"):
             getattr(self, name).copy_(state[name].to(self.device))
+
+
+class TDLearner(_BatchTDLearner):
+    """Learns the row table by synchronous batched TD(0) over ``batch_size`` envs (1 .. 2^20).
+
+    ``table``: the float32 (65536,) device tensor being learned (zeros, or a copy of the given finite table).
+    ``train(n_steps)`` makes ``n_steps`` steps and returns the summary of the episodes that ended in them
+    (``engine.play_stats_dict`` form).  Keys come from the runner's chain of ``init_seed``: sub key 0 initialises the
+    envs, and every step consumes one more.  ``state_dict`` / ``load_state_dict`` resume a run bit for bit."""
+
+    def __init__(self, init_seed: int, batch_size: int, alpha: float = DEFAULT_ALPHA, table=None, rng_mode=None,
+                 device=None):
+        self.batch_size, self.alpha = self._check_common(batch_size, alpha)
+        if table is not None:
+            table = _check_table(table)
+        self._start(rng_mode, device)
+        if table is None:
+            self.table = torch.zeros(65536, dtype=torch.float32, device=self.device)
+        else:
+            self.table = table.to(self.device).clone()
+        self._init_envs(init_seed)
+        self._scratch = E.td_scratch(self.device)
+
+    def _launch(self, subs, stats) -> None:
+        E.td_train(self.boards, self.after, self.scores, self.lengths, self.table, self.alpha, subs, self.rng_mode,
+                   self._scratch, stats)
+
+    def _values_state(self) -> dict:
+        return {"table": self.table.cpu().clone()}
+
+    def _check_values_state(self, state):
+        return _check_table(state["table"])
+
+    def _load_values(self, table) -> None:
+        self.table.copy_(table.to(self.device))
+
+
+class NTupleTDLearner(_BatchTDLearner):
+    """Learns an n-tuple network by synchronous batched TD(0) over ``batch_size`` envs (1 .. 2^20), as ``TDLearner``
+    learns the row table: the same greedy move, fixed-point update, key chain and statistics.
+
+    ``network``: the ``NTupleNetwork`` whose ``weights`` are learned in place (default: a zero ``four_six()``).
+    ``state_dict`` / ``load_state_dict`` resume a run bit for bit; the checkpoint holds the placements, and a load
+    whose placements or n_weights differ from the learner's network is rejected before anything changes."""
+
+    def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
+                 alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None):
+        self.batch_size, self.alpha = self._check_common(batch_size, alpha)
+        if network is not None and not isinstance(network, NTupleNetwork):
+            raise ValueError("network must be an NTupleNetwork")
+        self._start(rng_mode, device)
+        self.network = NTupleNetwork.four_six(device=self.device) if network is None else network
+        if _resolved(self.network.weights.device) != _resolved(self.device):
+            raise ValueError(f"the network's weights are on {self.network.weights.device}, the learner runs on {self.device}")
+        self._init_envs(init_seed)
+        self._scratch = E.ntuple_td_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
+
+    @property
+    def weights(self) -> torch.Tensor:
+        return self.network.weights
+
+    def _launch(self, subs, stats) -> None:
+        net = self.network
+        E.ntuple_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights, self.alpha,
+                          subs, self.rng_mode, self._scratch, stats)
+
+    def _values_state(self) -> dict:
+        net = self.network
+        return {"placements": net.placements.copy(), "n_weights": net.n_weights, "weights": net.weights.cpu().clone()}
+
+    def _check_values_state(self, state):
+        net = self.network
+        if int(state["n_weights"]) != net.n_weights:
+            raise ValueError("checkpoint was written for a network with a different n_weights")
+        placements = check_placements(state["placements"], net.n_weights)
+        if not np.array_equal(placements, net.placements):
+            raise ValueError("checkpoint was written for a network with different placements")
+        return _check_weights(state["weights"], net.n_weights)
+
+    def _load_values(self, weights) -> None:
+        self.network.weights.copy_(weights.to(self.device))

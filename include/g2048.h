@@ -262,6 +262,50 @@ int g2048_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, ui
                    float* d_row_values, float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
                    void* d_scratch, uint64_t* d_stats, void* stream);
 
+/* ---- N-tuple networks: a value function V over one flat float32 weight array W (n_weights entries), given as an
+ * ordered list of placements.  Placement p reads the k = n_cells cells cells[0..k) of the board:
+ *   idx_p(b) = sum over j < k of exp(b, cells[j]) << 4j        (cell = 4 * row + col, exp(b, c) = nibble c of b)
+ *   V(b)     = W[off_0 + idx_0(b)] + W[off_1 + idx_1(b)] + ... + W[off_{P-1} + idx_{P-1}(b)], float32, left to right
+ *              from the first term (no leading 0).
+ * Several placements with the same offset share one table (symmetric sharing).  The row heuristic H above is the
+ * network of one 65 536-entry table at offset 0 with the 8 placements (4r, 4r+1, 4r+2, 4r+3) for r = 0..3, then
+ * (c, c+4, c+8, c+12) for c = 0..3: V == H bit for bit.
+ * The placement list is a HOST array of 1..G2048_NTUPLE_MAX_PLACEMENTS entries, checked before any launch:
+ * G2048_ERR_INVALID for n_cells outside 1..6, a cell >= 16 or repeated within a placement, a nonzero reserved byte,
+ * off + 16^k > n_weights, or n_weights outside [1, 2^28]. */
+typedef struct G2048TuplePlacement {
+    uint32_t offset;  /* first entry of this placement's table in W */
+    uint8_t n_cells;  /* k, 1..6 */
+    uint8_t cells[6]; /* cell = 4*row + col; nibble j of the index is the exponent in cells[j] */
+    uint8_t reserved; /* 0 */
+} G2048TuplePlacement; /* 12 bytes */
+#define G2048_NTUPLE_MAX_PLACEMENTS 64
+#define G2048_NTUPLE_MAX_WEIGHTS (1ll << 28)
+
+/* Batched TD(0) afterstate learning of an n-tuple network: g2048_td_train's contract word for word, with V in place of
+ * H and, in step 2, for each placement p in order acc[off_p + idx_p(after)] += fx(delta) and cnt[...] += 1.  With
+ * P <= 64 and n <= 2^20, |acc[i]| <= 2^20 * 64 * 2^36 = 2^62: the int64 sums cannot overflow.  Step 4 is the same
+ * per-entry mean for every entry with cnt[i] > 0, so the result is bit-exact whatever the grid or the atomics' order.
+ *   d_weights: W, float[n_weights], updated in place (4-byte aligned).
+ *   d_scratch: g2048_ntuple_td_scratch_bytes(n, n_placements, n_weights) bytes, zeroed by the caller once; every call
+ *           leaves it zeroed.  The size grows with n_weights (the per-entry sums), and with n * n_placements (the
+ *           list of the entries touched in one step: the update after each step costs work proportional to those
+ *           entries, not to n_weights).  g2048_ntuple_td_scratch_bytes returns -1 for invalid sizes.
+ * G2048_ERR_INVALID for everything g2048_td_train rejects and for an invalid network (above). */
+int64_t g2048_ntuple_td_scratch_bytes(int64_t n, int n_placements, int64_t n_weights);
+int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths, int64_t n,
+                          const G2048TuplePlacement* h_placements, int n_placements, float* d_weights, int64_t n_weights,
+                          float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
+                          void* d_scratch, uint64_t* d_stats, void* stream);
+
+/* g2048_expectimax_values with V of an n-tuple network in place of H at the leaves: the same tree, float order, NaN
+ * for illegal actions and counters.  d_weights: W, float[n_weights] (device, read-only while the call runs).  Depth 1
+ * with reward_weight 1 is g2048_ntuple_td_train's greedy move. */
+int g2048_expectimax_values_ntuple(const uint64_t* d_boards, int64_t n, int depth,
+                                   const G2048TuplePlacement* h_placements, int n_placements,
+                                   const float* d_weights, int64_t n_weights, float reward_weight,
+                                   float* d_q, uint64_t* d_counters, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.

@@ -1,0 +1,283 @@
+"""Speed and learning of the n-tuple TD(0) learner (g2048_ntuple_td_train, g2048.NTupleTDLearner) and of expectimax
+over a network (g2048_expectimax_values_ntuple); prints one JSON line.
+
+  * speed: learning steps (env-steps) per second and microseconds per batch step for the 4x6 network at n = 2^14, 2^16
+    and 2^18, device-timed with CUDA events around one launch of `steps` steps after a warm-up launch.
+  * the accumulate / apply split per step and the entries touched per step, from a
+    second build of the library with -DG2048_NTUPLE_PHASES (compiled into a temporary directory, run in a subprocess).
+  * the `lines` network through g2048_ntuple_td_train next to g2048_td_train at n = 2^16 (the same computation).
+  * the step time with n_weights: a 2.2 M-weight network packed, and the same tables at high offsets of an array 16
+    times as large, at n = 2^16.
+  * an alpha sweep of the 4x6 network from zeros at n = 2^16: the learning curve (mean score of the episodes that
+    ended in each block of steps) and the greedy player over the same B seeded games.
+  * players: greedy / depth 2 / depth 3 with the learned 4x6 network, the learned row table (TDLearner, alpha 0.1) at
+    the same number of learning steps and at the same training wall time, and default_row_values(): mean score and
+    the share of games that reach 2048 / 4096 / 8192.
+  * search: expectimax leaves/s at depth 2 and 3 on bench_expectimax.py's 4 096 mid-game boards with the 4x6 network
+    leaf next to the row table (L2 flushed before every timed launch).
+
+    python tools/bench_ntuple.py [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
+"""
+import argparse
+import json
+import os
+import statistics
+import subprocess
+import sys
+import tempfile
+import time
+from pathlib import Path
+
+ROOT = Path(__file__).resolve().parent.parent
+sys.path[:0] = [str(ROOT), str(ROOT / "2048-ppo-agent_b200"), str(ROOT / "tools")]
+
+import torch  # noqa: E402
+
+import g2048  # noqa: E402
+from g2048 import engine as E  # noqa: E402
+from g2048.ntuple import NTupleNetwork, make_placements  # noqa: E402
+
+from bench_playout import device_times, gpu_info, mid_game_boards  # noqa: E402
+
+SIZES = (1 << 14, 1 << 16, 1 << 18)
+ALPHAS = (0.001, 0.0025, 0.005, 0.01, 0.02, 0.03)
+MODE = E.RNG_PARTITIONABLE
+
+
+def _timed(run, reps):
+    run()  # warm-up: module load, row tables, and games in progress rather than fresh envs
+    torch.cuda.synchronize()
+    times = []
+    for _ in range(reps):
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        run()
+        b.record()
+        torch.cuda.synchronize()
+        times.append(a.elapsed_time(b) * 1e-3)
+    return times
+
+
+def _row(name, n, steps, times, **extra):
+    best = min(times)
+    row = {"what": name, "n": n, "steps": steps, "seconds": [round(t, 4) for t in times],
+           "us_per_step": best / steps * 1e6, "learning_steps_per_s": n * steps / best}
+    row.update(extra)
+    print(json.dumps(row), file=sys.stderr, flush=True)
+    return row
+
+
+def _ntuple_run(lr, subs):
+    net = lr.network
+    return lambda: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements, net.weights, lr.alpha,
+                                     subs, MODE, lr._scratch)
+
+
+def speed(steps: int, reps: int = 3) -> list:
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        lr = g2048.NTupleTDLearner(0, n, alpha=0.0025, rng_mode=MODE)
+        out.append(_row("four_six", n, steps, _timed(_ntuple_run(lr, subs), reps)))
+        del lr
+        torch.cuda.empty_cache()
+    return out
+
+
+def phase_probe(steps: int) -> list:
+    """In a build with -DG2048_NTUPLE_PHASES: the accumulate / apply split of one launch of `steps` steps after a
+    warm-up launch, as CTA 0 timed it (%globaltimer up to each phase's closing grid.sync()), and the entries listed
+    (touched) per step."""
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        lr = g2048.NTupleTDLearner(0, n, alpha=0.0025, rng_mode=MODE)
+        net = lr.network
+        stats = torch.zeros(32, dtype=torch.int64, device="cuda")
+        run = lambda st=None: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,  # noqa: E731
+                                                net.weights, lr.alpha, subs, MODE, lr._scratch, st)
+        run()
+        torch.cuda.synchronize()
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        run(stats)
+        b.record()
+        torch.cuda.synchronize()
+        acc_ns, apply_ns, listed = (int(x) for x in stats[8:11].tolist())
+        out.append({"n": n, "steps": steps, "us_per_step": a.elapsed_time(b) * 1e3 / steps,
+                    "accumulate_us_per_step": acc_ns / 1e3 / steps, "apply_us_per_step": apply_ns / 1e3 / steps,
+                    "entries_listed_per_step": listed / steps})
+        print(json.dumps(out[-1]), file=sys.stderr, flush=True)
+        del lr, net
+        torch.cuda.empty_cache()
+    return out
+
+
+def phases(steps: int) -> dict:
+    """Builds the library with -DG2048_NTUPLE_PHASES into a temporary directory and runs phase_probe on it."""
+    tmp = Path(tempfile.mkdtemp(prefix="g2048_ntuple_phases_"))
+    lib = tmp / "libg2048_phases.so"
+    subprocess.run(["make", "-C", str(ROOT / "2048-ppo-agent_b200" / "csrc"), "-j16", f"OUT={lib}", f"BUILD={tmp / 'build'}",
+                    "EXTRA=-DG2048_NTUPLE_PHASES"], check=True, capture_output=True)
+    env = dict(os.environ, G2048_LIB=str(lib))
+    res = subprocess.run([sys.executable, __file__, "--phase-probe", "--steps", str(steps)], env=env, capture_output=True,
+                         text=True, check=True)
+    return {"build": "-DG2048_NTUPLE_PHASES", "rows": json.loads(res.stdout.strip().splitlines()[-1])}
+
+
+def lines_vs_row(steps: int, reps: int = 3) -> list:
+    n = 1 << 16
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    row = g2048.TDLearner(0, n, alpha=0.1, rng_mode=MODE)
+    run_row = lambda: E.td_train(row.boards, row.after, row.scores, row.lengths, row.table, row.alpha, subs, MODE,  # noqa: E731
+                                 row._scratch)
+    lines = g2048.NTupleTDLearner(0, n, network=NTupleNetwork.lines(), alpha=0.1, rng_mode=MODE)
+    return [_row("row_table_td_train", n, steps, _timed(run_row, reps)),
+            _row("lines_ntuple_td_train", n, steps, _timed(_ntuple_run(lines, subs), reps))]
+
+
+def weights_size(steps: int, reps: int = 3) -> list:
+    """A network of two 5-cell and two 4-cell tuples under the 8 symmetries (2.2 M weights), packed and at the top of
+    an array 16 times as large."""
+    n = 1 << 16
+    tuples = [(0, 1, 2, 3, 4), (4, 5, 6, 7, 8), (0, 1, 4, 5), (8, 9, 12, 13)]
+    sizes = [16 ** len(t) for t in tuples]
+    total = sum(sizes)
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    out = []
+    for name, shift in (("packed", 0), ("high_offsets", 15 * total)):
+        rows = [(shift + sum(sizes[:j]), im) for j, t in enumerate(tuples) for im in g2048.ntuple.symmetric_images(t)]
+        net = NTupleNetwork(make_placements(rows), shift + total)
+        lr = g2048.NTupleTDLearner(0, n, network=net, alpha=0.0025, rng_mode=MODE)
+        out.append(_row(name, n, steps, _timed(_ntuple_run(lr, subs), reps), n_weights=shift + total))
+        del lr, net
+        torch.cuda.empty_cache()
+    return out
+
+
+def _reach(summary, B):
+    hist = summary["max_tile_hist"]
+    return {str(t): sum(v for k, v in hist.items() if k >= t) / B for t in (2048, 4096, 8192)}
+
+
+def play(policy, B, seed=7) -> dict:
+    runner = g2048.BatchRunner(seed, policy)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    s = runner.run_eval_batch(B)["summary"] if isinstance(policy, g2048.ExpectimaxPolicy) else runner.run_stats_batch(B)["summary"]
+    torch.cuda.synchronize()
+    return {"games": B, "mean_score": s["score_sum"] / B, "reach": _reach(s, B), "mean_moves": s["env_steps"] / B,
+            "seconds": round(time.perf_counter() - t0, 2)}
+
+
+def _train(lr, total, block):
+    curve = []
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for _ in range(total // block):
+        s = lr.train(block)
+        curve.append(round(s["score_sum"] / max(s["episodes"], 1), 1))
+    torch.cuda.synchronize()
+    return curve, time.perf_counter() - t0
+
+
+def sweep(n: int, total: int, block: int, B: int) -> tuple:
+    rows, best = [], None
+    for alpha in ALPHAS:
+        lr = g2048.NTupleTDLearner(0, n, alpha=alpha)
+        curve, wall = _train(lr, total, block)
+        greedy = play(g2048.ExpectimaxPolicy(depth=1, network=lr.network, reward_weight=1.0), B)
+        rows.append({"alpha": alpha, "n": n, "steps": total, "block": block, "train_seconds": round(wall, 2),
+                     "curve_mean_score": curve, "greedy": greedy})
+        print(json.dumps(rows[-1]), file=sys.stderr, flush=True)
+        if best is None or greedy["mean_score"] > best[0]:
+            best = (greedy["mean_score"], alpha, lr.network, wall)
+        del lr
+        torch.cuda.empty_cache()
+    return rows, best
+
+
+def search(reps: int, net) -> list:
+    flush_buf = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
+    boards = mid_game_boards(4096, 100, MODE)
+    table = g2048.default_row_values()
+    out = []
+    for depth in (2, 3):
+        for leaf in ("row_table", "four_six"):
+            if leaf == "row_table":
+                fn = lambda c=None: E.expectimax_values(boards, depth, table, 0.0, c)  # noqa: E731
+            else:
+                fn = lambda c=None: E.expectimax_values_ntuple(boards, depth, net.placements, net.weights, 0.0, c)  # noqa: E731
+            counters = torch.zeros(2, dtype=torch.int64, device="cuda")
+            fn(counters)
+            leaves = int(counters[0].item())
+            times = device_times(fn, reps, flush_buf)
+            med = statistics.median(times)
+            out.append({"depth": depth, "leaf": leaf, "boards": 4096, "leaves": leaves,
+                        "ms": [round(t * 1e3, 3) for t in times], "leaves_per_s": leaves / med})
+            print(json.dumps(out[-1]), file=sys.stderr, flush=True)
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--steps", type=int, default=500, help="batch steps per timed launch")
+    ap.add_argument("--sweep-steps", type=int, default=4000)
+    ap.add_argument("--block", type=int, default=250)
+    ap.add_argument("--games", type=int, default=1024)
+    ap.add_argument("--deep-games", type=int, default=128, help="games for the depth-2 and depth-3 players")
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--speed-only", action="store_true", help="speed, phases, lines and n_weights only")
+    ap.add_argument("--skip-speed", action="store_true", help="the sweep, search and players only")
+    ap.add_argument("--phase-probe", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    if args.phase_probe:
+        print(json.dumps(phase_probe(args.steps)))
+        return
+    result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident); flushed for search"}
+    if not args.skip_speed:
+        result["speed"] = speed(args.steps)
+        result["phases"] = phases(args.steps)
+        result["lines_vs_row"] = lines_vs_row(args.steps)
+        result["n_weights"] = weights_size(args.steps)
+    if args.speed_only:
+        _emit(result, args.out)
+        return
+    B = args.games
+    rows, (_, alpha, net, wall) = sweep(1 << 16, args.sweep_steps, args.block, B)
+    result["sweep"] = rows
+    result["search"] = search(args.reps, net)
+    # the row table: the same learning steps, and the same training wall time as the chosen 4x6 run
+    row = g2048.TDLearner(0, 1 << 16)
+    _, row_wall = _train(row, args.sweep_steps, args.block)
+    row_time = g2048.TDLearner(0, 1 << 16)
+    steps_in_wall = max(args.block, int(args.sweep_steps * wall / row_wall) // args.block * args.block)
+    _train(row_time, steps_in_wall, args.block)
+    players = {"drul": play(g2048.act_drul, B)}
+    for depth in (1, 2, 3):
+        g = B if depth == 1 else args.deep_games
+        players[f"four_six_alpha{alpha}_depth{depth}"] = play(
+            g2048.ExpectimaxPolicy(depth=depth, network=net, reward_weight=1.0), g)
+        players[f"row_table_same_steps_depth{depth}"] = play(
+            g2048.ExpectimaxPolicy(depth=depth, row_values=row.table, reward_weight=1.0), g)
+        players[f"row_table_same_wall_depth{depth}"] = play(
+            g2048.ExpectimaxPolicy(depth=depth, row_values=row_time.table, reward_weight=1.0), g)
+        players[f"default_table_depth{depth}"] = play(g2048.ExpectimaxPolicy(depth=depth), g)
+        print(json.dumps({k: v for k, v in players.items() if k.endswith(f"depth{depth}")}), file=sys.stderr, flush=True)
+    result["players"] = {"seed": 7, "alpha": alpha, "four_six_train_seconds": round(wall, 2),
+                         "row_train_seconds": round(row_wall, 2), "row_steps_in_same_wall": steps_in_wall,
+                         "results": players}
+    _emit(result, args.out)
+
+
+def _emit(result: dict, out) -> None:
+    line = json.dumps(result)
+    print(line)
+    if out:
+        Path(out).parent.mkdir(parents=True, exist_ok=True)
+        Path(out).write_text(line + "\n")
+
+
+if __name__ == "__main__":
+    main()
