@@ -20,6 +20,12 @@
 // Hot entries: early boards give most placements index 0 (all cells empty).  Each entry is first aggregated in the warp
 // (__match_any_sync: the group's leader adds the group's sum), and index 0 of every placement is further summed per CTA
 // in shared memory, with one global atomic per CTA, placement and step.
+//
+// Temporal coherence (g2048_ntuple_tc_train, the TC instantiations): the same kernel, which also sums |fx| into
+// abs[i] next to acc[i] (the same warp aggregation and per-CTA index-0 sums), and whose apply phase scales each
+// entry's step by beta = |E[i]| / A[i] from the entry's float64 running sums, then adds the step's sums to E and A.
+// Only the apply phase touches E and A, one thread per listed entry, and grid.sync() orders the steps, so they use
+// ordinary loads and stores.  With TC = false none of it is compiled in.
 #include <cooperative_groups.h>
 
 #include "g2048_ntuple.cuh"
@@ -46,15 +52,17 @@ constexpr int NT_SMEM_BYTES = PLAY3_TABLE_BYTES;  // the row tables; the small a
 constexpr float NT_FX_CLAMP = 16777216.0f;        // 2^24: 2^20 envs * 64 placements * 2^24 * 4096 = 2^62
 constexpr float NT_FX_ONE = 4096.0f;
 
-// scratch: acc int64[n_weights], cnt uint32[n_weights], list uint32[min(n * P, n_weights)], then list_len uint32[2]
+// scratch: acc int64[n_weights], (TC: abs int64[n_weights],) cnt uint32[n_weights], list uint32[min(n * P,
+// n_weights)], then list_len uint32[2]
 struct NtScratch {
-    int64_t cnt_off, list_off, len_off, bytes;
+    int64_t abs_off, cnt_off, list_off, len_off, bytes;
 };
 
-static NtScratch nt_scratch_layout(int64_t n, int n_placements, int64_t n_weights) {
+static NtScratch nt_scratch_layout(int64_t n, int n_placements, int64_t n_weights, bool tc) {
     const int64_t touched = n * n_placements < n_weights ? n * n_placements : n_weights;
     NtScratch s;
-    s.cnt_off = 8 * n_weights;
+    s.abs_off = 8 * n_weights;
+    s.cnt_off = (tc ? 16 : 8) * n_weights;
     s.list_off = s.cnt_off + 4 * n_weights;
     s.len_off = (s.list_off + 4 * touched + 7) & ~7ll;
     s.bytes = s.len_off + 8;
@@ -77,6 +85,10 @@ struct NtTdArgs {
     uint32_t* list_len;  // [2]: step t appends through list_len[t & 1]
     unsigned long long* stats;
     NtNet net;  // net.W == W
+    // TC only (after net, so the TD instantiations see the parameter layout they always had)
+    unsigned long long* abs_acc;  // the sums of |fx|, next to acc
+    double* err_sum;              // E
+    double* abs_err_sum;          // A
 };
 
 // fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64, to nearest even (the multiply by a power of two is exact)
@@ -95,18 +107,20 @@ __device__ __forceinline__ void nt_append(bool first, uint32_t i, uint32_t* list
     }
 }
 
-template <int MODE>
+template <int MODE, bool TC>
 __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_constant__ NtTdArgs a) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     __shared__ unsigned long long s_stats[G2048_PLAY_STATS_WORDS];
     __shared__ long long s_fx[NT_THREADS];
     __shared__ unsigned long long s_acc0[G2048_NTUPLE_MAX_PLACEMENTS];
     __shared__ unsigned s_cnt0[G2048_NTUPLE_MAX_PLACEMENTS];
+    __shared__ unsigned long long s_abs0[TC ? G2048_NTUPLE_MAX_PLACEMENTS : 1];
     play3_copy_row_tables<NT_THREADS>(smem_raw);
     for (int i = threadIdx.x; i < G2048_PLAY_STATS_WORDS; i += NT_THREADS) s_stats[i] = 0ull;
     if (threadIdx.x < G2048_NTUPLE_MAX_PLACEMENTS) {
         s_acc0[threadIdx.x] = 0ull;
         s_cnt0[threadIdx.x] = 0u;
+        if constexpr (TC) s_abs0[threadIdx.x] = 0ull;
     }
     __syncthreads();
 
@@ -176,14 +190,20 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
                 const unsigned group = __match_any_sync(0xFFFFFFFFu, update ? i : 0xFFFFFFFFu);  // i < 2^28
                 bool first = false;
                 if (update && lane == (unsigned)(__ffs((int)group) - 1)) {
-                    long long sum = 0;
-                    for (unsigned m = group; m; m &= m - 1u) sum += warp_fx[__ffs((int)m) - 1];
+                    long long sum = 0, abs_sum = 0;
+                    for (unsigned m = group; m; m &= m - 1u) {
+                        const long long fx = warp_fx[__ffs((int)m) - 1];
+                        sum += fx;
+                        if constexpr (TC) abs_sum += fx < 0 ? -fx : fx;
+                    }
                     const unsigned count = (unsigned)__popc((int)group);
                     if (i == a.net.pl[p].offset) {
                         atomicAdd(&s_acc0[p], (unsigned long long)sum);
+                        if constexpr (TC) atomicAdd(&s_abs0[p], (unsigned long long)abs_sum);
                         atomicAdd(&s_cnt0[p], count);
                     } else {
                         atomicAdd(&a.acc[i], (unsigned long long)sum);
+                        if constexpr (TC) atomicAdd(&a.abs_acc[i], (unsigned long long)abs_sum);
                         first = atomicAdd(&a.cnt[i], count) == 0u;
                     }
                 }
@@ -222,6 +242,10 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
         if (threadIdx.x < P && s_cnt0[threadIdx.x]) {  // the CTA's index-0 sums, one placement per thread
             const uint32_t i = a.net.pl[threadIdx.x].offset;
             atomicAdd(&a.acc[i], s_acc0[threadIdx.x]);
+            if constexpr (TC) {
+                atomicAdd(&a.abs_acc[i], s_abs0[threadIdx.x]);
+                s_abs0[threadIdx.x] = 0ull;
+            }
             if (atomicAdd(&a.cnt[i], s_cnt0[threadIdx.x]) == 0u) a.list[atomicAdd(list_len, 1u)] = i;
             s_acc0[threadIdx.x] = 0ull;
             s_cnt0[threadIdx.x] = 0u;
@@ -235,15 +259,27 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
             listed += __ldcg(list_len);
         }
 #endif
-        // ---- apply: every listed entry moves by alpha times the mean of its errors; its sums and its list slot go
-        // back to zero, and the other list's length is cleared for the next step
+        // ---- apply: every listed entry moves by alpha times the mean of its errors (TC: times beta, from E and A
+        // before this step, which then take the step's sums); its sums and its list slot go back to zero, and the
+        // other list's length is cleared for the next step
         const uint32_t len = __ldcg(list_len);
         for (uint32_t j = blockIdx.x * NT_THREADS + threadIdx.x; j < len; j += stride) {
             const uint32_t i = __ldcg(&a.list[j]);
             const uint32_t count = __ldcg(&a.cnt[i]);
             const long long sum = (long long)__ldcg(&a.acc[i]);
-            const float mean = (float)((double)sum / (4096.0 * (double)count));
-            a.W[i] = a.W[i] + a.alpha * mean;
+            if constexpr (TC) {
+                const long long abs_sum = (long long)__ldcg(&a.abs_acc[i]);
+                const double m = (double)sum / (4096.0 * (double)count);
+                const double e = a.err_sum[i], A = a.abs_err_sum[i];
+                const double beta = A > 0.0 ? fmin(fabs(e) / A, 1.0) : 1.0;
+                a.W[i] = a.W[i] + a.alpha * (float)(beta * m);
+                a.err_sum[i] = e + (double)sum / 4096.0;
+                a.abs_err_sum[i] = A + (double)abs_sum / 4096.0;
+                a.abs_acc[i] = 0ull;
+            } else {
+                const float mean = (float)((double)sum / (4096.0 * (double)count));
+                a.W[i] = a.W[i] + a.alpha * mean;
+            }
             a.acc[i] = 0ull;
             a.cnt[i] = 0u;
             a.list[j] = 0u;
@@ -286,23 +322,24 @@ __global__ void build_ntuple_row_tables_kernel() {
     build_row_table_entry(row);
 }
 
-template <int MODE>
+template <int MODE, bool TC>
 static int launch_ntuple_td(const NtTdArgs& args, cudaStream_t st) {
-    auto kernel = ntuple_td_kernel<MODE>;
+    auto kernel = ntuple_td_kernel<MODE, TC>;
     static bool configured_on[64] = {false};
     bool* configured = device_once_flag(configured_on);
     if (!configured) return fail_arg("no CUDA device");
     int dev = 0;
-    int rc = check_cuda(cudaGetDevice(&dev), "ntuple_td_train: device");
+    int rc = check_cuda(cudaGetDevice(&dev), TC ? "ntuple_tc_train: device" : "ntuple_td_train: device");
     if (rc) return rc;
     if (!*configured) {
         int coop = 0;
         rc = check_cuda(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev),
-                        "ntuple_td_train: device attribute");
+                        TC ? "ntuple_tc_train: device attribute" : "ntuple_td_train: device attribute");
         if (rc) return rc;
-        if (!coop) return fail_arg("ntuple_td_train: the device does not support cooperative launches");
+        if (!coop) return fail_arg(TC ? "ntuple_tc_train: the device does not support cooperative launches"
+                             : "ntuple_td_train: the device does not support cooperative launches");
         rc = check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, NT_SMEM_BYTES),
-                        "ntuple_td_train: shared memory attribute");
+                        TC ? "ntuple_tc_train: shared memory attribute" : "ntuple_td_train: shared memory attribute");
         if (rc) return rc;
         *configured = true;
     }
@@ -310,49 +347,64 @@ static int launch_ntuple_td(const NtTdArgs& args, cudaStream_t st) {
     if (rc) return rc;
     int per_sm = 0;
     rc = check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT_THREADS, NT_SMEM_BYTES),
-                    "ntuple_td_train: occupancy");
+                    TC ? "ntuple_tc_train: occupancy" : "ntuple_td_train: occupancy");
     if (rc) return rc;
     const int sms = sm_count();
-    if (sms <= 0 || per_sm <= 0) return fail_arg("ntuple_td_train: the kernel does not fit on this device");
+    if (sms <= 0 || per_sm <= 0) return fail_arg(TC ? "ntuple_tc_train: the kernel does not fit on this device"
+                                           : "ntuple_td_train: the kernel does not fit on this device");
     const int64_t needed = ((int64_t)args.n + NT_THREADS - 1) / NT_THREADS;
     const int64_t resident = (int64_t)per_sm * sms;
     const unsigned grid = (unsigned)(needed < resident ? needed : resident);
     void* params[] = {const_cast<NtTdArgs*>(&args)};
     return check_cuda(cudaLaunchCooperativeKernel((const void*)kernel, dim3(grid), dim3(NT_THREADS), params,
                                                   (size_t)NT_SMEM_BYTES, st),
-                      "ntuple_td_train");
+                      TC ? "ntuple_tc_train" : "ntuple_td_train");
 }
 
 }  // namespace g2048
 
 using namespace g2048;
 
-extern "C" int64_t g2048_ntuple_td_scratch_bytes(int64_t n, int n_placements, int64_t n_weights) {
+namespace {
+
+int nt_fail(const char* who, const char* what) {
+    char msg[160];
+    snprintf(msg, sizeof(msg), "%s: %s", who, what);
+    return fail_arg(msg);
+}
+
+int64_t nt_scratch_bytes(int64_t n, int n_placements, int64_t n_weights, bool tc) {
     if (n < 1 || n > (1ll << 20) || n_placements < 1 || n_placements > G2048_NTUPLE_MAX_PLACEMENTS || n_weights < 1 ||
         n_weights > G2048_NTUPLE_MAX_WEIGHTS)
         return -1;
-    return nt_scratch_layout(n, n_placements, n_weights).bytes;
+    return nt_scratch_layout(n, n_placements, n_weights, tc).bytes;
 }
 
-extern "C" int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
-                                     int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
-                                     float* d_weights, int64_t n_weights, float alpha, const uint32_t* d_subs,
-                                     int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
-    G2048_REQUIRE(n >= 1 && n <= (1ll << 20), "ntuple_td_train: n must be in [1, 2^20]");
-    G2048_REQUIRE(n_steps >= 0, "ntuple_td_train: n_steps must be >= 0");
-    G2048_REQUIRE(alpha >= 0.0f && alpha <= 3.402823466e38f, "ntuple_td_train: alpha must be finite and >= 0");
-    G2048_REQUIRE(rng_mode == G2048_RNG_ORIGINAL || rng_mode == G2048_RNG_PARTITIONABLE, "ntuple_td_train: rng_mode");
-    int rc = ntuple_check(h_placements, n_placements, n_weights, "ntuple_td_train: invalid network");
+// g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train: the checks, then one launch
+int nt_train(const char* who, bool tc, uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+             int64_t n, const G2048TuplePlacement* h_placements, int n_placements, float* d_weights, int64_t n_weights,
+             double* d_err_sum, double* d_abs_err_sum, float alpha, const uint32_t* d_subs, int64_t n_steps,
+             int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+    if (!(n >= 1 && n <= (1ll << 20))) return nt_fail(who, "n must be in [1, 2^20]");
+    if (!(n_steps >= 0)) return nt_fail(who, "n_steps must be >= 0");
+    if (!(alpha >= 0.0f && alpha <= 3.402823466e38f)) return nt_fail(who, "alpha must be finite and >= 0");
+    if (!(rng_mode == G2048_RNG_ORIGINAL || rng_mode == G2048_RNG_PARTITIONABLE)) return nt_fail(who, "rng_mode");
+    char invalid[64];
+    snprintf(invalid, sizeof(invalid), "%s: invalid network", who);
+    int rc = ntuple_check(h_placements, n_placements, n_weights, invalid);
     if (rc) return rc;
-    G2048_REQUIRE(d_boards && d_after && d_scores && d_lengths && d_weights && d_scratch, "ntuple_td_train: pointers");
-    G2048_REQUIRE(n_steps == 0 || d_subs, "ntuple_td_train: pointers");
-    G2048_REQUIRE(((uintptr_t)d_boards & 7u) == 0 && ((uintptr_t)d_after & 7u) == 0 && ((uintptr_t)d_scratch & 7u) == 0 &&
-                      ((uintptr_t)d_subs & 7u) == 0 && ((uintptr_t)d_stats & 7u) == 0,
-                  "ntuple_td_train: d_boards, d_after, d_subs, d_scratch and d_stats must be 8-byte aligned");
-    G2048_REQUIRE(((uintptr_t)d_scores & 3u) == 0 && ((uintptr_t)d_lengths & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0,
-                  "ntuple_td_train: d_scores, d_lengths and d_weights must be 4-byte aligned");
+    if (!(d_boards && d_after && d_scores && d_lengths && d_weights && d_scratch)) return nt_fail(who, "pointers");
+    if (!(n_steps == 0 || d_subs)) return nt_fail(who, "pointers");
+    if (tc && !(d_err_sum && d_abs_err_sum)) return nt_fail(who, "pointers");
+    if (!(((uintptr_t)d_boards & 7u) == 0 && ((uintptr_t)d_after & 7u) == 0 && ((uintptr_t)d_scratch & 7u) == 0 &&
+          ((uintptr_t)d_subs & 7u) == 0 && ((uintptr_t)d_stats & 7u) == 0))
+        return nt_fail(who, "d_boards, d_after, d_subs, d_scratch and d_stats must be 8-byte aligned");
+    if (tc && !(((uintptr_t)d_err_sum & 7u) == 0 && ((uintptr_t)d_abs_err_sum & 7u) == 0))
+        return nt_fail(who, "d_err_sum and d_abs_err_sum must be 8-byte aligned");
+    if (!(((uintptr_t)d_scores & 3u) == 0 && ((uintptr_t)d_lengths & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0))
+        return nt_fail(who, "d_scores, d_lengths and d_weights must be 4-byte aligned");
     if (n_steps == 0) return G2048_OK;
-    const NtScratch lay = nt_scratch_layout(n, n_placements, n_weights);
+    const NtScratch lay = nt_scratch_layout(n, n_placements, n_weights, tc);
     NtTdArgs args;
     args.boards = (u64*)d_boards;
     args.after = (u64*)d_after;
@@ -369,7 +421,43 @@ extern "C" int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint
     args.list_len = (uint32_t*)((uint8_t*)d_scratch + lay.len_off);
     args.stats = (unsigned long long*)d_stats;
     ntuple_net(args.net, h_placements, n_placements, d_weights);
+    args.abs_acc = tc ? (unsigned long long*)((uint8_t*)d_scratch + lay.abs_off) : nullptr;
+    args.err_sum = tc ? d_err_sum : nullptr;
+    args.abs_err_sum = tc ? d_abs_err_sum : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
-    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE>(args, st);
-    return launch_ntuple_td<G2048_RNG_ORIGINAL>(args, st);
+    if (tc) {
+        if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, true>(args, st);
+        return launch_ntuple_td<G2048_RNG_ORIGINAL, true>(args, st);
+    }
+    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, false>(args, st);
+    return launch_ntuple_td<G2048_RNG_ORIGINAL, false>(args, st);
+}
+
+}  // namespace
+
+extern "C" int64_t g2048_ntuple_td_scratch_bytes(int64_t n, int n_placements, int64_t n_weights) {
+    return nt_scratch_bytes(n, n_placements, n_weights, false);
+}
+
+extern "C" int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                     int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                     float* d_weights, int64_t n_weights, float alpha, const uint32_t* d_subs,
+                                     int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+    return nt_train("ntuple_td_train", false, d_boards, d_after, d_scores, d_lengths, n, h_placements, n_placements,
+                    d_weights, n_weights, nullptr, nullptr, alpha, d_subs, n_steps, rng_mode, d_scratch, d_stats,
+                    stream);
+}
+
+extern "C" int64_t g2048_ntuple_tc_scratch_bytes(int64_t n, int n_placements, int64_t n_weights) {
+    return nt_scratch_bytes(n, n_placements, n_weights, true);
+}
+
+extern "C" int g2048_ntuple_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                     int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                     float* d_weights, int64_t n_weights, double* d_err_sum, double* d_abs_err_sum,
+                                     float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
+                                     void* d_scratch, uint64_t* d_stats, void* stream) {
+    return nt_train("ntuple_tc_train", true, d_boards, d_after, d_scores, d_lengths, n, h_placements, n_placements,
+                    d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha, d_subs, n_steps, rng_mode, d_scratch,
+                    d_stats, stream);
 }

@@ -15,11 +15,11 @@ from .runs import BatchRunner, FixedHorizonRunner, FixedRollout, FlatRollout, Pa
 from .state import State
 from .stats import RunningStatsVec
 from .ntuple import NTupleNetwork
-from .td import NTupleTDLearner, TDLearner
+from .td import NTupleTCLearner, NTupleTDLearner, TDLearner
 
 __all__ = [
     "ACTION_DIM", "BOARD_DIM", "BOARD_FLAT_DIM", "OBS_DIM", "BatchRunner", "DevicePPOBatches", "ExpectimaxPolicy", "ExpectimaxValues", "FixedHorizonRunner", "FixedRollout", "FlatRollout",
-    "MonteCarloPolicy", "NTupleNetwork", "NTupleTDLearner", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
+    "MonteCarloPolicy", "NTupleNetwork", "NTupleTCLearner", "NTupleTDLearner", "PPODataset", "PPOIterationLoop", "PackedRollout", "PlayoutValues",
     "RolloutBuffer", "RunningStatsVec", "State", "TDLearner", "TorchActionFunction", "act_drul", "act_randomly", "compute_gae",
     "create_ppo_dataloader", "default_row_values", "engine", "expectimax_values", "keys", "playout_values", "run_actions_batch", "run_actions_max_tile",
 ]

@@ -382,6 +382,36 @@ def ntuple_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Ten
          ptr(scratch), ptr(stats), stream_ptr())
 
 
+def ntuple_tc_scratch(n: int, placements: np.ndarray, n_weights: int, device) -> torch.Tensor:
+    """Zeroed scratch of g2048_ntuple_tc_train for n envs and this network (every call leaves it zeroed)."""
+    size = int(N.lib.g2048_ntuple_tc_scratch_bytes(n, placements.shape[0], n_weights))
+    if size < 0:
+        raise ValueError("ntuple_tc_scratch: invalid sizes")
+    return torch.zeros(size // 8, dtype=torch.int64, device=device)
+
+
+def ntuple_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                    placements: np.ndarray, weights: torch.Tensor, err_sum: torch.Tensor, abs_err_sum: torch.Tensor,
+                    alpha: float, subs: torch.Tensor, rng_mode: int, scratch: torch.Tensor,
+                    stats: torch.Tensor | None = None) -> None:
+    """``subs.shape[0]`` synchronous temporal-coherence steps of an n-tuple network (g2048_ntuple_tc_train): as
+    ``ntuple_td_train``, and in place on ``err_sum`` / ``abs_err_sum`` (E and A: float64, the network's n_weights
+    each; zeros at the start of a run).  ``scratch``: from ``ntuple_tc_scratch``."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    for s in (err_sum, abs_err_sum):
+        assert s.dtype == torch.float64 and s.is_contiguous() and s.numel() == weights.numel()
+    need = int(N.lib.g2048_ntuple_tc_scratch_bytes(n, placements.shape[0], weights.numel()))
+    if need < 0 or scratch.numel() * scratch.element_size() < need:
+        raise ValueError(f"ntuple_tc_train: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch "
+                         f"and network need {need} (ntuple_tc_scratch)")
+    call("g2048_ntuple_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, _placements_ptr(placements),
+         placements.shape[0], ptr(weights), weights.numel(), ptr(err_sum), ptr(abs_err_sum), float(alpha),
+         ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
+
+
 def expectimax_values_ntuple(boards: torch.Tensor, depth: int, placements: np.ndarray, weights: torch.Tensor,
                              reward_weight: float = 0.0, counters: torch.Tensor | None = None) -> torch.Tensor:
     """``expectimax_values`` with V of an n-tuple network at the leaves (g2048_expectimax_values_ntuple): (n, 4)

@@ -13,6 +13,8 @@ steps).  A call of ``train`` is one launch of ``g2048_td_train`` (include/g2048.
 
 ``NTupleTDLearner`` learns an n-tuple network (``g2048.NTupleNetwork``) the same way, through
 ``g2048_ntuple_td_train``: V in place of H, and the update at every placement of the previous afterstate.
+``NTupleTCLearner`` learns it by temporal coherence (``g2048_ntuple_tc_train``): the same step, with every weight's
+step scaled by |E| / A, its running sum of errors over the sum of their absolute values.
 """
 from __future__ import annotations
 
@@ -30,6 +32,9 @@ from .ntuple import NTupleNetwork, check_placements, _check_weights
 DEFAULT_ALPHA = 0.1
 # the step size of the round-8 sweep on one B200 whose greedy 4x6 player scored best (profiles/README.md, round 8)
 DEFAULT_NTUPLE_ALPHA = 0.02
+# round 9: TD's default, so that no TC step is larger than the TD step it starts as (beta <= 1, and from E = A = 0 a TC
+# step is a TD step with the same alpha; profiles/README.md, round 9)
+DEFAULT_NTUPLE_TC_ALPHA = DEFAULT_NTUPLE_ALPHA
 MAX_BATCH = 1 << 20
 _FLT_MAX = float(np.finfo(np.float32).max)
 
@@ -191,7 +196,10 @@ class NTupleTDLearner(_BatchTDLearner):
         if _resolved(self.network.weights.device) != _resolved(self.device):
             raise ValueError(f"the network's weights are on {self.network.weights.device}, the learner runs on {self.device}")
         self._init_envs(init_seed)
-        self._scratch = E.ntuple_td_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
+        self._scratch = self._new_scratch()
+
+    def _new_scratch(self) -> torch.Tensor:
+        return E.ntuple_td_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
 
     @property
     def weights(self) -> torch.Tensor:
@@ -217,3 +225,61 @@ class NTupleTDLearner(_BatchTDLearner):
 
     def _load_values(self, weights) -> None:
         self.network.weights.copy_(weights.to(self.device))
+
+
+def _check_sums(sums, n_weights: int, name: str) -> torch.Tensor:
+    """A checkpoint's E or A: float64 (n_weights,) finite values as a tensor, or ValueError."""
+    if sums is None:
+        raise ValueError(f"checkpoint has no {name} (it was not written by NTupleTCLearner)")
+    t = sums.detach() if isinstance(sums, torch.Tensor) else torch.from_numpy(np.asarray(sums))
+    if t.dtype != torch.float64 or tuple(t.shape) != (n_weights,):
+        raise ValueError(f"{name} must be a float64 array of n_weights = {n_weights} values, got {t.dtype} {tuple(t.shape)}")
+    if not bool(torch.isfinite(t).all()):
+        raise ValueError(f"{name} must be finite")
+    return t
+
+
+class NTupleTCLearner(NTupleTDLearner):
+    """Learns an n-tuple network by synchronous batched temporal coherence (TC) learning: ``NTupleTDLearner``'s
+    greedy move, fixed-point errors, key chain and statistics, with every weight's step scaled by
+    ``beta = |E| / A`` (1 while A is 0).  ``err_sum`` (E) and ``abs_err_sum`` (A) are the float64 (n_weights,) device
+    sums of each weight's errors and of their absolute values, zero at construction; weights whose errors keep one
+    sign keep a large step, weights whose errors cancel stop moving (g2048_ntuple_tc_train, include/g2048.h).
+
+    ``network`` may hold weights learned before (for example by ``NTupleTDLearner``): TC starts from them with
+    E = A = 0.  ``state_dict`` / ``load_state_dict`` resume a run bit for bit, E and A included."""
+
+    def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
+                 alpha: float = DEFAULT_NTUPLE_TC_ALPHA, rng_mode=None, device=None):
+        super().__init__(init_seed, batch_size, network=network, alpha=alpha, rng_mode=rng_mode, device=device)
+        n_weights = self.network.n_weights
+        self.err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
+        self.abs_err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
+
+    def _new_scratch(self) -> torch.Tensor:
+        return E.ntuple_tc_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
+
+    def _launch(self, subs, stats) -> None:
+        net = self.network
+        E.ntuple_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
+                          self.err_sum, self.abs_err_sum, self.alpha, subs, self.rng_mode, self._scratch, stats)
+
+    def _values_state(self) -> dict:
+        out = super()._values_state()
+        out.update({"err_sum": self.err_sum.cpu().clone(), "abs_err_sum": self.abs_err_sum.cpu().clone()})
+        return out
+
+    def _check_values_state(self, state):
+        weights = super()._check_values_state(state)
+        n_weights = self.network.n_weights
+        err_sum = _check_sums(state.get("err_sum"), n_weights, "err_sum")
+        abs_err_sum = _check_sums(state.get("abs_err_sum"), n_weights, "abs_err_sum")
+        if bool((abs_err_sum < 0).any()):
+            raise ValueError("abs_err_sum must be >= 0")
+        return weights, err_sum, abs_err_sum
+
+    def _load_values(self, values) -> None:
+        weights, err_sum, abs_err_sum = values
+        super()._load_values(weights)
+        self.err_sum.copy_(err_sum.to(self.device))
+        self.abs_err_sum.copy_(abs_err_sum.to(self.device))

@@ -298,6 +298,34 @@ int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_sco
                           float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
                           void* d_scratch, uint64_t* d_stats, void* stream);
 
+/* Batched temporal coherence (TC) learning of an n-tuple network (Beal & Smith 1999; Jaskowski 2018): every weight
+ * has its own step size, scaled by how consistently its errors agree in sign.  Steps 1 to 3 are g2048_ntuple_td_train
+ * word for word, and step 2 also adds |fx(delta)| into abs[off_p + idx_p(after)] for each placement p (int64, the same
+ * 2^62 bound as acc).  Step 4, for every i with cnt[i] > 0, in double unless stated otherwise:
+ *     m    = (double)acc[i] / (4096.0 * (double)cnt[i])
+ *     beta = A[i] > 0 ? fmin(fabs(E[i]) / A[i], 1.0) : 1.0          (E and A as they were before this step)
+ *     W[i] = W[i] + alpha * (float)(beta * m)                       (float multiply and add, not fused)
+ *     E[i] = E[i] + (double)acc[i] / 4096.0
+ *     A[i] = A[i] + (double)abs[i] / 4096.0
+ * then acc[i] = abs[i] = cnt[i] = 0.  A weight whose errors keep one sign keeps beta near 1; one whose errors cancel
+ * stops moving.  |E| <= A holds exactly; the fmin absorbs the rounding of the two double sums.  From E = A = 0 one
+ * step equals one g2048_ntuple_td_train step with the same alpha, bit for bit.  With alpha = 0 W stays fixed while E
+ * and A still accumulate.
+ *   d_err_sum, d_abs_err_sum: E and A, float64[n_weights] each, 8-byte aligned, updated in place (zero at the start of
+ *           a run).  They are float64 because A only grows: by an estimate from the sizes, a hot entry at n = 2^16
+ *           can gain about 2^41 a step, so an int64 fixed-point A would reach 2^63 after a few million steps, and a
+ *           float32 A would stop absorbing increments long before that.
+ *   d_scratch: g2048_ntuple_tc_scratch_bytes(n, n_placements, n_weights) bytes (acc int64[n_weights], abs
+ *           int64[n_weights], cnt uint32[n_weights], the touched list, the two list lengths), zeroed by the caller
+ *           once; every call leaves it zeroed.  g2048_ntuple_tc_scratch_bytes returns -1 for invalid sizes.
+ * G2048_ERR_INVALID for everything g2048_ntuple_td_train rejects and for NULL or misaligned d_err_sum / d_abs_err_sum.
+ * The `lines` network through this entry point is TC learning of the row table. */
+int64_t g2048_ntuple_tc_scratch_bytes(int64_t n, int n_placements, int64_t n_weights);
+int g2048_ntuple_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths, int64_t n,
+                          const G2048TuplePlacement* h_placements, int n_placements, float* d_weights, int64_t n_weights,
+                          double* d_err_sum, double* d_abs_err_sum, float alpha, const uint32_t* d_subs,
+                          int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream);
+
 /* g2048_expectimax_values with V of an n-tuple network in place of H at the leaves: the same tree, float order, NaN
  * for illegal actions and counters.  d_weights: W, float[n_weights] (device, read-only while the call runs).  Depth 1
  * with reward_weight 1 is g2048_ntuple_td_train's greedy move. */

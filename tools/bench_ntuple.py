@@ -16,7 +16,14 @@ over a network (g2048_expectimax_values_ntuple); prints one JSON line.
   * search: expectimax leaves/s at depth 2 and 3 on bench_expectimax.py's 4 096 mid-game boards with the 4x6 network
     leaf next to the row table (L2 flushed before every timed launch).
 
-    python tools/bench_ntuple.py [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
+With --tc, the temporal coherence learner (g2048_ntuple_tc_train, g2048.NTupleTCLearner) instead:
+  * speed: TC and TD for the 4x6 network at n = 2^14, 2^16 and 2^18, their timed launches alternated in one process;
+  * the accumulate / apply split of both from the -DG2048_NTUPLE_PHASES build;
+  * an alpha sweep of TC from the zero 4x6 network at n = 2^16 (learning curves, greedy player on the seed-7 games);
+  * TC at its best alpha against TD at its default alpha 0.02 at equal steps (--sweep-steps and --long-steps): greedy
+    and depth-2 mean scores, the 2048 / 4096 / 8192 / 16384 reach rates, and the training wall time.
+
+    python tools/bench_ntuple.py [--tc] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
 """
 import argparse
 import json
@@ -41,21 +48,23 @@ from bench_playout import device_times, gpu_info, mid_game_boards  # noqa: E402
 
 SIZES = (1 << 14, 1 << 16, 1 << 18)
 ALPHAS = (0.001, 0.0025, 0.005, 0.01, 0.02, 0.03)
+TC_ALPHAS = (0.01, 0.02, 0.05, 0.1, 0.2, 0.5, 1.0)
 MODE = E.RNG_PARTITIONABLE
 
 
 def _timed(run, reps):
     run()  # warm-up: module load, row tables, and games in progress rather than fresh envs
     torch.cuda.synchronize()
-    times = []
-    for _ in range(reps):
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        run()
-        b.record()
-        torch.cuda.synchronize()
-        times.append(a.elapsed_time(b) * 1e-3)
-    return times
+    return [_timed_once(run) for _ in range(reps)]
+
+
+def _timed_once(run) -> float:
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    run()
+    b.record()
+    torch.cuda.synchronize()
+    return a.elapsed_time(b) * 1e-3
 
 
 def _row(name, n, steps, times, **extra):
@@ -73,6 +82,33 @@ def _ntuple_run(lr, subs):
                                      subs, MODE, lr._scratch)
 
 
+def _tc_run(lr, subs):
+    net = lr.network
+    return lambda: E.ntuple_tc_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements, net.weights,
+                                     lr.err_sum, lr.abs_err_sum, lr.alpha, subs, MODE, lr._scratch)
+
+
+def tc_speed(steps: int, reps: int = 3) -> list:
+    """TD and TC at each size: both warmed up, then their timed launches alternated."""
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        td = g2048.NTupleTDLearner(0, n, alpha=0.0025, rng_mode=MODE)
+        tc = g2048.NTupleTCLearner(0, n, alpha=0.0025, rng_mode=MODE)
+        runs = {"four_six_td": _ntuple_run(td, subs), "four_six_tc": _tc_run(tc, subs)}
+        for run in runs.values():
+            run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in runs}
+        for _ in range(reps):
+            for k, run in runs.items():
+                times[k].append(_timed_once(run))
+        out += [_row(k, n, steps, times[k]) for k in runs]
+        del td, tc, runs
+        torch.cuda.empty_cache()
+    return out
+
+
 def speed(steps: int, reps: int = 3) -> list:
     out = []
     subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
@@ -84,18 +120,23 @@ def speed(steps: int, reps: int = 3) -> list:
     return out
 
 
-def phase_probe(steps: int) -> list:
+def phase_probe(steps: int, tc: bool = False) -> list:
     """In a build with -DG2048_NTUPLE_PHASES: the accumulate / apply split of one launch of `steps` steps after a
     warm-up launch, as CTA 0 timed it (%globaltimer up to each phase's closing grid.sync()), and the entries listed
-    (touched) per step."""
+    (touched) per step.  With tc, the TC learner at each size after the TD learner."""
     out = []
     subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
-    for n in SIZES:
-        lr = g2048.NTupleTDLearner(0, n, alpha=0.0025, rng_mode=MODE)
+    for n, kind in [(n, k) for n in SIZES for k in (("td", "tc") if tc else ("td",))]:
+        lr = (g2048.NTupleTCLearner if kind == "tc" else g2048.NTupleTDLearner)(0, n, alpha=0.0025, rng_mode=MODE)
         net = lr.network
         stats = torch.zeros(32, dtype=torch.int64, device="cuda")
-        run = lambda st=None: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,  # noqa: E731
-                                                net.weights, lr.alpha, subs, MODE, lr._scratch, st)
+        if kind == "tc":
+            run = lambda st=None: E.ntuple_tc_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,  # noqa: E731
+                                                    net.weights, lr.err_sum, lr.abs_err_sum, lr.alpha, subs, MODE,
+                                                    lr._scratch, st)
+        else:
+            run = lambda st=None: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,  # noqa: E731
+                                                    net.weights, lr.alpha, subs, MODE, lr._scratch, st)
         run()
         torch.cuda.synchronize()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -105,6 +146,7 @@ def phase_probe(steps: int) -> list:
         torch.cuda.synchronize()
         acc_ns, apply_ns, listed = (int(x) for x in stats[8:11].tolist())
         out.append({"n": n, "steps": steps, "us_per_step": a.elapsed_time(b) * 1e3 / steps,
+                    **({"learner": kind} if tc else {}),
                     "accumulate_us_per_step": acc_ns / 1e3 / steps, "apply_us_per_step": apply_ns / 1e3 / steps,
                     "entries_listed_per_step": listed / steps})
         print(json.dumps(out[-1]), file=sys.stderr, flush=True)
@@ -113,15 +155,15 @@ def phase_probe(steps: int) -> list:
     return out
 
 
-def phases(steps: int) -> dict:
+def phases(steps: int, tc: bool = False) -> dict:
     """Builds the library with -DG2048_NTUPLE_PHASES into a temporary directory and runs phase_probe on it."""
     tmp = Path(tempfile.mkdtemp(prefix="g2048_ntuple_phases_"))
     lib = tmp / "libg2048_phases.so"
     subprocess.run(["make", "-C", str(ROOT / "2048-ppo-agent_b200" / "csrc"), "-j16", f"OUT={lib}", f"BUILD={tmp / 'build'}",
                     "EXTRA=-DG2048_NTUPLE_PHASES"], check=True, capture_output=True)
     env = dict(os.environ, G2048_LIB=str(lib))
-    res = subprocess.run([sys.executable, __file__, "--phase-probe", "--steps", str(steps)], env=env, capture_output=True,
-                         text=True, check=True)
+    res = subprocess.run([sys.executable, __file__, "--phase-probe", "--steps", str(steps)] + (["--tc"] if tc else []),
+                         env=env, capture_output=True, text=True, check=True)
     return {"build": "-DG2048_NTUPLE_PHASES", "rows": json.loads(res.stdout.strip().splitlines()[-1])}
 
 
@@ -157,7 +199,7 @@ def weights_size(steps: int, reps: int = 3) -> list:
 
 def _reach(summary, B):
     hist = summary["max_tile_hist"]
-    return {str(t): sum(v for k, v in hist.items() if k >= t) / B for t in (2048, 4096, 8192)}
+    return {str(t): sum(v for k, v in hist.items() if k >= t) / B for t in (2048, 4096, 8192, 16384)}
 
 
 def play(policy, B, seed=7) -> dict:
@@ -181,10 +223,10 @@ def _train(lr, total, block):
     return curve, time.perf_counter() - t0
 
 
-def sweep(n: int, total: int, block: int, B: int) -> tuple:
+def sweep(n: int, total: int, block: int, B: int, alphas=ALPHAS, learner=g2048.NTupleTDLearner) -> tuple:
     rows, best = [], None
-    for alpha in ALPHAS:
-        lr = g2048.NTupleTDLearner(0, n, alpha=alpha)
+    for alpha in alphas:
+        lr = learner(0, n, alpha=alpha)
         curve, wall = _train(lr, total, block)
         greedy = play(g2048.ExpectimaxPolicy(depth=1, network=lr.network, reward_weight=1.0), B)
         rows.append({"alpha": alpha, "n": n, "steps": total, "block": block, "train_seconds": round(wall, 2),
@@ -219,6 +261,41 @@ def search(reps: int, net) -> list:
     return out
 
 
+def equal_steps(tc_alpha: float, lengths, block: int, B: int, deep: int) -> list:
+    """TD at its default alpha against TC at tc_alpha, from the zero 4x6 network at n = 2^16 (seed 0), for each number
+    of steps: training wall time, learning curve, and the greedy and depth-2 players on the seed-7 games."""
+    out = []
+    for steps in lengths:
+        for name, learner, alpha in (("td", g2048.NTupleTDLearner, g2048.td.DEFAULT_NTUPLE_ALPHA),
+                                     ("tc", g2048.NTupleTCLearner, tc_alpha)):
+            lr = learner(0, 1 << 16, alpha=alpha)
+            curve, wall = _train(lr, steps, block)
+            row = {"learner": name, "alpha": alpha, "n": 1 << 16, "steps": steps, "block": block,
+                   "train_seconds": round(wall, 2), "curve_mean_score": curve}
+            for depth, games in ((1, B), (2, deep)):
+                row[f"depth{depth}"] = play(g2048.ExpectimaxPolicy(depth=depth, network=lr.network, reward_weight=1.0),
+                                            games)
+            out.append(row)
+            print(json.dumps(row), file=sys.stderr, flush=True)
+            del lr
+            torch.cuda.empty_cache()
+    return out
+
+
+def main_tc(args) -> None:
+    result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
+    if not args.skip_speed:
+        result["speed"] = tc_speed(args.steps)
+        result["phases"] = phases(args.steps, tc=True)
+    if not args.speed_only:
+        rows, (_, alpha, _, _) = sweep(1 << 16, args.sweep_steps, args.block, args.games, TC_ALPHAS,
+                                       g2048.NTupleTCLearner)
+        result["tc_sweep"] = rows
+        result["equal_steps"] = equal_steps(alpha, (args.sweep_steps, args.long_steps), args.block, args.games,
+                                            args.deep_games)
+    _emit(result, args.out)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=500, help="batch steps per timed launch")
@@ -229,11 +306,16 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--speed-only", action="store_true", help="speed, phases, lines and n_weights only")
     ap.add_argument("--skip-speed", action="store_true", help="the sweep, search and players only")
+    ap.add_argument("--tc", action="store_true", help="the temporal coherence learner against TD (see above)")
+    ap.add_argument("--long-steps", type=int, default=40000, help="the longer equal-steps comparison of --tc")
     ap.add_argument("--phase-probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if args.phase_probe:
-        print(json.dumps(phase_probe(args.steps)))
+        print(json.dumps(phase_probe(args.steps, args.tc)))
+        return
+    if args.tc:
+        main_tc(args)
         return
     result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident); flushed for search"}
     if not args.skip_speed:
