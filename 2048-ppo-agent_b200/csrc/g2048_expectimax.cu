@@ -107,11 +107,26 @@ struct XmRowLeaf {
 };
 
 // ... or an n-tuple network (g2048_expectimax_values_ntuple): V at the leaves, its placements read from the parameter's
-// constant bank
+// constant bank ...
 struct XmTupleLeaf {
     using Param = NtNet;
     static __device__ __forceinline__ const float* table(const Param&) { return nullptr; }
     static __device__ __forceinline__ float value(const XmCtx&, const Param& net, u64 b, u64) { return nt_value<false>(net, b); }
+};
+
+// ... or a multi-stage n-tuple network (g2048_expectimax_values_ntuple_staged): V_S at the leaves, the stage taken
+// from each leaf board
+struct XmStagedTupleNet {
+    NtNet net;
+    NtStages stages;
+};
+
+struct XmStagedTupleLeaf {
+    using Param = XmStagedTupleNet;
+    static __device__ __forceinline__ const float* table(const Param&) { return nullptr; }
+    static __device__ __forceinline__ float value(const XmCtx&, const Param& p, u64 b, u64) {
+        return nt_value_staged<false>(p.net, p.stages, b);
+    }
 };
 
 // Item j < n * 4 is (board j / 4, first action j % 4), one warp each.
@@ -286,4 +301,26 @@ extern "C" int g2048_expectimax_values_ntuple(const uint64_t* d_boards, int64_t 
     NtNet net;
     ntuple_net(net, h_placements, n_placements, d_weights);
     return launch_expectimax_leaf<XmTupleLeaf>(depth, d_boards, n, net, reward_weight, d_q, d_counters, stream);
+}
+
+extern "C" int g2048_expectimax_values_ntuple_staged(const uint64_t* d_boards, int64_t n, int depth,
+                                                     const G2048TuplePlacement* h_placements, int n_placements,
+                                                     const G2048TupleStages* h_stages, const float* d_weights,
+                                                     int64_t n_weights, float reward_weight, float* d_q,
+                                                     uint64_t* d_counters, void* stream) {
+    G2048_REQUIRE(depth >= 1 && depth <= 4, "expectimax_values_ntuple_staged: depth must be in 1..4");
+    G2048_REQUIRE(n >= 0 && n < (1ll << 29), "expectimax_values_ntuple_staged: n must be in [0, 2^29)");
+    G2048_REQUIRE(((uintptr_t)d_q & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0,
+                  "expectimax_values_ntuple_staged: d_q and d_weights must be 4-byte aligned");
+    int rc = ntuple_check(h_placements, n_placements, n_weights, "expectimax_values_ntuple_staged: invalid network");
+    if (rc) return rc;
+    rc = ntuple_stages_check(h_stages, h_placements, n_placements, n_weights,
+                             "expectimax_values_ntuple_staged: invalid stages");
+    if (rc) return rc;
+    if (n == 0) return G2048_OK;
+    G2048_REQUIRE(d_boards && d_weights && d_q, "expectimax_values_ntuple_staged: pointers");
+    XmStagedTupleNet p;
+    ntuple_net(p.net, h_placements, n_placements, d_weights);
+    p.stages = ntuple_stages(*h_stages);
+    return launch_expectimax_leaf<XmStagedTupleLeaf>(depth, d_boards, n, p, reward_weight, d_q, d_counters, stream);
 }

@@ -26,6 +26,12 @@
 // entry's step by beta = |E[i]| / A[i] from the entry's float64 running sums, then adds the step's sums to E and A.
 // Only the apply phase touches E and A, one thread per listed entry, and grid.sync() orders the steps, so they use
 // ordinary loads and stores.  With TC = false none of it is compiled in.
+//
+// Multi-stage networks (g2048_ntuple_staged_td_train / _tc_train, the STAGED instantiations): each of the 5 boards
+// valued per env gets its stage base stage(b) * stride once, before the placement loop, and every entry of that board
+// is moved by it; the accumulate phase uses the previous afterstate's base.  Nothing else changes: the listing, the
+// apply walk and the fixed-point sums work on entries, whatever stage they belong to.  With STAGED = false none of it
+// is compiled in.
 #include <cooperative_groups.h>
 
 #include "g2048_ntuple.cuh"
@@ -89,6 +95,8 @@ struct NtTdArgs {
     unsigned long long* abs_acc;  // the sums of |fx|, next to acc
     double* err_sum;              // E
     double* abs_err_sum;          // A
+    // STAGED only (after the TC fields, so the unstaged instantiations see the parameter layout they always had)
+    NtStages stages;
 };
 
 // fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64, to nearest even (the multiply by a power of two is exact)
@@ -107,7 +115,7 @@ __device__ __forceinline__ void nt_append(bool first, uint32_t i, uint32_t* list
     }
 }
 
-template <int MODE, bool TC>
+template <int MODE, bool TC, bool STAGED>
 __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_constant__ NtTdArgs a) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     __shared__ unsigned long long s_stats[G2048_PLAY_STATS_WORDS];
@@ -164,7 +172,16 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
             }
             cand[4] = aft;
             float v[5];
-            nt_values<true, 5>(a.net, cand, v);
+            uint32_t aft_base = 0u;  // the previous afterstate's stage base
+            if constexpr (STAGED) {
+                uint32_t base[5];
+#pragma unroll
+                for (int j = 0; j < 5; ++j) base[j] = nt_stage_base(a.stages, cand[j]);
+                nt_values_at<true, 5>(a.net, cand, base, v);
+                aft_base = base[4];
+            } else {
+                nt_values<true, 5>(a.net, cand, v);
+            }
             float target = 0.0f;
             u64 best = 0ull;
             uint32_t best_r = 0u;
@@ -186,7 +203,7 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
             __syncwarp();
 #pragma unroll 1
             for (uint32_t p = 0; p < P; ++p) {
-                const uint32_t i = nt_entry(a.net.pl[p], aft);
+                const uint32_t i = aft_base + nt_entry(a.net.pl[p], aft);
                 const unsigned group = __match_any_sync(0xFFFFFFFFu, update ? i : 0xFFFFFFFFu);  // i < 2^28
                 bool first = false;
                 if (update && lane == (unsigned)(__ffs((int)group) - 1)) {
@@ -197,6 +214,9 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
                         if constexpr (TC) abs_sum += fx < 0 ? -fx : fx;
                     }
                     const unsigned count = (unsigned)__popc((int)group);
+                    // index 0 of placement p in stage 0.  The per-CTA sums are flushed to off_p, so this relies on
+                    // no other entry of p equalling off_p: an entry of stage s >= 1 is at least stride + off_p with
+                    // stride >= 1, so the later stages' index 0 goes through the global atomics.
                     if (i == a.net.pl[p].offset) {
                         atomicAdd(&s_acc0[p], (unsigned long long)sum);
                         if constexpr (TC) atomicAdd(&s_abs0[p], (unsigned long long)abs_sum);
@@ -322,24 +342,28 @@ __global__ void build_ntuple_row_tables_kernel() {
     build_row_table_entry(row);
 }
 
-template <int MODE, bool TC>
-static int launch_ntuple_td(const NtTdArgs& args, cudaStream_t st) {
-    auto kernel = ntuple_td_kernel<MODE, TC>;
+// who: the entry point's name, which prefixes every message
+template <int MODE, bool TC, bool STAGED>
+static int launch_ntuple_td(const char* who, const NtTdArgs& args, cudaStream_t st) {
+    auto kernel = ntuple_td_kernel<MODE, TC, STAGED>;
+    char msg[128];
+    auto what = [&](const char* s) {
+        snprintf(msg, sizeof(msg), "%s%s%s", who, *s ? ": " : "", s);
+        return msg;
+    };
     static bool configured_on[64] = {false};
     bool* configured = device_once_flag(configured_on);
     if (!configured) return fail_arg("no CUDA device");
     int dev = 0;
-    int rc = check_cuda(cudaGetDevice(&dev), TC ? "ntuple_tc_train: device" : "ntuple_td_train: device");
+    int rc = check_cuda(cudaGetDevice(&dev), what("device"));
     if (rc) return rc;
     if (!*configured) {
         int coop = 0;
-        rc = check_cuda(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev),
-                        TC ? "ntuple_tc_train: device attribute" : "ntuple_td_train: device attribute");
+        rc = check_cuda(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev), what("device attribute"));
         if (rc) return rc;
-        if (!coop) return fail_arg(TC ? "ntuple_tc_train: the device does not support cooperative launches"
-                             : "ntuple_td_train: the device does not support cooperative launches");
+        if (!coop) return fail_arg(what("the device does not support cooperative launches"));
         rc = check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, NT_SMEM_BYTES),
-                        TC ? "ntuple_tc_train: shared memory attribute" : "ntuple_td_train: shared memory attribute");
+                        what("shared memory attribute"));
         if (rc) return rc;
         *configured = true;
     }
@@ -347,18 +371,17 @@ static int launch_ntuple_td(const NtTdArgs& args, cudaStream_t st) {
     if (rc) return rc;
     int per_sm = 0;
     rc = check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT_THREADS, NT_SMEM_BYTES),
-                    TC ? "ntuple_tc_train: occupancy" : "ntuple_td_train: occupancy");
+                    what("occupancy"));
     if (rc) return rc;
     const int sms = sm_count();
-    if (sms <= 0 || per_sm <= 0) return fail_arg(TC ? "ntuple_tc_train: the kernel does not fit on this device"
-                                           : "ntuple_td_train: the kernel does not fit on this device");
+    if (sms <= 0 || per_sm <= 0) return fail_arg(what("the kernel does not fit on this device"));
     const int64_t needed = ((int64_t)args.n + NT_THREADS - 1) / NT_THREADS;
     const int64_t resident = (int64_t)per_sm * sms;
     const unsigned grid = (unsigned)(needed < resident ? needed : resident);
     void* params[] = {const_cast<NtTdArgs*>(&args)};
     return check_cuda(cudaLaunchCooperativeKernel((const void*)kernel, dim3(grid), dim3(NT_THREADS), params,
                                                   (size_t)NT_SMEM_BYTES, st),
-                      TC ? "ntuple_tc_train" : "ntuple_td_train");
+                      what(""));
 }
 
 }  // namespace g2048
@@ -380,11 +403,19 @@ int64_t nt_scratch_bytes(int64_t n, int n_placements, int64_t n_weights, bool tc
     return nt_scratch_layout(n, n_placements, n_weights, tc).bytes;
 }
 
-// g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train: the checks, then one launch
-int nt_train(const char* who, bool tc, uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
-             int64_t n, const G2048TuplePlacement* h_placements, int n_placements, float* d_weights, int64_t n_weights,
-             double* d_err_sum, double* d_abs_err_sum, float alpha, const uint32_t* d_subs, int64_t n_steps,
-             int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+template <bool TC, bool STAGED>
+int nt_launch(const char* who, int rng_mode, const NtTdArgs& args, cudaStream_t st) {
+    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, TC, STAGED>(who, args, st);
+    return launch_ntuple_td<G2048_RNG_ORIGINAL, TC, STAGED>(who, args, st);
+}
+
+// g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train, and their staged forms (h_stages not
+// NULL; staged = false passes NULL): the checks, then one launch
+int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+             uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+             const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, double* d_err_sum,
+             double* d_abs_err_sum, float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
+             void* d_scratch, uint64_t* d_stats, void* stream) {
     if (!(n >= 1 && n <= (1ll << 20))) return nt_fail(who, "n must be in [1, 2^20]");
     if (!(n_steps >= 0)) return nt_fail(who, "n_steps must be >= 0");
     if (!(alpha >= 0.0f && alpha <= 3.402823466e38f)) return nt_fail(who, "alpha must be finite and >= 0");
@@ -393,6 +424,11 @@ int nt_train(const char* who, bool tc, uint64_t* d_boards, uint64_t* d_after, ui
     snprintf(invalid, sizeof(invalid), "%s: invalid network", who);
     int rc = ntuple_check(h_placements, n_placements, n_weights, invalid);
     if (rc) return rc;
+    if (staged) {
+        snprintf(invalid, sizeof(invalid), "%s: invalid stages", who);
+        rc = ntuple_stages_check(h_stages, h_placements, n_placements, n_weights, invalid);
+        if (rc) return rc;
+    }
     if (!(d_boards && d_after && d_scores && d_lengths && d_weights && d_scratch)) return nt_fail(who, "pointers");
     if (!(n_steps == 0 || d_subs)) return nt_fail(who, "pointers");
     if (tc && !(d_err_sum && d_abs_err_sum)) return nt_fail(who, "pointers");
@@ -424,13 +460,10 @@ int nt_train(const char* who, bool tc, uint64_t* d_boards, uint64_t* d_after, ui
     args.abs_acc = tc ? (unsigned long long*)((uint8_t*)d_scratch + lay.abs_off) : nullptr;
     args.err_sum = tc ? d_err_sum : nullptr;
     args.abs_err_sum = tc ? d_abs_err_sum : nullptr;
+    args.stages = staged ? ntuple_stages(*h_stages) : NtStages{0ull, 0u};
     cudaStream_t st = (cudaStream_t)stream;
-    if (tc) {
-        if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, true>(args, st);
-        return launch_ntuple_td<G2048_RNG_ORIGINAL, true>(args, st);
-    }
-    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, false>(args, st);
-    return launch_ntuple_td<G2048_RNG_ORIGINAL, false>(args, st);
+    if (staged) return tc ? nt_launch<true, true>(who, rng_mode, args, st) : nt_launch<false, true>(who, rng_mode, args, st);
+    return tc ? nt_launch<true, false>(who, rng_mode, args, st) : nt_launch<false, false>(who, rng_mode, args, st);
 }
 
 }  // namespace
@@ -443,9 +476,9 @@ extern "C" int g2048_ntuple_td_train(uint64_t* d_boards, uint64_t* d_after, uint
                                      int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
                                      float* d_weights, int64_t n_weights, float alpha, const uint32_t* d_subs,
                                      int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
-    return nt_train("ntuple_td_train", false, d_boards, d_after, d_scores, d_lengths, n, h_placements, n_placements,
-                    d_weights, n_weights, nullptr, nullptr, alpha, d_subs, n_steps, rng_mode, d_scratch, d_stats,
-                    stream);
+    return nt_train("ntuple_td_train", false, false, d_boards, d_after, d_scores, d_lengths, n, h_placements,
+                    n_placements, nullptr, d_weights, n_weights, nullptr, nullptr, alpha, d_subs, n_steps, rng_mode,
+                    d_scratch, d_stats, stream);
 }
 
 extern "C" int64_t g2048_ntuple_tc_scratch_bytes(int64_t n, int n_placements, int64_t n_weights) {
@@ -457,7 +490,28 @@ extern "C" int g2048_ntuple_tc_train(uint64_t* d_boards, uint64_t* d_after, uint
                                      float* d_weights, int64_t n_weights, double* d_err_sum, double* d_abs_err_sum,
                                      float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
                                      void* d_scratch, uint64_t* d_stats, void* stream) {
-    return nt_train("ntuple_tc_train", true, d_boards, d_after, d_scores, d_lengths, n, h_placements, n_placements,
-                    d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha, d_subs, n_steps, rng_mode, d_scratch,
-                    d_stats, stream);
+    return nt_train("ntuple_tc_train", true, false, d_boards, d_after, d_scores, d_lengths, n, h_placements,
+                    n_placements, nullptr, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha, d_subs, n_steps,
+                    rng_mode, d_scratch, d_stats, stream);
+}
+
+extern "C" int g2048_ntuple_staged_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                            uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                            int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                            int64_t n_weights, float alpha, const uint32_t* d_subs, int64_t n_steps,
+                                            int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+    return nt_train("ntuple_staged_td_train", false, true, d_boards, d_after, d_scores, d_lengths, n, h_placements,
+                    n_placements, h_stages, d_weights, n_weights, nullptr, nullptr, alpha, d_subs, n_steps, rng_mode,
+                    d_scratch, d_stats, stream);
+}
+
+extern "C" int g2048_ntuple_staged_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                            uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                            int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                            int64_t n_weights, double* d_err_sum, double* d_abs_err_sum, float alpha,
+                                            const uint32_t* d_subs, int64_t n_steps, int rng_mode, void* d_scratch,
+                                            uint64_t* d_stats, void* stream) {
+    return nt_train("ntuple_staged_tc_train", true, true, d_boards, d_after, d_scores, d_lengths, n, h_placements,
+                    n_placements, h_stages, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha, d_subs, n_steps,
+                    rng_mode, d_scratch, d_stats, stream);
 }

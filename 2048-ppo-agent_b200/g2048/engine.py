@@ -355,6 +355,15 @@ def _placements_ptr(placements: np.ndarray) -> int:
     return placements.ctypes.data
 
 
+def _stages_ptr(stages: np.ndarray, placements: np.ndarray, n_weights: int) -> tuple[np.ndarray, int]:
+    """A checked copy of a G2048TupleStages record (``g2048.ntuple.STAGES_DTYPE``, ValueError when the staged entry
+    points would reject it) and its host pointer; keep the copy alive over the call."""
+    from .ntuple import check_stages
+
+    st = check_stages(stages, placements, n_weights)
+    return st, st.ctypes.data
+
+
 def ntuple_td_scratch(n: int, placements: np.ndarray, n_weights: int, device) -> torch.Tensor:
     """Zeroed scratch of g2048_ntuple_td_train for n envs and this network (every call leaves it zeroed)."""
     size = int(N.lib.g2048_ntuple_td_scratch_bytes(n, placements.shape[0], n_weights))
@@ -365,10 +374,12 @@ def ntuple_td_scratch(n: int, placements: np.ndarray, n_weights: int, device) ->
 
 def ntuple_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
                     placements: np.ndarray, weights: torch.Tensor, alpha: float, subs: torch.Tensor, rng_mode: int,
-                    scratch: torch.Tensor, stats: torch.Tensor | None = None) -> None:
+                    scratch: torch.Tensor, stats: torch.Tensor | None = None, stages: np.ndarray | None = None) -> None:
     """``subs.shape[0]`` synchronous TD(0) steps of an n-tuple network (g2048_ntuple_td_train), in place on the env
     state (as ``td_train``) and on ``weights`` (float32, the network's n_weights).  ``placements``: the host
-    G2048TuplePlacement array (``g2048.ntuple.PLACEMENT_DTYPE``).  ``scratch``: from ``ntuple_td_scratch``."""
+    G2048TuplePlacement array (``g2048.ntuple.PLACEMENT_DTYPE``).  ``scratch``: from ``ntuple_td_scratch``.
+    ``stages``: None, or a G2048TupleStages record (``g2048.ntuple.STAGES_DTYPE``) for a multi-stage network
+    (g2048_ntuple_staged_td_train)."""
     n = boards.shape[0]
     assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
     assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
@@ -377,6 +388,12 @@ def ntuple_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Ten
     if need < 0 or scratch.numel() * scratch.element_size() < need:
         raise ValueError(f"ntuple_td_train: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch "
                          f"and network need {need} (ntuple_td_scratch)")
+    if stages is not None:
+        st, st_ptr = _stages_ptr(stages, placements, weights.numel())
+        call("g2048_ntuple_staged_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+             _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), float(alpha),
+             ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
+        return
     call("g2048_ntuple_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, _placements_ptr(placements),
          placements.shape[0], ptr(weights), weights.numel(), float(alpha), ptr(_i32(subs)), subs.shape[0], rng_mode,
          ptr(scratch), ptr(stats), stream_ptr())
@@ -393,10 +410,11 @@ def ntuple_tc_scratch(n: int, placements: np.ndarray, n_weights: int, device) ->
 def ntuple_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
                     placements: np.ndarray, weights: torch.Tensor, err_sum: torch.Tensor, abs_err_sum: torch.Tensor,
                     alpha: float, subs: torch.Tensor, rng_mode: int, scratch: torch.Tensor,
-                    stats: torch.Tensor | None = None) -> None:
+                    stats: torch.Tensor | None = None, stages: np.ndarray | None = None) -> None:
     """``subs.shape[0]`` synchronous temporal-coherence steps of an n-tuple network (g2048_ntuple_tc_train): as
     ``ntuple_td_train``, and in place on ``err_sum`` / ``abs_err_sum`` (E and A: float64, the network's n_weights
-    each; zeros at the start of a run).  ``scratch``: from ``ntuple_tc_scratch``."""
+    each; zeros at the start of a run).  ``scratch``: from ``ntuple_tc_scratch``.  ``stages``: as for
+    ``ntuple_td_train`` (g2048_ntuple_staged_tc_train)."""
     n = boards.shape[0]
     assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
     assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
@@ -407,16 +425,32 @@ def ntuple_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Ten
     if need < 0 or scratch.numel() * scratch.element_size() < need:
         raise ValueError(f"ntuple_tc_train: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch "
                          f"and network need {need} (ntuple_tc_scratch)")
+    if stages is not None:
+        st, st_ptr = _stages_ptr(stages, placements, weights.numel())
+        call("g2048_ntuple_staged_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+             _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), ptr(err_sum),
+             ptr(abs_err_sum), float(alpha), ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats),
+             stream_ptr())
+        return
     call("g2048_ntuple_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, _placements_ptr(placements),
          placements.shape[0], ptr(weights), weights.numel(), ptr(err_sum), ptr(abs_err_sum), float(alpha),
          ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
 
 
 def expectimax_values_ntuple(boards: torch.Tensor, depth: int, placements: np.ndarray, weights: torch.Tensor,
-                             reward_weight: float = 0.0, counters: torch.Tensor | None = None) -> torch.Tensor:
+                             reward_weight: float = 0.0, counters: torch.Tensor | None = None,
+                             stages: np.ndarray | None = None) -> torch.Tensor:
     """``expectimax_values`` with V of an n-tuple network at the leaves (g2048_expectimax_values_ntuple): (n, 4)
-    float32 Q values, NaN where the action is illegal."""
+    float32 Q values, NaN where the action is illegal.  ``stages``: as for ``ntuple_td_train``
+    (g2048_expectimax_values_ntuple_staged)."""
     assert weights.dtype == torch.float32 and weights.is_contiguous()
+    if stages is not None:
+        st, st_ptr = _stages_ptr(stages, placements, weights.numel())
+        q = torch.empty((boards.shape[0], 4), dtype=torch.float32, device=boards.device)
+        call("g2048_expectimax_values_ntuple_staged", ptr(boards), boards.shape[0], depth, _placements_ptr(placements),
+             placements.shape[0], st_ptr, ptr(weights), weights.numel(), float(reward_weight), ptr(q), ptr(counters),
+             stream_ptr())
+        return q
     q = torch.empty((boards.shape[0], 4), dtype=torch.float32, device=boards.device)
     call("g2048_expectimax_values_ntuple", ptr(boards), boards.shape[0], depth, _placements_ptr(placements),
          placements.shape[0], ptr(weights), weights.numel(), float(reward_weight), ptr(q), ptr(counters), stream_ptr())

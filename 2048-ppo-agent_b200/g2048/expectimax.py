@@ -11,7 +11,8 @@ empty cell with a 2 (probability 0.9) or a 4 (0.1), and at depth ``depth`` (coun
 ``H(b) = sum of T[row] over the 4 rows and 4 columns``.  A move's value adds ``reward_weight`` times its merge reward.
 All arithmetic is float32 in a fixed order (include/g2048.h), so the values are bit-exact and a game is deterministic
 given the spawns.  With ``network=`` (a ``g2048.NTupleNetwork``) the leaves are the network's value V instead of H
-(``g2048_expectimax_values_ntuple``), with the same tree and float order.
+(``g2048_expectimax_values_ntuple``), with the same tree and float order; a multi-stage network takes each leaf's
+stage from the leaf board (``g2048_expectimax_values_ntuple_staged``).
 """
 from __future__ import annotations
 
@@ -131,7 +132,7 @@ def expectimax_values(boards, depth: int = 2, row_values=None, reward_weight: fl
     counters = torch.zeros(2, dtype=torch.int64, device=device)
     if network is not None:
         q = E.expectimax_values_ntuple(boards, int(depth), network.placements, network.weights_on(device),
-                                       float(reward_weight), counters)
+                                       float(reward_weight), counters, stages=network.stages)
     else:
         q = E.expectimax_values(boards, int(depth), _table_on(row_values, device), float(reward_weight), counters)
     return ExpectimaxValues(q, counters)

@@ -9,6 +9,12 @@ A network is an ordered list of placements over one flat float32 weight array ``
 board and indexes its table with their exponents (nibble j = the exponent in cells[j]):
 ``V(b) = W[off_0 + idx_0(b)] + ... + W[off_{P-1} + idx_{P-1}(b)]`` in float32, left to right (include/g2048.h).
 Placements with the same offset share a table: the 8 symmetric images of a tuple learn one set of weights.
+
+A multi-stage network (Yeh et al. 2016; Jaśkowski 2018) splits the game into S stages by the largest tile on the board,
+and gives each stage its own copy of every table, ``stage_stride`` entries after the previous stage's:
+``stage(b)`` is the number of ``stage_thresholds`` (tile exponents) that the board's largest exponent reaches, and
+``V_S(b) = W[stage(b) * stride + off_0 + idx_0(b)] + ...``.  ``NTupleNetwork.staged(net, (13,))`` splits a trained
+single-stage network into stages that start as copies of it.
 """
 from __future__ import annotations
 
@@ -21,6 +27,9 @@ from . import _native as N
 PLACEMENT_DTYPE = np.dtype([("offset", "<u4"), ("n_cells", "u1"), ("cells", "u1", (6,)), ("reserved", "u1")])
 MAX_PLACEMENTS = 64
 MAX_WEIGHTS = 1 << 28
+# G2048TupleStages (include/g2048.h), 20 bytes
+STAGES_DTYPE = np.dtype([("stride", "<u4"), ("n_thresholds", "u1"), ("thresholds", "u1", (15,))])
+MAX_STAGES = 16
 
 # the 8 symmetries of the square, as maps of (row, col), in the order of NTupleNetwork.from_tuples
 SYMMETRIES = (
@@ -75,6 +84,41 @@ def check_placements(placements, n_weights: int) -> np.ndarray:
     return pl.copy()
 
 
+def make_stages(thresholds, stride: int) -> np.ndarray:
+    """A (1,) STAGES_DTYPE array (a G2048TupleStages) from tile exponents and a stride, unchecked."""
+    thresholds = [int(t) for t in thresholds]
+    if len(thresholds) > MAX_STAGES - 1 or any(not 0 <= t < 256 for t in thresholds) or not 0 <= int(stride) < 1 << 32:
+        raise ValueError(f"stages have at most 15 thresholds in 1..15 and a uint32 stride, got {thresholds}, {stride}")
+    st = np.zeros(1, STAGES_DTYPE)
+    st[0]["stride"] = int(stride)
+    st[0]["n_thresholds"] = len(thresholds)
+    st[0]["thresholds"][: len(thresholds)] = thresholds
+    return st
+
+
+def check_stages(stages, placements, n_weights: int) -> np.ndarray:
+    """The stage checks of the staged C entry points (include/g2048.h), for a network that check_placements accepts: a
+    C-contiguous (1,) STAGES_DTYPE copy, or ValueError."""
+    st = np.ascontiguousarray(np.asarray(stages)).reshape(-1)
+    if st.dtype != STAGES_DTYPE or st.shape[0] != 1:
+        raise ValueError("stages must be one STAGES_DTYPE record")
+    k, stride = int(st[0]["n_thresholds"]), int(st[0]["stride"])
+    thresholds = [int(t) for t in st[0]["thresholds"]]
+    if k > MAX_STAGES - 1:
+        raise ValueError(f"a network has at most 15 stage thresholds, got {k}")
+    if any(not 1 <= t <= 15 for t in thresholds[:k]) or any(a >= b for a, b in zip(thresholds[:k], thresholds[1:k])):
+        raise ValueError(f"stage thresholds must be strictly increasing tile exponents in 1..15, got {thresholds[:k]}")
+    if any(thresholds[k:]):
+        raise ValueError("unused stage threshold bytes must be 0")
+    if (k == 0) != (stride == 0):
+        raise ValueError(f"the stage stride must be 0 exactly for a single-stage network, got {stride} with {k + 1} stages")
+    pl = np.asarray(placements)
+    for i, p in enumerate(pl):
+        if k * stride + int(p["offset"]) + 16 ** int(p["n_cells"]) > int(n_weights):
+            raise ValueError(f"placement {i}: its table in the last stage exceeds n_weights = {n_weights}")
+    return st.copy()
+
+
 def _check_weights(weights, n_weights: int) -> torch.Tensor:
     w = weights.detach() if isinstance(weights, torch.Tensor) else torch.from_numpy(np.asarray(weights, np.float32))
     if w.numel() != n_weights:
@@ -87,12 +131,15 @@ def _check_weights(weights, n_weights: int) -> torch.Tensor:
 
 class NTupleNetwork:
     """``placements`` (PLACEMENT_DTYPE host array, 1..64 entries), ``n_weights`` (1 .. 2^28) and ``weights``, the
-    float32 (n_weights,) device tensor: zeros, or a copy of the given finite values.  The placements are checked as
-    the C entry points check them, before anything touches a device."""
+    float32 (n_weights,) device tensor: zeros, or a copy of the given finite values.  ``stage_thresholds`` (strictly
+    increasing tile exponents in 1..15, at most 15) and ``stage_stride`` (0 exactly when there are none) make it a
+    network of ``n_stages = len(stage_thresholds) + 1`` stages.  The placements and stages are checked as the C entry
+    points check them, before anything touches a device."""
 
-    def __init__(self, placements, n_weights: int, weights=None, device=None):
+    def __init__(self, placements, n_weights: int, weights=None, device=None, stage_thresholds=(), stage_stride: int = 0):
         self.placements = check_placements(placements, n_weights)
         self.n_weights = int(n_weights)
+        self._stages = check_stages(make_stages(stage_thresholds, stage_stride), self.placements, self.n_weights)
         if weights is not None:
             weights = _check_weights(weights, self.n_weights)
         device = N.require_cuda() if device is None else torch.device(device)
@@ -104,6 +151,40 @@ class NTupleNetwork:
     @property
     def n_placements(self) -> int:
         return int(self.placements.shape[0])
+
+    @property
+    def stage_thresholds(self) -> tuple[int, ...]:
+        return tuple(int(t) for t in self._stages[0]["thresholds"][: self._stages[0]["n_thresholds"]])
+
+    @property
+    def stage_stride(self) -> int:
+        return int(self._stages[0]["stride"])
+
+    @property
+    def n_stages(self) -> int:
+        return len(self.stage_thresholds) + 1
+
+    @property
+    def stages(self) -> np.ndarray | None:
+        """The G2048TupleStages record of the staged entry points, or None for a single-stage network, which takes the
+        unstaged ones."""
+        return self._stages if self.n_stages > 1 else None
+
+    @classmethod
+    def staged(cls, base: "NTupleNetwork", thresholds) -> "NTupleNetwork":
+        """``base`` split into ``len(thresholds) + 1`` stages at these tile exponents: its placements, stride =
+        ``base.n_weights``, and every stage starting as a copy of ``base.weights`` (whole-stage promotion), so that the
+        new network has exactly ``base``'s values until it learns.  ``base`` must have one stage."""
+        if not isinstance(base, NTupleNetwork) or base.n_stages != 1:
+            raise ValueError("staged() splits a single-stage NTupleNetwork")
+        thresholds = tuple(int(t) for t in thresholds)
+        n_stages = len(thresholds) + 1
+        n_weights = n_stages * base.n_weights
+        stride = base.n_weights if n_stages > 1 else 0
+        if n_weights > MAX_WEIGHTS:
+            raise ValueError(f"{n_stages} stages of {base.n_weights} weights exceed 2^28 weights")
+        check_stages(make_stages(thresholds, stride), base.placements, n_weights)  # before the copy touches a device
+        return cls(base.placements, n_weights, base.weights.repeat(n_stages), base.weights.device, thresholds, stride)
 
     @classmethod
     def from_tuples(cls, tuples, symmetric: bool = True, weights=None, device=None) -> "NTupleNetwork":

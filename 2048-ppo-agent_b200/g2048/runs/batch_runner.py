@@ -360,11 +360,12 @@ class BatchRunner:
         legal action and gets action 0, which the step ignores); the act sub key is not used."""
         fn = self._act_fn
         if fn.network is not None:
-            placements, weights = fn.network.placements, fn.network.weights_on(self.device)
+            net = fn.network
+            placements, weights, stages = net.placements, net.weights_on(self.device), net.stages
 
             def choose(live_boards, board_ids, sub_act):
                 return expectimax_best_actions(E.expectimax_values_ntuple(live_boards, int(fn.depth), placements, weights,
-                                                                          float(fn.reward_weight)))
+                                                                          float(fn.reward_weight), stages=stages))
 
             return self._run_eval_search(batch_size, choose)
         table = fn.table(self.device)

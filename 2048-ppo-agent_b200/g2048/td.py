@@ -14,7 +14,9 @@ steps).  A call of ``train`` is one launch of ``g2048_td_train`` (include/g2048.
 ``NTupleTDLearner`` learns an n-tuple network (``g2048.NTupleNetwork``) the same way, through
 ``g2048_ntuple_td_train``: V in place of H, and the update at every placement of the previous afterstate.
 ``NTupleTCLearner`` learns it by temporal coherence (``g2048_ntuple_tc_train``): the same step, with every weight's
-step scaled by |E| / A, its running sum of errors over the sum of their absolute values.
+step scaled by |E| / A, its running sum of errors over the sum of their absolute values.  A multi-stage network
+(``NTupleNetwork.staged``) is learned by the staged entry points, all its stages in one launch; a single-stage network
+takes the unstaged ones.
 """
 from __future__ import annotations
 
@@ -183,8 +185,9 @@ class NTupleTDLearner(_BatchTDLearner):
     learns the row table: the same greedy move, fixed-point update, key chain and statistics.
 
     ``network``: the ``NTupleNetwork`` whose ``weights`` are learned in place (default: a zero ``four_six()``).
-    ``state_dict`` / ``load_state_dict`` resume a run bit for bit; the checkpoint holds the placements, and a load
-    whose placements or n_weights differ from the learner's network is rejected before anything changes."""
+    ``state_dict`` / ``load_state_dict`` resume a run bit for bit; the checkpoint holds the placements and the stages,
+    and a load whose placements, n_weights or stages differ from the learner's network is rejected before anything
+    changes (a checkpoint without stages is a single-stage network's)."""
 
     def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
                  alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None):
@@ -208,11 +211,13 @@ class NTupleTDLearner(_BatchTDLearner):
     def _launch(self, subs, stats) -> None:
         net = self.network
         E.ntuple_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights, self.alpha,
-                          subs, self.rng_mode, self._scratch, stats)
+                          subs, self.rng_mode, self._scratch, stats, stages=net.stages)
 
     def _values_state(self) -> dict:
         net = self.network
-        return {"placements": net.placements.copy(), "n_weights": net.n_weights, "weights": net.weights.cpu().clone()}
+        return {"placements": net.placements.copy(), "n_weights": net.n_weights,
+                "stage_thresholds": list(net.stage_thresholds), "stage_stride": net.stage_stride,
+                "weights": net.weights.cpu().clone()}
 
     def _check_values_state(self, state):
         net = self.network
@@ -221,6 +226,9 @@ class NTupleTDLearner(_BatchTDLearner):
         placements = check_placements(state["placements"], net.n_weights)
         if not np.array_equal(placements, net.placements):
             raise ValueError("checkpoint was written for a network with different placements")
+        thresholds = tuple(int(t) for t in state.get("stage_thresholds", ()))
+        if thresholds != net.stage_thresholds or int(state.get("stage_stride", 0)) != net.stage_stride:
+            raise ValueError("checkpoint was written for a network with different stages")
         return _check_weights(state["weights"], net.n_weights)
 
     def _load_values(self, weights) -> None:
@@ -262,7 +270,8 @@ class NTupleTCLearner(NTupleTDLearner):
     def _launch(self, subs, stats) -> None:
         net = self.network
         E.ntuple_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
-                          self.err_sum, self.abs_err_sum, self.alpha, subs, self.rng_mode, self._scratch, stats)
+                          self.err_sum, self.abs_err_sum, self.alpha, subs, self.rng_mode, self._scratch, stats,
+                          stages=net.stages)
 
     def _values_state(self) -> dict:
         out = super()._values_state()

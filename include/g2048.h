@@ -334,6 +334,45 @@ int g2048_expectimax_values_ntuple(const uint64_t* d_boards, int64_t n, int dept
                                    const float* d_weights, int64_t n_weights, float reward_weight,
                                    float* d_q, uint64_t* d_counters, void* stream);
 
+/* ---- Multi-stage n-tuple networks (Yeh et al. 2016; Jaskowski 2018): the game is split into S = n_thresholds + 1
+ * stages by the largest tile on the board, and each stage has its own copy of every table, `stride` entries after the
+ * previous stage's.
+ *   stage(b) = the number of j < n_thresholds with max_exponent(b) >= thresholds[j]    (the empty board: stage 0)
+ *   V_S(b)   = W[stage(b) * stride + off_0 + idx_0(b)] + ... + W[stage(b) * stride + off_{P-1} + idx_{P-1}(b)],
+ *              float32, left to right from the first term: V's float order, and V itself when S = 1.
+ * The stage is that of the board being valued: a TD target r + V_S(s'') may lie in a higher stage than V_S(after), so
+ * errors cross stage borders, and all stages learn in one launch.  The stages are a HOST struct, checked with the
+ * placements before any launch: G2048_ERR_INVALID for a NULL pointer, n_thresholds > 15, thresholds that are not
+ * strictly increasing in 1..15, a nonzero unused threshold byte, stride != 0 when S = 1 or stride == 0 when S > 1, or
+ * (S - 1) * stride + off_p + 16^k > n_weights for some placement.  n_weights stays at most 2^28, so the 4x6 network
+ * (2^26 weights a stage) has at most 4 stages. */
+typedef struct G2048TupleStages {
+    uint32_t stride;         /* entries from one stage's tables to the next stage's; 0 when n_thresholds == 0 */
+    uint8_t n_thresholds;    /* S - 1, 0..15 */
+    uint8_t thresholds[15];  /* tile exponents, strictly increasing, each in 1..15; unused bytes 0 */
+} G2048TupleStages;          /* 20 bytes */
+#define G2048_NTUPLE_MAX_STAGES 16
+
+/* The three n-tuple entry points above, word for word, with V_S in place of V.  The scratch sizes are those of the
+ * unstaged calls (g2048_ntuple_td_scratch_bytes, g2048_ntuple_tc_scratch_bytes): they depend on n, P and n_weights
+ * only, and one step still touches at most min(n * P, n_weights) entries.  The results are bit-exact and independent
+ * of the grid, as for the unstaged calls: each entry still receives one integer sum (and count) per step.  With
+ * S = 1 each call equals its unstaged form bit for bit. */
+int g2048_ntuple_staged_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                 int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                 const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, float alpha,
+                                 const uint32_t* d_subs, int64_t n_steps, int rng_mode, void* d_scratch,
+                                 uint64_t* d_stats, void* stream);
+int g2048_ntuple_staged_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                 int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                 const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights,
+                                 double* d_err_sum, double* d_abs_err_sum, float alpha, const uint32_t* d_subs,
+                                 int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream);
+int g2048_expectimax_values_ntuple_staged(const uint64_t* d_boards, int64_t n, int depth,
+                                          const G2048TuplePlacement* h_placements, int n_placements,
+                                          const G2048TupleStages* h_stages, const float* d_weights, int64_t n_weights,
+                                          float reward_weight, float* d_q, uint64_t* d_counters, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.

@@ -23,7 +23,18 @@ With --tc, the temporal coherence learner (g2048_ntuple_tc_train, g2048.NTupleTC
   * TC at its best alpha against TD at its default alpha 0.02 at equal steps (--sweep-steps and --long-steps): greedy
     and depth-2 mean scores, the 2048 / 4096 / 8192 / 16384 reach rates, and the training wall time.
 
-    python tools/bench_ntuple.py [--tc] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
+With --stages, multi-stage networks (g2048_ntuple_staged_td_train, NTupleNetwork.staged) instead:
+  * speed: at n = 2^14, 2^16 and 2^18, the 4x6 network trained for --pretrain-steps untimed steps, against 2-stage
+    copies of it split at 11 (a 2048 tile) and at 13 (an 8192 tile) that carry on from the same envs, so that the
+    timed window has a real share of envs in each stage; their timed launches alternated in one process, with the
+    rate ratio and the time-averaged share of envs per stage;
+  * search: expectimax leaves/s at depth 2 and 3 with the staged leaves next to the unstaged one, on the same values
+    (the trained network of the n = 2^16 run and its staged copies) and 4 096 boards of that run's envs;
+  * quality at n = 2^16, --long-steps steps of TD at alpha 0.02 from zeros (seed 0): unstaged; staged with thresholds
+    (13,) and (14,); and half the steps unstaged, then staged((13,)), then the other half.  For each, the training wall
+    time and the greedy and depth-2 players on the seed-7 games: mean score and the 4096 / 8192 / 16384 reach rates.
+
+    python tools/bench_ntuple.py [--tc | --stages] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
 """
 import argparse
 import json
@@ -282,6 +293,150 @@ def equal_steps(tc_alpha: float, lengths, block: int, B: int, deep: int) -> list
     return out
 
 
+def _staged_run(lr, subs):
+    net = lr.network
+    return lambda: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements, net.weights, lr.alpha,
+                                     subs, MODE, lr._scratch, stages=net.stages)
+
+
+def _promoted(lr, thresholds):
+    """A learner of staged(lr.network, thresholds) that carries on from lr's env state and key chain: at the start it
+    has exactly lr's values, so it plays lr's games."""
+    promoted = g2048.NTupleTDLearner(0, lr.batch_size, network=NTupleNetwork.staged(lr.network, thresholds),
+                                     alpha=lr.alpha, rng_mode=lr.rng_mode)
+    ckpt = lr.state_dict()
+    for k in ("placements", "n_weights", "weights", "stage_thresholds", "stage_stride"):
+        ckpt.pop(k)
+    ckpt.update(promoted._values_state())
+    promoted.load_state_dict(ckpt)
+    return promoted
+
+
+def _stage_shares(boards, thresholds) -> list:
+    """The share of the boards in each stage of these thresholds."""
+    me = E.boards_numpy(boards).max(axis=1)
+    stage = sum((me >= t).astype(int) for t in thresholds)
+    return [round(float((stage == s).mean()), 4) for s in range(len(thresholds) + 1)]
+
+
+STAGE_SPLITS = ((11,), (13,))
+
+
+def stages_speed(steps: int, pretrain: int, reps: int = 3) -> tuple:
+    """At each size, the 4x6 network trained by TD (alpha 0.02, seed 0) for `pretrain` untimed steps, so that the envs
+    play the long games of a trained player; then staged copies of it at each split of STAGE_SPLITS, which carry on from
+    the same env state and key chain.  The unstaged and staged learners' timed launches are alternated.  Each staged row
+    carries its rate over the unstaged one and the share of envs in each stage, averaged over samples taken before and
+    after every timed launch.  Also returns the network and 4 096 env boards of the n = 2^16 run, for the search."""
+    out, search_net, search_boards = [], None, None
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        flat = g2048.NTupleTDLearner(0, n, alpha=g2048.td.DEFAULT_NTUPLE_ALPHA, rng_mode=MODE)
+        flat.train(pretrain)
+        learners = {"four_six": flat}
+        for t in STAGE_SPLITS:
+            learners["four_six_2_stages_t%d" % t[0]] = _promoted(flat, t)
+        runs = {k: (_ntuple_run if k == "four_six" else _staged_run)(lr, subs) for k, lr in learners.items()}
+        for run in runs.values():
+            run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in runs}
+        shares = {k: [] for k in runs if k != "four_six"}
+        for _ in range(reps):
+            for k, run in runs.items():
+                if k in shares:
+                    shares[k].append(_stage_shares(learners[k].boards, learners[k].network.stage_thresholds))
+                times[k].append(_timed_once(run))
+                if k in shares:
+                    shares[k].append(_stage_shares(learners[k].boards, learners[k].network.stage_thresholds))
+        rows = [_row(k, n, steps, times[k], pretrain_steps=pretrain) for k in runs]
+        for row in rows[1:]:
+            row["rate_over_unstaged"] = row["learning_steps_per_s"] / rows[0]["learning_steps_per_s"]
+            samples = shares[row["what"]]
+            row["mean_share_of_envs_per_stage"] = [round(sum(x[s] for x in samples) / len(samples), 4)
+                                                   for s in range(len(samples[0]))]
+            print(json.dumps(row), file=sys.stderr, flush=True)
+        out += rows
+        if n == 1 << 16:
+            search_net = NTupleNetwork(flat.network.placements, flat.network.n_weights, flat.network.weights)
+            search_boards = flat.boards[:4096].clone()
+        del flat, learners, runs
+        torch.cuda.empty_cache()
+    return out, search_net, search_boards
+
+
+def stages_search(reps: int, net, boards) -> list:
+    """Leaves/s of the staged leaf next to the unstaged one, on the same values (staged copies of `net`) and on boards
+    of the trained learner's own games, whose stages are reported per split."""
+    flush_buf = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
+    leaves_nets = [("four_six", net, None)]
+    leaves_nets += [("four_six_2_stages_t%d" % t[0], NTupleNetwork.staged(net, t), _stage_shares(boards, t))
+                    for t in STAGE_SPLITS]
+    out = []
+    for depth in (2, 3):
+        for leaf, nw, share in leaves_nets:
+            fn = lambda c=None, nw=nw: E.expectimax_values_ntuple(boards, depth, nw.placements, nw.weights, 0.0, c,  # noqa: E731
+                                                                   stages=nw.stages)
+            counters = torch.zeros(2, dtype=torch.int64, device="cuda")
+            fn(counters)
+            leaves = int(counters[0].item())
+            times = device_times(fn, reps, flush_buf)
+            med = statistics.median(times)
+            out.append({"depth": depth, "leaf": leaf, "boards": int(boards.shape[0]), "leaves": leaves,
+                        "share_of_boards_per_stage": share, "ms": [round(t * 1e3, 3) for t in times],
+                        "leaves_per_s": leaves / med})
+            print(json.dumps(out[-1]), file=sys.stderr, flush=True)
+    del leaves_nets
+    torch.cuda.empty_cache()
+    return out
+
+
+def stages_quality(total: int, block: int, B: int, deep: int) -> list:
+    """TD at alpha 0.02 from zeros at n = 2^16 (seed 0) for `total` steps: unstaged, staged (13,) and (14,), and half
+    unstaged then staged((13,)); each with its training wall time and its greedy and depth-2 players on the seed-7
+    games."""
+    alpha, n = g2048.td.DEFAULT_NTUPLE_ALPHA, 1 << 16
+    out = []
+    for name in ("unstaged", "staged_t13", "staged_t14", "half_unstaged_then_staged_t13"):
+        if name == "unstaged" or name.startswith("half"):
+            net = NTupleNetwork.four_six()
+        else:
+            net = NTupleNetwork.staged(NTupleNetwork.four_six(), (13,) if name.endswith("13") else (14,))
+        lr = g2048.NTupleTDLearner(0, n, network=net, alpha=alpha)
+        if name.startswith("half"):
+            curve, wall = _train(lr, total // 2, block)
+            promoted = _promoted(lr, (13,))
+            del lr
+            torch.cuda.empty_cache()
+            lr = promoted
+            curve2, wall2 = _train(lr, total - total // 2, block)
+            curve, wall = curve + curve2, wall + wall2
+        else:
+            curve, wall = _train(lr, total, block)
+        row = {"run": name, "alpha": alpha, "n": n, "steps": total, "block": block, "train_seconds": round(wall, 2),
+               "curve_mean_score": curve}
+        for depth, games in ((1, B), (2, deep)):
+            row[f"depth{depth}"] = play(g2048.ExpectimaxPolicy(depth=depth, network=lr.network, reward_weight=1.0),
+                                        games)
+        out.append(row)
+        print(json.dumps(row), file=sys.stderr, flush=True)
+        del lr
+        torch.cuda.empty_cache()
+    return out
+
+
+def main_stages(args) -> None:
+    result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident); flushed for search"}
+    if not args.skip_speed:
+        result["speed"], net, boards = stages_speed(args.steps, args.pretrain_steps)
+        result["search"] = stages_search(args.reps, net, boards)
+        del net, boards
+        torch.cuda.empty_cache()
+    if not args.speed_only:
+        result["quality"] = stages_quality(args.long_steps, args.block, args.games, args.deep_games)
+    _emit(result, args.out)
+
+
 def main_tc(args) -> None:
     result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
     if not args.skip_speed:
@@ -307,7 +462,10 @@ def main():
     ap.add_argument("--speed-only", action="store_true", help="speed, phases, lines and n_weights only")
     ap.add_argument("--skip-speed", action="store_true", help="the sweep, search and players only")
     ap.add_argument("--tc", action="store_true", help="the temporal coherence learner against TD (see above)")
-    ap.add_argument("--long-steps", type=int, default=40000, help="the longer equal-steps comparison of --tc")
+    ap.add_argument("--stages", action="store_true", help="multi-stage networks against the unstaged one (see above)")
+    ap.add_argument("--pretrain-steps", type=int, default=20000, help="untimed training before the --stages speed runs")
+    ap.add_argument("--long-steps", type=int, default=40000,
+                    help="the longer equal-steps comparison of --tc, and the runs of --stages")
     ap.add_argument("--phase-probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
@@ -316,6 +474,9 @@ def main():
         return
     if args.tc:
         main_tc(args)
+        return
+    if args.stages:
+        main_stages(args)
         return
     result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident); flushed for search"}
     if not args.skip_speed:
