@@ -32,6 +32,13 @@
 // is moved by it; the accumulate phase uses the previous afterstate's base.  Nothing else changes: the listing, the
 // apply walk and the fixed-point sums work on entries, whatever stage they belong to.  With STAGED = false none of it
 // is compiled in.
+//
+// Delayed TD(lambda) / TC(lambda) (g2048_ntuple_lambda_td_train / _tc_train, the LAMBDA instantiations): each env keeps
+// its last h afterstates and errors in a slot-major ring.  After v[] is used, a lane stores delta_L, reads the errors of
+// the afterstates it releases (one a step in steady state, up to h when its episode ends) and the released board, and
+// forms each e_m with __fmul_rn / __fadd_rn.  The placement loop (match, per-CTA index-0 sums, listing) runs once per
+// release round; the round count is the warp's largest release count, so it stays warp-uniform, and a lane with nothing
+// to release in a round takes part with the "no update" key.  With LAMBDA = false none of it is compiled in.
 #include <cooperative_groups.h>
 
 #include "g2048_ntuple.cuh"
@@ -59,7 +66,8 @@ constexpr float NT_FX_CLAMP = 16777216.0f;        // 2^24: 2^20 envs * 64 placem
 constexpr float NT_FX_ONE = 4096.0f;
 
 // scratch: acc int64[n_weights], (TC: abs int64[n_weights],) cnt uint32[n_weights], list uint32[min(n * P,
-// n_weights)], then list_len uint32[2]
+// n_weights)], then list_len uint32[2]; the lambda forms lay it out for n * h envs, as an env releases up to h
+// afterstates a step
 struct NtScratch {
     int64_t abs_off, cnt_off, list_off, len_off, bytes;
 };
@@ -97,6 +105,11 @@ struct NtTdArgs {
     double* abs_err_sum;          // A
     // STAGED only (after the TC fields, so the unstaged instantiations see the parameter layout they always had)
     NtStages stages;
+    // LAMBDA only (after the stages, for the same reason)
+    float c[G2048_NTUPLE_MAX_HORIZON];  // c_0 .. c_{h-1}, 0 beyond
+    uint32_t horizon;                   // h
+    u64* hist_after;                    // [h * n], slot-major
+    float* hist_delta;                  // [h * n], slot-major
 };
 
 // fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64, to nearest even (the multiply by a power of two is exact)
@@ -115,7 +128,7 @@ __device__ __forceinline__ void nt_append(bool first, uint32_t i, uint32_t* list
     }
 }
 
-template <int MODE, bool TC, bool STAGED>
+template <int MODE, bool TC, bool STAGED, bool LAMBDA>
 __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_constant__ NtTdArgs a) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     __shared__ unsigned long long s_stats[G2048_PLAY_STATS_WORDS];
@@ -199,37 +212,91 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
                 }
             }
             const bool update = aft != 0ull;  // inactive lanes hold after = 0
-            warp_fx[lane] = update ? nt_fx(target - v[4]) : 0ll;
-            __syncwarp();
+            // the placement loop over board x (stage base xbase) of the lanes with upd, whose fx are in warp_fx
+            auto accumulate = [&](bool upd, u64 x, uint32_t xbase) {
 #pragma unroll 1
-            for (uint32_t p = 0; p < P; ++p) {
-                const uint32_t i = aft_base + nt_entry(a.net.pl[p], aft);
-                const unsigned group = __match_any_sync(0xFFFFFFFFu, update ? i : 0xFFFFFFFFu);  // i < 2^28
-                bool first = false;
-                if (update && lane == (unsigned)(__ffs((int)group) - 1)) {
-                    long long sum = 0, abs_sum = 0;
-                    for (unsigned m = group; m; m &= m - 1u) {
-                        const long long fx = warp_fx[__ffs((int)m) - 1];
-                        sum += fx;
-                        if constexpr (TC) abs_sum += fx < 0 ? -fx : fx;
+                for (uint32_t p = 0; p < P; ++p) {
+                    const uint32_t i = xbase + nt_entry(a.net.pl[p], x);
+                    const unsigned group = __match_any_sync(0xFFFFFFFFu, upd ? i : 0xFFFFFFFFu);  // i < 2^28
+                    bool first = false;
+                    if (upd && lane == (unsigned)(__ffs((int)group) - 1)) {
+                        long long sum = 0, abs_sum = 0;
+                        for (unsigned m = group; m; m &= m - 1u) {
+                            const long long fx = warp_fx[__ffs((int)m) - 1];
+                            sum += fx;
+                            if constexpr (TC) abs_sum += fx < 0 ? -fx : fx;
+                        }
+                        const unsigned count = (unsigned)__popc((int)group);
+                        // index 0 of placement p in stage 0.  The per-CTA sums are flushed to off_p, so this relies
+                        // on no other entry of p equalling off_p: an entry of stage s >= 1 is at least stride + off_p
+                        // with stride >= 1, so the later stages' index 0 goes through the global atomics.
+                        if (i == a.net.pl[p].offset) {
+                            atomicAdd(&s_acc0[p], (unsigned long long)sum);
+                            if constexpr (TC) atomicAdd(&s_abs0[p], (unsigned long long)abs_sum);
+                            atomicAdd(&s_cnt0[p], count);
+                        } else {
+                            atomicAdd(&a.acc[i], (unsigned long long)sum);
+                            if constexpr (TC) atomicAdd(&a.abs_acc[i], (unsigned long long)abs_sum);
+                            first = atomicAdd(&a.cnt[i], count) == 0u;
+                        }
                     }
-                    const unsigned count = (unsigned)__popc((int)group);
-                    // index 0 of placement p in stage 0.  The per-CTA sums are flushed to off_p, so this relies on
-                    // no other entry of p equalling off_p: an entry of stage s >= 1 is at least stride + off_p with
-                    // stride >= 1, so the later stages' index 0 goes through the global atomics.
-                    if (i == a.net.pl[p].offset) {
-                        atomicAdd(&s_acc0[p], (unsigned long long)sum);
-                        if constexpr (TC) atomicAdd(&s_abs0[p], (unsigned long long)abs_sum);
-                        atomicAdd(&s_cnt0[p], count);
+                    nt_append(first, i, a.list, list_len, lane);
+                }
+            };
+            if constexpr (LAMBDA) {
+                // L = length; delta_L goes to slot (L - 1) mod h.  Released: x_m for m0 <= m < m0 + n_rel.  An env
+                // with an afterstate but L outside [1, 2^31) is outside the contract and stores and releases nothing.
+                const int h = (int)a.horizon, L = (int)length;
+                const float dL = target - v[4];
+                int m0 = L - h + 1, n_rel = 0;
+                if (update && L >= 1) {
+                    a.hist_delta[(size_t)((L - 1) % h) * a.n + e] = dL;
+                    if (lm == 0u) {
+                        m0 = m0 > 1 ? m0 : 1;
+                        n_rel = L - m0 + 1;
                     } else {
-                        atomicAdd(&a.acc[i], (unsigned long long)sum);
-                        if constexpr (TC) atomicAdd(&a.abs_acc[i], (unsigned long long)abs_sum);
-                        first = atomicAdd(&a.cnt[i], count) == 0u;
+                        n_rel = L >= h ? 1 : 0;
                     }
                 }
-                nt_append(first, i, a.list, list_len, lane);
+                // d[k] = delta_{m0 + k} while m0 + k <= L (the fresh delta_L in place of its slot)
+                float d[G2048_NTUPLE_MAX_HORIZON];
+                const int slot0 = n_rel ? (m0 - 1) % h : 0;
+#pragma unroll
+                for (int k = 0; k < G2048_NTUPLE_MAX_HORIZON; ++k) {
+                    d[k] = 0.0f;
+                    int slot = slot0 + k;
+                    slot = slot >= h ? slot - h : slot;
+                    if (n_rel && m0 + k < L) d[k] = a.hist_delta[(size_t)slot * a.n + e];
+                    if (n_rel && m0 + k == L) d[k] = dL;
+                }
+                const uint32_t rounds = __reduce_max_sync(0xFFFFFFFFu, (unsigned)n_rel);
+                int slot = slot0;
+#pragma unroll 1
+                for (uint32_t r = 0; r < rounds; ++r) {
+                    const int m = m0 + (int)r;
+                    const bool upd = (int)r < n_rel;
+                    u64 x = 0ull;
+                    float em = d[0];
+                    if (upd) {
+                        x = a.hist_after[(size_t)slot * a.n + e];
+#pragma unroll
+                        for (int k = 1; k < G2048_NTUPLE_MAX_HORIZON; ++k)
+                            if (m + k <= L) em = __fadd_rn(em, __fmul_rn(a.c[k], d[k]));
+                    }
+#pragma unroll
+                    for (int k = 0; k + 1 < G2048_NTUPLE_MAX_HORIZON; ++k) d[k] = d[k + 1];  // the next release's window
+                    slot = slot + 1 == h ? 0 : slot + 1;
+                    warp_fx[lane] = upd ? nt_fx(em) : 0ll;
+                    __syncwarp();
+                    accumulate(upd, x, STAGED && upd ? nt_stage_base(a.stages, x) : 0u);
+                    __syncwarp();  // warp_fx is rewritten by the next round
+                }
+            } else {
+                warp_fx[lane] = update ? nt_fx(target - v[4]) : 0ll;
+                __syncwarp();
+                accumulate(update, aft, aft_base);
+                __syncwarp();  // warp_fx is rewritten by the next env
             }
-            __syncwarp();  // warp_fx is rewritten by the next env
 
             if (active) {
                 const Key k = split_at<MODE>(Key{sub.x, sub.y}, a.n, e);
@@ -253,6 +320,7 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
                     split2<MODE>(k, k1, k2);
                     a.boards[e] = spawn_tile(best, bits_scalar<MODE>(k1), bits_scalar<MODE>(k2));
                     a.after[e] = best;
+                    if constexpr (LAMBDA) a.hist_after[(size_t)(length % a.horizon) * a.n + e] = best;  // x_{L+1}
                     a.scores[e] = score + best_r;
                     a.lengths[e] = length + 1u;
                 }
@@ -343,9 +411,9 @@ __global__ void build_ntuple_row_tables_kernel() {
 }
 
 // who: the entry point's name, which prefixes every message
-template <int MODE, bool TC, bool STAGED>
+template <int MODE, bool TC, bool STAGED, bool LAMBDA>
 static int launch_ntuple_td(const char* who, const NtTdArgs& args, cudaStream_t st) {
-    auto kernel = ntuple_td_kernel<MODE, TC, STAGED>;
+    auto kernel = ntuple_td_kernel<MODE, TC, STAGED, LAMBDA>;
     char msg[128];
     auto what = [&](const char* s) {
         snprintf(msg, sizeof(msg), "%s%s%s", who, *s ? ": " : "", s);
@@ -403,19 +471,29 @@ int64_t nt_scratch_bytes(int64_t n, int n_placements, int64_t n_weights, bool tc
     return nt_scratch_layout(n, n_placements, n_weights, tc).bytes;
 }
 
-template <bool TC, bool STAGED>
+template <bool TC, bool STAGED, bool LAMBDA>
 int nt_launch(const char* who, int rng_mode, const NtTdArgs& args, cudaStream_t st) {
-    if (rng_mode == G2048_RNG_PARTITIONABLE) return launch_ntuple_td<G2048_RNG_PARTITIONABLE, TC, STAGED>(who, args, st);
-    return launch_ntuple_td<G2048_RNG_ORIGINAL, TC, STAGED>(who, args, st);
+    if (rng_mode == G2048_RNG_PARTITIONABLE)
+        return launch_ntuple_td<G2048_RNG_PARTITIONABLE, TC, STAGED, LAMBDA>(who, args, st);
+    return launch_ntuple_td<G2048_RNG_ORIGINAL, TC, STAGED, LAMBDA>(who, args, st);
 }
 
-// g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train, and their staged forms (h_stages not
-// NULL; staged = false passes NULL): the checks, then one launch
+// the window of the lambda entry points
+struct NtLambda {
+    float lambda;
+    int horizon;
+    uint64_t* hist_after;
+    float* hist_delta;
+};
+
+// g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train, their staged forms (h_stages not
+// NULL; staged = false passes NULL), and their lambda forms (lam not NULL; staged when h_stages is not NULL): the
+// checks, then one launch
 int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
              uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
              const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, double* d_err_sum,
              double* d_abs_err_sum, float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
-             void* d_scratch, uint64_t* d_stats, void* stream) {
+             void* d_scratch, uint64_t* d_stats, void* stream, const NtLambda* lam = nullptr) {
     if (!(n >= 1 && n <= (1ll << 20))) return nt_fail(who, "n must be in [1, 2^20]");
     if (!(n_steps >= 0)) return nt_fail(who, "n_steps must be >= 0");
     if (!(alpha >= 0.0f && alpha <= 3.402823466e38f)) return nt_fail(who, "alpha must be finite and >= 0");
@@ -439,8 +517,17 @@ int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t
         return nt_fail(who, "d_err_sum and d_abs_err_sum must be 8-byte aligned");
     if (!(((uintptr_t)d_scores & 3u) == 0 && ((uintptr_t)d_lengths & 3u) == 0 && ((uintptr_t)d_weights & 3u) == 0))
         return nt_fail(who, "d_scores, d_lengths and d_weights must be 4-byte aligned");
+    if (lam) {
+        if (!(lam->lambda >= 0.0f && lam->lambda <= 1.0f)) return nt_fail(who, "lambda must be finite and in [0, 1]");
+        if (!(lam->horizon >= 1 && lam->horizon <= G2048_NTUPLE_MAX_HORIZON))
+            return nt_fail(who, "horizon must be in [1, G2048_NTUPLE_MAX_HORIZON]");
+        if (n * lam->horizon > (1ll << 20)) return nt_fail(who, "n * horizon must be <= 2^20");
+        if (!(lam->hist_after && lam->hist_delta)) return nt_fail(who, "pointers");
+        if (!(((uintptr_t)lam->hist_after & 7u) == 0 && ((uintptr_t)lam->hist_delta & 3u) == 0))
+            return nt_fail(who, "d_hist_after must be 8-byte and d_hist_delta 4-byte aligned");
+    }
     if (n_steps == 0) return G2048_OK;
-    const NtScratch lay = nt_scratch_layout(n, n_placements, n_weights, tc);
+    const NtScratch lay = nt_scratch_layout(lam ? n * lam->horizon : n, n_placements, n_weights, tc);
     NtTdArgs args;
     args.boards = (u64*)d_boards;
     args.after = (u64*)d_after;
@@ -461,9 +548,25 @@ int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t
     args.err_sum = tc ? d_err_sum : nullptr;
     args.abs_err_sum = tc ? d_abs_err_sum : nullptr;
     args.stages = staged ? ntuple_stages(*h_stages) : NtStages{0ull, 0u};
+    // c_k by repeated multiplication in double (no pow), so that the host-side restatements get the same bits
+    double d = 1.0;
+    for (int k = 0; k < G2048_NTUPLE_MAX_HORIZON; ++k) {
+        args.c[k] = lam && k < lam->horizon ? (float)d : 0.0f;
+        if (lam) d *= (double)lam->lambda;
+    }
+    args.horizon = lam ? (uint32_t)lam->horizon : 0u;
+    args.hist_after = lam ? (u64*)lam->hist_after : nullptr;
+    args.hist_delta = lam ? lam->hist_delta : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
-    if (staged) return tc ? nt_launch<true, true>(who, rng_mode, args, st) : nt_launch<false, true>(who, rng_mode, args, st);
-    return tc ? nt_launch<true, false>(who, rng_mode, args, st) : nt_launch<false, false>(who, rng_mode, args, st);
+    if (lam) {
+        if (staged) return tc ? nt_launch<true, true, true>(who, rng_mode, args, st)
+                              : nt_launch<false, true, true>(who, rng_mode, args, st);
+        return tc ? nt_launch<true, false, true>(who, rng_mode, args, st)
+                  : nt_launch<false, false, true>(who, rng_mode, args, st);
+    }
+    if (staged) return tc ? nt_launch<true, true, false>(who, rng_mode, args, st)
+                          : nt_launch<false, true, false>(who, rng_mode, args, st);
+    return tc ? nt_launch<true, false, false>(who, rng_mode, args, st) : nt_launch<false, false, false>(who, rng_mode, args, st);
 }
 
 }  // namespace
@@ -514,4 +617,30 @@ extern "C" int g2048_ntuple_staged_tc_train(uint64_t* d_boards, uint64_t* d_afte
     return nt_train("ntuple_staged_tc_train", true, true, d_boards, d_after, d_scores, d_lengths, n, h_placements,
                     n_placements, h_stages, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha, d_subs, n_steps,
                     rng_mode, d_scratch, d_stats, stream);
+}
+
+extern "C" int g2048_ntuple_lambda_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                            uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                            int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                            int64_t n_weights, float alpha, float lambda, int horizon,
+                                            uint64_t* d_hist_after, float* d_hist_delta, const uint32_t* d_subs,
+                                            int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats,
+                                            void* stream) {
+    const NtLambda lam{lambda, horizon, d_hist_after, d_hist_delta};
+    return nt_train("ntuple_lambda_td_train", false, h_stages != nullptr, d_boards, d_after, d_scores, d_lengths, n,
+                    h_placements, n_placements, h_stages, d_weights, n_weights, nullptr, nullptr, alpha, d_subs,
+                    n_steps, rng_mode, d_scratch, d_stats, stream, &lam);
+}
+
+extern "C" int g2048_ntuple_lambda_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                            uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                            int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                            int64_t n_weights, double* d_err_sum, double* d_abs_err_sum, float alpha,
+                                            float lambda, int horizon, uint64_t* d_hist_after, float* d_hist_delta,
+                                            const uint32_t* d_subs, int64_t n_steps, int rng_mode, void* d_scratch,
+                                            uint64_t* d_stats, void* stream) {
+    const NtLambda lam{lambda, horizon, d_hist_after, d_hist_delta};
+    return nt_train("ntuple_lambda_tc_train", true, h_stages != nullptr, d_boards, d_after, d_scores, d_lengths, n,
+                    h_placements, n_placements, h_stages, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha,
+                    d_subs, n_steps, rng_mode, d_scratch, d_stats, stream, &lam);
 }

@@ -81,6 +81,10 @@ _SIGNATURES = {
     "g2048_ntuple_staged_tc_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _P, _P, _FLT, _P, _I64, _INT, _P,
                                             _P, _P]),
     "g2048_expectimax_values_ntuple_staged": (_INT, [_P, _I64, _INT, _P, _INT, _P, _P, _I64, _FLT, _P, _P, _P]),
+    "g2048_ntuple_lambda_td_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _FLT, _FLT, _INT, _P, _P, _P,
+                                            _I64, _INT, _P, _P, _P]),
+    "g2048_ntuple_lambda_tc_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _P, _P, _FLT, _FLT, _INT, _P, _P,
+                                            _P, _I64, _INT, _P, _P, _P]),
     "g2048_play_host": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),
     "g2048_play_host_packed": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P]),
     "g2048_play_packed": (_INT, [_INT, _P, _I64, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),

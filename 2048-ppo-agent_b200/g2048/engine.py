@@ -6,6 +6,7 @@ Boards travel as ``torch.int64`` tensors holding the uint64 bitboard bits; keys 
 """
 from __future__ import annotations
 
+import math
 import os
 import threading
 
@@ -435,6 +436,82 @@ def ntuple_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Ten
     call("g2048_ntuple_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n, _placements_ptr(placements),
          placements.shape[0], ptr(weights), weights.numel(), ptr(err_sum), ptr(abs_err_sum), float(alpha),
          ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
+
+
+def _lambda_checks(who: str, boards: torch.Tensor, placements: np.ndarray, weights: torch.Tensor, lam: float,
+                   hist_after: torch.Tensor, hist_delta: torch.Tensor, scratch: torch.Tensor, tc: bool) -> int:
+    """The checks of the lambda wrappers (ValueError); returns the horizon h = hist_after.shape[0]."""
+    from .ntuple import MAX_HORIZON
+
+    n = boards.shape[0]
+    lam = float(lam)
+    if not (math.isfinite(lam) and 0.0 <= lam <= 1.0):
+        raise ValueError(f"{who}: lambda must be finite and in [0, 1], got {lam}")
+    if hist_after.dim() != 2 or not 1 <= hist_after.shape[0] <= MAX_HORIZON:
+        raise ValueError(f"{who}: hist_after must be (h, n) with h in [1, {MAX_HORIZON}], got {tuple(hist_after.shape)}")
+    h = hist_after.shape[0]
+    if tuple(hist_after.shape) != (h, n) or tuple(hist_delta.shape) != (h, n):
+        raise ValueError(f"{who}: hist_after and hist_delta must be ({h}, {n}), got {tuple(hist_after.shape)} and "
+                         f"{tuple(hist_delta.shape)}")
+    if hist_after.dtype != torch.int64 or hist_delta.dtype != torch.float32:
+        raise ValueError(f"{who}: hist_after must be int64 and hist_delta float32, got {hist_after.dtype} and "
+                         f"{hist_delta.dtype}")
+    for t in (hist_after, hist_delta):
+        if t.device != boards.device or not t.is_contiguous():
+            raise ValueError(f"{who}: the rings must be contiguous and on {boards.device}")
+    if n * h > 1 << 20:
+        raise ValueError(f"{who}: n * h must be <= 2^20, got {n} * {h}")
+    size_of = N.lib.g2048_ntuple_tc_scratch_bytes if tc else N.lib.g2048_ntuple_td_scratch_bytes
+    need = int(size_of(n * h, placements.shape[0], weights.numel()))
+    if need < 0 or scratch.numel() * scratch.element_size() < need:
+        raise ValueError(f"{who}: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch, horizon "
+                         f"and network need {need} (ntuple_{'tc' if tc else 'td'}_scratch(n * h, ...))")
+    return h
+
+
+def ntuple_lambda_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                           placements: np.ndarray, weights: torch.Tensor, alpha: float, lam: float,
+                           hist_after: torch.Tensor, hist_delta: torch.Tensor, subs: torch.Tensor, rng_mode: int,
+                           scratch: torch.Tensor, stats: torch.Tensor | None = None,
+                           stages: np.ndarray | None = None) -> None:
+    """``subs.shape[0]`` synchronous delayed TD(lambda) steps of an n-tuple network (g2048_ntuple_lambda_td_train): as
+    ``ntuple_td_train``, with every afterstate updated h - 1 steps late by the lambda-weighted sum of its h errors.
+    ``hist_after`` (int64) and ``hist_delta`` (float32) are the (h, n) window rings, updated in place (zeros at the
+    start of a run); h = ``hist_after.shape[0]``, 1..8.  ``scratch``: ``ntuple_td_scratch(n * h, ...)``.  ``stages``:
+    None for one stage, or a G2048TupleStages record."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    h = _lambda_checks("ntuple_lambda_td_train", boards, placements, weights, lam, hist_after, hist_delta, scratch,
+                       False)
+    st, st_ptr = _stages_ptr(stages, placements, weights.numel()) if stages is not None else (None, None)
+    call("g2048_ntuple_lambda_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+         _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), float(alpha),
+         float(lam), h, ptr(hist_after), ptr(hist_delta), ptr(_i32(subs)), subs.shape[0], rng_mode, ptr(scratch),
+         ptr(stats), stream_ptr())
+
+
+def ntuple_lambda_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                           placements: np.ndarray, weights: torch.Tensor, err_sum: torch.Tensor,
+                           abs_err_sum: torch.Tensor, alpha: float, lam: float, hist_after: torch.Tensor,
+                           hist_delta: torch.Tensor, subs: torch.Tensor, rng_mode: int, scratch: torch.Tensor,
+                           stats: torch.Tensor | None = None, stages: np.ndarray | None = None) -> None:
+    """``subs.shape[0]`` synchronous delayed TC(lambda) steps (g2048_ntuple_lambda_tc_train): ``ntuple_tc_train``'s
+    E / A update with ``ntuple_lambda_td_train``'s window.  ``scratch``: ``ntuple_tc_scratch(n * h, ...)``."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    for s in (err_sum, abs_err_sum):
+        assert s.dtype == torch.float64 and s.is_contiguous() and s.numel() == weights.numel()
+    h = _lambda_checks("ntuple_lambda_tc_train", boards, placements, weights, lam, hist_after, hist_delta, scratch,
+                       True)
+    st, st_ptr = _stages_ptr(stages, placements, weights.numel()) if stages is not None else (None, None)
+    call("g2048_ntuple_lambda_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+         _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), ptr(err_sum),
+         ptr(abs_err_sum), float(alpha), float(lam), h, ptr(hist_after), ptr(hist_delta), ptr(_i32(subs)),
+         subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
 
 
 def expectimax_values_ntuple(boards: torch.Tensor, depth: int, placements: np.ndarray, weights: torch.Tensor,

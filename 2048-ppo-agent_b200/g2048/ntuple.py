@@ -30,6 +30,8 @@ MAX_WEIGHTS = 1 << 28
 # G2048TupleStages (include/g2048.h), 20 bytes
 STAGES_DTYPE = np.dtype([("stride", "<u4"), ("n_thresholds", "u1"), ("thresholds", "u1", (15,))])
 MAX_STAGES = 16
+# G2048_NTUPLE_MAX_HORIZON (include/g2048.h): the longest window of the TD(lambda) / TC(lambda) learners
+MAX_HORIZON = 8
 
 # the 8 symmetries of the square, as maps of (row, col), in the order of NTupleNetwork.from_tuples
 SYMMETRIES = (

@@ -17,6 +17,15 @@ steps).  A call of ``train`` is one launch of ``g2048_td_train`` (include/g2048.
 step scaled by |E| / A, its running sum of errors over the sum of their absolute values.  A multi-stage network
 (``NTupleNetwork.staged``) is learned by the staged entry points, all its stages in one launch; a single-stage network
 takes the unstaged ones.
+
+Both n-tuple learners take ``lam`` and ``horizon`` (h, 1..8) for delayed TD(lambda) / TC(lambda)
+(``g2048_ntuple_lambda_td_train`` / ``_tc_train``): every env keeps its last h afterstates and their errors, and an
+afterstate is updated h - 1 steps late with the lambda-weighted sum of its h errors (each computed with the weights of
+its own step).  ``horizon=1`` (the default) is TD(0) / TC exactly, through the entry points above.  On the 4x6
+network TC(lambda) learned better players than TC and TD(0), and TD(lambda) worse ones than TD(0) after 40 000 steps
+(profiles/README.md, round 11):
+
+    learner = g2048.NTupleTCLearner(0, batch_size=1 << 16, lam=0.5, horizon=3)
 """
 from __future__ import annotations
 
@@ -28,7 +37,7 @@ import torch
 from . import _native as N
 from . import engine as E
 from .keys import KeyChain
-from .ntuple import NTupleNetwork, check_placements, _check_weights
+from .ntuple import MAX_HORIZON, NTupleNetwork, check_placements, _check_weights
 
 # the step size of the round-7 sweep on one B200 whose greedy player scored best (profiles/README.md, round 7)
 DEFAULT_ALPHA = 0.1
@@ -57,6 +66,31 @@ def _check_table(table) -> torch.Tensor:
     if not bool(torch.isfinite(table).all()):
         raise ValueError("table must be finite")
     return table
+
+
+def _check_lam(lam) -> float:
+    lam = float(lam)
+    if not (math.isfinite(lam) and 0.0 <= lam <= 1.0):
+        raise ValueError(f"lam must be finite and in [0, 1], got {lam}")
+    return lam
+
+
+def _check_horizon(horizon) -> int:
+    try:
+        h = int(horizon)
+    except (TypeError, ValueError, OverflowError):
+        h = None
+    if h is None or isinstance(horizon, bool) or h != horizon or not 1 <= h <= MAX_HORIZON:
+        raise ValueError(f"horizon must be an integer in [1, {MAX_HORIZON}], got {horizon!r}")
+    return h
+
+
+def _check_ring(ring, shape, dtype, name) -> torch.Tensor:
+    """A checkpoint's window ring: a (h, n) tensor of the given dtype, or ValueError."""
+    if not isinstance(ring, torch.Tensor) or ring.dtype != dtype or tuple(ring.shape) != shape:
+        got = (ring.dtype, tuple(ring.shape)) if isinstance(ring, torch.Tensor) else type(ring).__name__
+        raise ValueError(f"{name} must be a {dtype} tensor of shape {shape}, got {got}")
+    return ring
 
 
 def _resolved(device) -> torch.device:
@@ -185,13 +219,22 @@ class NTupleTDLearner(_BatchTDLearner):
     learns the row table: the same greedy move, fixed-point update, key chain and statistics.
 
     ``network``: the ``NTupleNetwork`` whose ``weights`` are learned in place (default: a zero ``four_six()``).
+    ``lam`` / ``horizon``: delayed TD(lambda) over a window of each env's last ``horizon`` afterstates (1..8;
+    ``batch_size * horizon <= 2^20``), held in ``hist_after`` / ``hist_delta`` ((horizon, batch_size) device tensors)
+    when ``horizon > 1``.  ``horizon=1`` is TD(0), whatever ``lam``.
     ``state_dict`` / ``load_state_dict`` resume a run bit for bit; the checkpoint holds the placements and the stages,
     and a load whose placements, n_weights or stages differ from the learner's network is rejected before anything
-    changes (a checkpoint without stages is a single-stage network's)."""
+    changes (a checkpoint without stages is a single-stage network's).  With ``horizon > 1`` it also holds ``lam``,
+    ``horizon`` and both rings; a load with another horizon or with rings of the wrong shape or dtype is rejected, and
+    a checkpoint without them is a ``horizon=1`` learner's."""
 
     def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
-                 alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None):
+                 alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None, lam: float = 0.0, horizon: int = 1):
         self.batch_size, self.alpha = self._check_common(batch_size, alpha)
+        self.lam = _check_lam(lam)
+        self.horizon = _check_horizon(horizon)
+        if self.batch_size * self.horizon > MAX_BATCH:
+            raise ValueError(f"batch_size * horizon must be <= 2^20, got {self.batch_size} * {self.horizon}")
         if network is not None and not isinstance(network, NTupleNetwork):
             raise ValueError("network must be an NTupleNetwork")
         self._start(rng_mode, device)
@@ -199,10 +242,15 @@ class NTupleTDLearner(_BatchTDLearner):
         if _resolved(self.network.weights.device) != _resolved(self.device):
             raise ValueError(f"the network's weights are on {self.network.weights.device}, the learner runs on {self.device}")
         self._init_envs(init_seed)
+        if self.horizon > 1:
+            shape = (self.horizon, self.batch_size)
+            self.hist_after = torch.zeros(shape, dtype=torch.int64, device=self.device)
+            self.hist_delta = torch.zeros(shape, dtype=torch.float32, device=self.device)
         self._scratch = self._new_scratch()
 
     def _new_scratch(self) -> torch.Tensor:
-        return E.ntuple_td_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
+        return E.ntuple_td_scratch(self.batch_size * self.horizon, self.network.placements, self.network.n_weights,
+                                   self.device)
 
     @property
     def weights(self) -> torch.Tensor:
@@ -210,14 +258,38 @@ class NTupleTDLearner(_BatchTDLearner):
 
     def _launch(self, subs, stats) -> None:
         net = self.network
+        if self.horizon > 1:
+            E.ntuple_lambda_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
+                                     self.alpha, self.lam, self.hist_after, self.hist_delta, subs, self.rng_mode,
+                                     self._scratch, stats, stages=net.stages)
+            return
         E.ntuple_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights, self.alpha,
                           subs, self.rng_mode, self._scratch, stats, stages=net.stages)
 
     def _values_state(self) -> dict:
         net = self.network
-        return {"placements": net.placements.copy(), "n_weights": net.n_weights,
-                "stage_thresholds": list(net.stage_thresholds), "stage_stride": net.stage_stride,
-                "weights": net.weights.cpu().clone()}
+        out = {"placements": net.placements.copy(), "n_weights": net.n_weights,
+               "stage_thresholds": list(net.stage_thresholds), "stage_stride": net.stage_stride,
+               "weights": net.weights.cpu().clone()}
+        if self.horizon > 1:
+            out.update({"lam": self.lam, "horizon": self.horizon, "hist_after": self.hist_after.cpu().clone(),
+                        "hist_delta": self.hist_delta.cpu().clone()})
+        return out
+
+    def _check_window_state(self, state):
+        """The checkpoint's window: None for horizon 1, else (lam, hist_after, hist_delta); ValueError if it does not
+        fit this learner."""
+        horizon = _check_horizon(state.get("horizon", 1))
+        if horizon != self.horizon:
+            raise ValueError(f"checkpoint was written with horizon {horizon}, this learner's is {self.horizon}")
+        if self.horizon == 1:
+            return None
+        if "lam" not in state:
+            raise ValueError("checkpoint has no lam")
+        lam = _check_lam(state["lam"])
+        shape = (self.horizon, self.batch_size)
+        return (lam, _check_ring(state.get("hist_after"), shape, torch.int64, "hist_after"),
+                _check_ring(state.get("hist_delta"), shape, torch.float32, "hist_delta"))
 
     def _check_values_state(self, state):
         net = self.network
@@ -229,10 +301,16 @@ class NTupleTDLearner(_BatchTDLearner):
         thresholds = tuple(int(t) for t in state.get("stage_thresholds", ()))
         if thresholds != net.stage_thresholds or int(state.get("stage_stride", 0)) != net.stage_stride:
             raise ValueError("checkpoint was written for a network with different stages")
-        return _check_weights(state["weights"], net.n_weights)
+        window = self._check_window_state(state)
+        return _check_weights(state["weights"], net.n_weights), window
 
-    def _load_values(self, weights) -> None:
+    def _load_values(self, values) -> None:
+        weights, window = values
         self.network.weights.copy_(weights.to(self.device))
+        if window is not None:
+            self.lam = window[0]
+            self.hist_after.copy_(window[1].to(self.device))
+            self.hist_delta.copy_(window[2].to(self.device))
 
 
 def _check_sums(sums, n_weights: int, name: str) -> torch.Tensor:
@@ -255,20 +333,29 @@ class NTupleTCLearner(NTupleTDLearner):
     sign keep a large step, weights whose errors cancel stop moving (g2048_ntuple_tc_train, include/g2048.h).
 
     ``network`` may hold weights learned before (for example by ``NTupleTDLearner``): TC starts from them with
-    E = A = 0.  ``state_dict`` / ``load_state_dict`` resume a run bit for bit, E and A included."""
+    E = A = 0.  ``lam`` / ``horizon``: delayed TC(lambda), the window of ``NTupleTDLearner``.  ``state_dict`` /
+    ``load_state_dict`` resume a run bit for bit, E and A included."""
 
     def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
-                 alpha: float = DEFAULT_NTUPLE_TC_ALPHA, rng_mode=None, device=None):
-        super().__init__(init_seed, batch_size, network=network, alpha=alpha, rng_mode=rng_mode, device=device)
+                 alpha: float = DEFAULT_NTUPLE_TC_ALPHA, rng_mode=None, device=None, lam: float = 0.0,
+                 horizon: int = 1):
+        super().__init__(init_seed, batch_size, network=network, alpha=alpha, rng_mode=rng_mode, device=device,
+                         lam=lam, horizon=horizon)
         n_weights = self.network.n_weights
         self.err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
         self.abs_err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
 
     def _new_scratch(self) -> torch.Tensor:
-        return E.ntuple_tc_scratch(self.batch_size, self.network.placements, self.network.n_weights, self.device)
+        return E.ntuple_tc_scratch(self.batch_size * self.horizon, self.network.placements, self.network.n_weights,
+                                   self.device)
 
     def _launch(self, subs, stats) -> None:
         net = self.network
+        if self.horizon > 1:
+            E.ntuple_lambda_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
+                                     self.err_sum, self.abs_err_sum, self.alpha, self.lam, self.hist_after,
+                                     self.hist_delta, subs, self.rng_mode, self._scratch, stats, stages=net.stages)
+            return
         E.ntuple_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
                           self.err_sum, self.abs_err_sum, self.alpha, subs, self.rng_mode, self._scratch, stats,
                           stages=net.stages)
@@ -279,16 +366,16 @@ class NTupleTCLearner(NTupleTDLearner):
         return out
 
     def _check_values_state(self, state):
-        weights = super()._check_values_state(state)
+        base = super()._check_values_state(state)  # (weights, window)
         n_weights = self.network.n_weights
         err_sum = _check_sums(state.get("err_sum"), n_weights, "err_sum")
         abs_err_sum = _check_sums(state.get("abs_err_sum"), n_weights, "abs_err_sum")
         if bool((abs_err_sum < 0).any()):
             raise ValueError("abs_err_sum must be >= 0")
-        return weights, err_sum, abs_err_sum
+        return base, err_sum, abs_err_sum
 
     def _load_values(self, values) -> None:
-        weights, err_sum, abs_err_sum = values
-        super()._load_values(weights)
+        base, err_sum, abs_err_sum = values
+        super()._load_values(base)
         self.err_sum.copy_(err_sum.to(self.device))
         self.abs_err_sum.copy_(abs_err_sum.to(self.device))

@@ -373,6 +373,50 @@ int g2048_expectimax_values_ntuple_staged(const uint64_t* d_boards, int64_t n, i
                                           const G2048TupleStages* h_stages, const float* d_weights, int64_t n_weights,
                                           float reward_weight, float* d_q, uint64_t* d_counters, void* stream);
 
+/* ---- Delayed TD(lambda) and TC(lambda) learning of an n-tuple network (Jaskowski 2018, delayed temporal coherence):
+ * each env keeps a window of its last h = horizon afterstates and their errors, and an afterstate is updated h - 1
+ * steps late with the lambda-weighted sum of its h errors (a truncated lambda-return).  g2048_ntuple_td_train's contract
+ * (g2048_ntuple_tc_train's for the TC form; V_S of h_stages, or V when h_stages is NULL) word for word except step 2.
+ *   c_k (k < h): computed on the host in double by repeated multiplication, d_0 = 1, d_k = d_{k-1} * (double)lambda,
+ *           c_k = (float)d_k (no pow).
+ *   d_hist_after: uint64[h * n], the afterstates; d_hist_delta: float[h * n], their errors.  Slot-major: entry (j, e)
+ *           is at j * n + e.  Caller-owned, updated in place; zeros are a valid start.
+ * Let L = lengths[e] at the start of the step.  x_m (m = 1..L) is the afterstate of the episode's m-th move and lives in
+ * slot (m - 1) mod h with its error delta_m.  The window is defined by L alone: slots of an earlier episode are never
+ * read.  Step 2 becomes: if after != 0 (after = x_L) and 1 <= L < 2^31 (an env with an afterstate and L outside that
+ * range is outside the contract; it stores and releases nothing):
+ *   a. delta_L = target - V_t(x_L) as in step 2 of g2048_ntuple_td_train; it is stored in hist_delta slot (L - 1) mod h.
+ *   b. Released afterstates: if the env moves, x_{L-h+1} when L >= h; if the episode ends, every x_m with
+ *      max(1, L - h + 1) <= m <= L (their missing later errors count as 0).
+ *   c. A released x_m carries e_m = delta_m, then e_m = e_m + c_k * delta_{m+k} for k = 1, 2, ... while m + k <= L
+ *      (so k <= h - 1), float32, the product rounded before the add (no contraction).
+ *   d. For each released x_m and each placement p in order: fx(e_m) into acc, 1 into cnt (TC: |fx(e_m)| into abs) at
+ *      stage(x_m) * stride + off_p + idx_p(x_m).
+ * Step 3 also stores the new afterstate x_{L+1} in hist_after slot L mod h (the slot just released) when the env moves.
+ * Step 4 (TC: beta, E and A) is unchanged.  The errors of a window were computed with the weights of their own steps,
+ * not with the weights at the release ("delayed" lambda-returns).  With h = 1 (any lambda) each call equals
+ * g2048_ntuple_td_train / g2048_ntuple_tc_train (staged: their staged forms) bit for bit.  An env releases at most h
+ * afterstates a step, so |acc[i]| <= n * h * 64 * 2^36; n * h <= 2^20 keeps the 2^62 bound.  The results are bit-exact
+ * and independent of the grid: each entry still receives one integer (sum, |sum|, count) per step.
+ *   d_scratch: g2048_ntuple_td_scratch_bytes(n * h, n_placements, n_weights) bytes (TC: g2048_ntuple_tc_scratch_bytes),
+ *           zeroed by the caller once; every call leaves it zeroed (a step touches at most n * h * P entries).
+ * G2048_ERR_INVALID before any launch for everything the corresponding call rejects, lambda not finite or outside
+ * [0, 1], horizon outside 1..G2048_NTUPLE_MAX_HORIZON, n * horizon > 2^20, and NULL or misaligned hist pointers (8 bytes
+ * for d_hist_after, 4 for d_hist_delta). */
+#define G2048_NTUPLE_MAX_HORIZON 8
+int g2048_ntuple_lambda_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                 int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                 const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, float alpha,
+                                 float lambda, int horizon, uint64_t* d_hist_after, float* d_hist_delta,
+                                 const uint32_t* d_subs, int64_t n_steps, int rng_mode, void* d_scratch,
+                                 uint64_t* d_stats, void* stream);
+int g2048_ntuple_lambda_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                 int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                 const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights,
+                                 double* d_err_sum, double* d_abs_err_sum, float alpha, float lambda, int horizon,
+                                 uint64_t* d_hist_after, float* d_hist_delta, const uint32_t* d_subs, int64_t n_steps,
+                                 int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.

@@ -34,7 +34,20 @@ With --stages, multi-stage networks (g2048_ntuple_staged_td_train, NTupleNetwork
     (13,) and (14,); and half the steps unstaged, then staged((13,)), then the other half.  For each, the training wall
     time and the greedy and depth-2 players on the seed-7 games: mean score and the 4096 / 8192 / 16384 reach rates.
 
-    python tools/bench_ntuple.py [--tc | --stages] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
+With --lambda, delayed TD(lambda) / TC(lambda) (g2048_ntuple_lambda_td_train / _tc_train, the learners' lam and
+horizon) instead:
+  * speed: at n = 2^14, 2^16 and 2^18, the 4x6 network trained by TD for --pretrain-steps untimed steps; then TD(0), TC
+    and TD(lambda) / TC(lambda) at h = 2, 3, 5 (h capped so that n * h <= 2^20), each on its own copy of the weights
+    and env state, their timed launches alternated in one process, with each rate over TD(0)'s (TC(lambda) also over
+    TC's);
+  * the accumulate / apply split of TD(0), TC, TD(lambda) and TC(lambda) at h = 3 from the -DG2048_NTUPLE_PHASES build,
+    from the same pretrained start;
+  * quality from the zero 4x6 network at n = 2^16 (seed 0): TD(0), TC and TD / TC(lambda) over lambda in {0.25, 0.5,
+    0.75} x h in {2, 3, 5}, evaluated after --sweep-steps and after --long-steps steps (one run each: the second
+    evaluation continues the first): learning curve, training wall time, greedy and depth-2 players on the seed-7 games;
+    then one staged (13,) run of the best setting at --long-steps, next to staged TD(0).
+
+    python tools/bench_ntuple.py [--tc | --stages | --lambda] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
 """
 import argparse
 import json
@@ -437,6 +450,168 @@ def main_stages(args) -> None:
     _emit(result, args.out)
 
 
+LAMBDA_HS = (2, 3, 5)
+LAMBDA_GRID = tuple((lam, h) for lam in (0.25, 0.5, 0.75) for h in LAMBDA_HS)
+
+
+def _lambda_learner(kind, n, lam, h, network=None):
+    cls = g2048.NTupleTCLearner if kind == "tc" else g2048.NTupleTDLearner
+    alpha = g2048.td.DEFAULT_NTUPLE_TC_ALPHA if kind == "tc" else g2048.td.DEFAULT_NTUPLE_ALPHA
+    return cls(0, n, network=network, alpha=alpha, rng_mode=MODE, lam=lam, horizon=h)
+
+
+def _lambda_run(lr, subs, stats=None):
+    net = lr.network
+    tc = isinstance(lr, g2048.NTupleTCLearner)
+    if lr.horizon == 1:
+        if tc:
+            return lambda st=stats: E.ntuple_tc_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,
+                                                      net.weights, lr.err_sum, lr.abs_err_sum, lr.alpha, subs, MODE,
+                                                      lr._scratch, st)
+        return lambda st=stats: E.ntuple_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,
+                                                  net.weights, lr.alpha, subs, MODE, lr._scratch, st)
+    if tc:
+        return lambda st=stats: E.ntuple_lambda_tc_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,
+                                                         net.weights, lr.err_sum, lr.abs_err_sum, lr.alpha, lr.lam,
+                                                         lr.hist_after, lr.hist_delta, subs, MODE, lr._scratch, st)
+    return lambda st=stats: E.ntuple_lambda_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements,
+                                                     net.weights, lr.alpha, lr.lam, lr.hist_after, lr.hist_delta,
+                                                     subs, MODE, lr._scratch, st)
+
+
+def _lambda_learners(n, pretrain, hs):
+    """The 4x6 network trained by TD (alpha 0.02, seed 0) for `pretrain` steps at n envs, and learners that carry on
+    from its weights and env state: name -> learner, for TD(0), TC and TD / TC(lambda = 0.5) at each h of hs."""
+    flat = g2048.NTupleTDLearner(0, n, alpha=g2048.td.DEFAULT_NTUPLE_ALPHA, rng_mode=MODE)
+    flat.train(pretrain)
+    specs = [("td", "td", 0.0, 1), ("tc", "tc", 0.0, 1)]
+    specs += [(f"{kind}_lambda_h{h}", kind, 0.5, h) for h in hs for kind in ("td", "tc")]
+    out = {}
+    for name, kind, lam, h in specs:
+        net = NTupleNetwork(flat.network.placements, flat.network.n_weights, flat.network.weights.clone())
+        lr = _lambda_learner(kind, n, lam, h, net)
+        for k in ("boards", "after", "scores", "lengths"):
+            getattr(lr, k).copy_(getattr(flat, k))
+        out[name] = lr
+    del flat
+    torch.cuda.empty_cache()
+    return out
+
+
+def lambda_speed(steps: int, pretrain: int, reps: int = 3) -> list:
+    """At each size: the learners of _lambda_learners (h capped so that n * h <= 2^20), all warmed up, then their timed
+    launches alternated on the same sub keys."""
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        learners = _lambda_learners(n, pretrain, [h for h in LAMBDA_HS if n * h <= 1 << 20])
+        runs = {k: _lambda_run(lr, subs) for k, lr in learners.items()}
+        for run in runs.values():
+            run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in runs}
+        for _ in range(reps):
+            for k, run in runs.items():
+                times[k].append(_timed_once(run))
+        rows = [_row(k, n, steps, times[k], pretrain_steps=pretrain, horizon=learners[k].horizon) for k in runs]
+        rate = {r["what"]: r["learning_steps_per_s"] for r in rows}
+        for row in rows:
+            row["rate_over_td0"] = row["learning_steps_per_s"] / rate["td"]
+            if row["what"].startswith("tc"):
+                row["rate_over_tc"] = row["learning_steps_per_s"] / rate["tc"]
+            print(json.dumps(row), file=sys.stderr, flush=True)
+        out += rows
+        del learners, runs
+        torch.cuda.empty_cache()
+    return out
+
+
+def lambda_phase_probe(steps: int, pretrain: int) -> list:
+    """In a build with -DG2048_NTUPLE_PHASES: the accumulate / apply split of TD(0), TC and TD / TC(lambda) at h = 3,
+    one launch of `steps` steps after a warm-up launch, from the pretrained start of lambda_speed."""
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        learners = _lambda_learners(n, pretrain, (3,))
+        for name, lr in learners.items():
+            stats = torch.zeros(32, dtype=torch.int64, device="cuda")
+            run = _lambda_run(lr, subs)
+            run()
+            torch.cuda.synchronize()
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            run(stats)
+            b.record()
+            torch.cuda.synchronize()
+            acc_ns, apply_ns, listed = (int(x) for x in stats[8:11].tolist())
+            out.append({"n": n, "learner": name, "steps": steps, "us_per_step": a.elapsed_time(b) * 1e3 / steps,
+                        "accumulate_us_per_step": acc_ns / 1e3 / steps, "apply_us_per_step": apply_ns / 1e3 / steps,
+                        "entries_listed_per_step": listed / steps})
+            print(json.dumps(out[-1]), file=sys.stderr, flush=True)
+        del learners
+        torch.cuda.empty_cache()
+    return out
+
+
+def lambda_phases(steps: int, pretrain: int) -> dict:
+    tmp = Path(tempfile.mkdtemp(prefix="g2048_ntuple_phases_"))
+    lib = tmp / "libg2048_phases.so"
+    subprocess.run(["make", "-C", str(ROOT / "2048-ppo-agent_b200" / "csrc"), "-j16", f"OUT={lib}", f"BUILD={tmp / 'build'}",
+                    "EXTRA=-DG2048_NTUPLE_PHASES"], check=True, capture_output=True)
+    env = dict(os.environ, G2048_LIB=str(lib))
+    res = subprocess.run([sys.executable, __file__, "--phase-probe", "--lambda", "--steps", str(steps),
+                          "--pretrain-steps", str(pretrain)], env=env, capture_output=True, text=True, check=True)
+    return {"build": "-DG2048_NTUPLE_PHASES", "rows": json.loads(res.stdout.strip().splitlines()[-1])}
+
+
+def _players(net, B, deep) -> dict:
+    return {f"depth{depth}": play(g2048.ExpectimaxPolicy(depth=depth, network=net, reward_weight=1.0), games)
+            for depth, games in ((1, B), (2, deep))}
+
+
+def lambda_quality(short: int, long: int, block: int, B: int, deep: int) -> list:
+    """From the zero 4x6 network at n = 2^16: every setting evaluated after `short` steps and, continuing the same
+    run, after `long` steps; then the best lambda setting at `long` (greedy mean) as a staged (13,) run next to staged
+    TD(0)."""
+    n = 1 << 16
+    out = []
+    settings = [("td", 0.0, 1), ("tc", 0.0, 1)] + [(k, lam, h) for k in ("td", "tc") for lam, h in LAMBDA_GRID]
+    for kind, lam, h in settings:
+        lr = _lambda_learner(kind, n, lam, h)
+        curve, wall = _train(lr, short, block)
+        row = {"learner": kind, "lam": lam, "horizon": h, "alpha": lr.alpha, "n": n, "block": block}
+        row[f"steps{short}"] = {"train_seconds": round(wall, 2), **_players(lr.network, B, deep)}
+        curve2, wall2 = _train(lr, long - short, block)
+        row[f"steps{long}"] = {"train_seconds": round(wall + wall2, 2), **_players(lr.network, B, deep)}
+        row["curve_mean_score"] = curve + curve2
+        out.append(row)
+        print(json.dumps(row), file=sys.stderr, flush=True)
+        del lr
+        torch.cuda.empty_cache()
+    best = max((r for r in out if r["horizon"] > 1), key=lambda r: r[f"steps{long}"]["depth1"]["mean_score"])
+    for kind, lam, h in (("td", 0.0, 1), (best["learner"], best["lam"], best["horizon"])):
+        lr = _lambda_learner(kind, n, lam, h, NTupleNetwork.staged(NTupleNetwork.four_six(), (13,)))
+        curve, wall = _train(lr, long, block)
+        row = {"learner": kind, "lam": lam, "horizon": h, "alpha": lr.alpha, "n": n, "block": block,
+               "stage_thresholds": [13], f"steps{long}": {"train_seconds": round(wall, 2), **_players(lr.network, B, deep)},
+               "curve_mean_score": curve}
+        out.append(row)
+        print(json.dumps(row), file=sys.stderr, flush=True)
+        del lr
+        torch.cuda.empty_cache()
+    return out
+
+
+def main_lambda(args) -> None:
+    result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
+    if not args.skip_speed:
+        result["speed"] = lambda_speed(args.steps, args.pretrain_steps)
+        result["phases"] = lambda_phases(args.steps, args.pretrain_steps)
+    if not args.speed_only:
+        result["quality"] = lambda_quality(args.sweep_steps, args.long_steps, args.block, args.games, args.deep_games)
+    _emit(result, args.out)
+
+
 def main_tc(args) -> None:
     result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
     if not args.skip_speed:
@@ -463,14 +638,21 @@ def main():
     ap.add_argument("--skip-speed", action="store_true", help="the sweep, search and players only")
     ap.add_argument("--tc", action="store_true", help="the temporal coherence learner against TD (see above)")
     ap.add_argument("--stages", action="store_true", help="multi-stage networks against the unstaged one (see above)")
-    ap.add_argument("--pretrain-steps", type=int, default=20000, help="untimed training before the --stages speed runs")
+    ap.add_argument("--lambda", dest="lam", action="store_true",
+                    help="delayed TD(lambda) / TC(lambda) against TD(0) and TC (see above)")
+    ap.add_argument("--pretrain-steps", type=int, default=20000,
+                    help="untimed training before the --stages and --lambda speed runs")
     ap.add_argument("--long-steps", type=int, default=40000,
                     help="the longer equal-steps comparison of --tc, and the runs of --stages")
     ap.add_argument("--phase-probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if args.phase_probe:
-        print(json.dumps(phase_probe(args.steps, args.tc)))
+        probe = lambda_phase_probe(args.steps, args.pretrain_steps) if args.lam else phase_probe(args.steps, args.tc)
+        print(json.dumps(probe))
+        return
+    if args.lam:
+        main_lambda(args)
         return
     if args.tc:
         main_tc(args)
