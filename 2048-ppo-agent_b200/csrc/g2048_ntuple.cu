@@ -39,6 +39,13 @@
 // forms each e_m with __fmul_rn / __fadd_rn.  The placement loop (match, per-CTA index-0 sums, listing) runs once per
 // release round; the round count is the warp's largest release count, so it stays warp-uniform, and a lane with nothing
 // to release in a round takes part with the "no update" key.  With LAMBDA = false none of it is compiled in.
+//
+// Carousel shaping (g2048_ntuple_carousel_td_train / _tc_train, the CAROUSEL instantiations, always STAGED): an env
+// whose move raises the stage stores its new board in its pending word in the scratch; the apply phase, after the
+// first grid.sync(), commits each pending word of the envs the thread owns to the pool and clears it, so no draw of
+// the step sees it.  An env whose episode ends reads its start stage and draws one pool slot; it restarts from that
+// board, or from init(k) when the slot is empty or the carousel is back at the opening.  With CAROUSEL = false none of
+// it is compiled in.
 #include <cooperative_groups.h>
 
 #include "g2048_ntuple.cuh"
@@ -67,7 +74,7 @@ constexpr float NT_FX_ONE = 4096.0f;
 
 // scratch: acc int64[n_weights], (TC: abs int64[n_weights],) cnt uint32[n_weights], list uint32[min(n * P,
 // n_weights)], then list_len uint32[2]; the lambda forms lay it out for n * h envs, as an env releases up to h
-// afterstates a step
+// afterstates a step.  The carousel forms append the pending words, uint64[n], at `bytes`.
 struct NtScratch {
     int64_t abs_off, cnt_off, list_off, len_off, bytes;
 };
@@ -110,6 +117,10 @@ struct NtTdArgs {
     uint32_t horizon;                   // h
     u64* hist_after;                    // [h * n], slot-major
     float* hist_delta;                  // [h * n], slot-major
+    // CAROUSEL only (after the lambda fields, for the same reason)
+    uint32_t* start_stage;  // [n]
+    u64* pool;              // [(S - 1) * n], stage-major
+    u64* pending;           // [n], in the scratch: the board with which the env entered a stage this step, or 0
 };
 
 // fx(d) = rint(clamp(d, -2^24, 2^24) * 4096) as int64, to nearest even (the multiply by a power of two is exact)
@@ -128,8 +139,9 @@ __device__ __forceinline__ void nt_append(bool first, uint32_t i, uint32_t* list
     }
 }
 
-template <int MODE, bool TC, bool STAGED, bool LAMBDA>
+template <int MODE, bool TC, bool STAGED, bool LAMBDA, bool CAROUSEL>
 __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_constant__ NtTdArgs a) {
+    static_assert(!CAROUSEL || STAGED, "carousel shaping needs stages");
     extern __shared__ __align__(16) uint8_t smem_raw[];
     __shared__ unsigned long long s_stats[G2048_PLAY_STATS_WORDS];
     __shared__ long long s_fx[NT_THREADS];
@@ -301,24 +313,50 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
             if (active) {
                 const Key k = split_at<MODE>(Key{sub.x, sub.y}, a.n, e);
                 if (lm == 0u) {  // the episode ends here: count it and start the next one
-                    const uint32_t me = max_exponent(s);
-                    const unsigned long long tile = 1ull << me;
-                    atomicAdd(&s_stats[0], 1ull);
-                    atomicAdd(&s_stats[1], (unsigned long long)length);
-                    atomicAdd(&s_stats[2], (unsigned long long)score);
-                    if (has_max_nibble(s)) atomicAdd(&s_stats[4], 1ull);
-                    atomicMax(&s_stats[5], (unsigned long long)length);
-                    atomicAdd(&s_stats[6], tile);
-                    atomicAdd(&s_stats[7], tile * tile);
-                    atomicAdd(&s_stats[16 + me], 1ull);
-                    a.boards[e] = env_init<MODE>(k).board;
+                    bool opening = true;  // the episode began at the opening (always, without the carousel)
+                    u64 next = 0ull;      // the restart board; 0: init(k)
+                    uint32_t next_stage = 0u;
+                    if constexpr (CAROUSEL) {
+                        // l = c + 1, or 0 when c + 1 >= S (the wrap); S - 1 is the stage of exponent 15
+                        const uint32_t c0 = a.start_stage[e];
+                        const uint32_t l = c0 + 1u <= (uint32_t)(a.stages.stage_of >> 60) ? c0 + 1u : 0u;
+                        opening = c0 == 0u;
+                        if (l) {
+                            Key k1, k2;
+                            split2<MODE>(k, k1, k2);
+                            const uint32_t j = (uint32_t)(((u64)bits_scalar<MODE>(k1) * a.n) >> 32);
+                            next = a.pool[(size_t)(l - 1u) * a.n + j];
+                            next_stage = next ? l : 0u;
+                        }
+                        a.start_stage[e] = next_stage;
+                    }
+                    if (opening) {
+                        const uint32_t me = max_exponent(s);
+                        const unsigned long long tile = 1ull << me;
+                        atomicAdd(&s_stats[0], 1ull);
+                        atomicAdd(&s_stats[1], (unsigned long long)length);
+                        atomicAdd(&s_stats[2], (unsigned long long)score);
+                        if (has_max_nibble(s)) atomicAdd(&s_stats[4], 1ull);
+                        atomicMax(&s_stats[5], (unsigned long long)length);
+                        atomicAdd(&s_stats[6], tile);
+                        atomicAdd(&s_stats[7], tile * tile);
+                        atomicAdd(&s_stats[16 + me], 1ull);
+                    } else {  // an episode that began from a pool board
+                        atomicAdd(&s_stats[12], 1ull);
+                        atomicAdd(&s_stats[13], (unsigned long long)length);
+                    }
+                    a.boards[e] = next ? next : env_init<MODE>(k).board;
                     a.after[e] = 0ull;
                     a.scores[e] = 0u;
                     a.lengths[e] = 0u;
                 } else {
                     Key k1, k2;
                     split2<MODE>(k, k1, k2);
-                    a.boards[e] = spawn_tile(best, bits_scalar<MODE>(k1), bits_scalar<MODE>(k2));
+                    const u64 spawned = spawn_tile(best, bits_scalar<MODE>(k1), bits_scalar<MODE>(k2));
+                    a.boards[e] = spawned;
+                    // the stage rises by at most 1 a move; the apply phase commits the board to the pool
+                    if constexpr (CAROUSEL)
+                        if (nt_stage(a.stages, spawned) > nt_stage(a.stages, s)) a.pending[e] = spawned;
                     a.after[e] = best;
                     if constexpr (LAMBDA) a.hist_after[(size_t)(length % a.horizon) * a.n + e] = best;  // x_{L+1}
                     a.scores[e] = score + best_r;
@@ -372,6 +410,15 @@ __global__ void __launch_bounds__(NT_THREADS, 1) ntuple_td_kernel(const __grid_c
             a.cnt[i] = 0u;
             a.list[j] = 0u;
         }
+        if constexpr (CAROUSEL) {  // the envs this thread stepped: their stage entries go to the pool
+            for (uint32_t e = blockIdx.x * NT_THREADS + threadIdx.x; e < a.n; e += stride) {
+                const u64 b = a.pending[e];
+                if (b) {
+                    a.pool[(size_t)(nt_stage(a.stages, b) - 1u) * a.n + e] = b;
+                    a.pending[e] = 0ull;
+                }
+            }
+        }
         if (blockIdx.x == 0 && threadIdx.x == 0) a.list_len[(t + 1) & 1] = 0u;
         grid.sync();
 #ifdef G2048_NTUPLE_PHASES
@@ -411,9 +458,9 @@ __global__ void build_ntuple_row_tables_kernel() {
 }
 
 // who: the entry point's name, which prefixes every message
-template <int MODE, bool TC, bool STAGED, bool LAMBDA>
+template <int MODE, bool TC, bool STAGED, bool LAMBDA, bool CAROUSEL>
 static int launch_ntuple_td(const char* who, const NtTdArgs& args, cudaStream_t st) {
-    auto kernel = ntuple_td_kernel<MODE, TC, STAGED, LAMBDA>;
+    auto kernel = ntuple_td_kernel<MODE, TC, STAGED, LAMBDA, CAROUSEL>;
     char msg[128];
     auto what = [&](const char* s) {
         snprintf(msg, sizeof(msg), "%s%s%s", who, *s ? ": " : "", s);
@@ -471,11 +518,11 @@ int64_t nt_scratch_bytes(int64_t n, int n_placements, int64_t n_weights, bool tc
     return nt_scratch_layout(n, n_placements, n_weights, tc).bytes;
 }
 
-template <bool TC, bool STAGED, bool LAMBDA>
+template <bool TC, bool STAGED, bool LAMBDA, bool CAROUSEL = false>
 int nt_launch(const char* who, int rng_mode, const NtTdArgs& args, cudaStream_t st) {
     if (rng_mode == G2048_RNG_PARTITIONABLE)
-        return launch_ntuple_td<G2048_RNG_PARTITIONABLE, TC, STAGED, LAMBDA>(who, args, st);
-    return launch_ntuple_td<G2048_RNG_ORIGINAL, TC, STAGED, LAMBDA>(who, args, st);
+        return launch_ntuple_td<G2048_RNG_PARTITIONABLE, TC, STAGED, LAMBDA, CAROUSEL>(who, args, st);
+    return launch_ntuple_td<G2048_RNG_ORIGINAL, TC, STAGED, LAMBDA, CAROUSEL>(who, args, st);
 }
 
 // the window of the lambda entry points
@@ -486,14 +533,21 @@ struct NtLambda {
     float* hist_delta;
 };
 
+// the arrays of the carousel entry points
+struct NtCarousel {
+    uint32_t* start_stage;
+    uint64_t* stage_pool;
+};
+
 // g2048_ntuple_td_train (tc = false; E and A unused) and g2048_ntuple_tc_train, their staged forms (h_stages not
-// NULL; staged = false passes NULL), and their lambda forms (lam not NULL; staged when h_stages is not NULL): the
-// checks, then one launch
+// NULL; staged = false passes NULL), their lambda forms (lam not NULL; staged when h_stages is not NULL) and their
+// carousel forms (lam and car not NULL, staged): the checks, then one launch
 int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
              uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
              const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, double* d_err_sum,
              double* d_abs_err_sum, float alpha, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
-             void* d_scratch, uint64_t* d_stats, void* stream, const NtLambda* lam = nullptr) {
+             void* d_scratch, uint64_t* d_stats, void* stream, const NtLambda* lam = nullptr,
+             const NtCarousel* car = nullptr) {
     if (!(n >= 1 && n <= (1ll << 20))) return nt_fail(who, "n must be in [1, 2^20]");
     if (!(n_steps >= 0)) return nt_fail(who, "n_steps must be >= 0");
     if (!(alpha >= 0.0f && alpha <= 3.402823466e38f)) return nt_fail(who, "alpha must be finite and >= 0");
@@ -507,6 +561,7 @@ int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t
         rc = ntuple_stages_check(h_stages, h_placements, n_placements, n_weights, invalid);
         if (rc) return rc;
     }
+    if (car && !(staged && h_stages->n_thresholds >= 1)) return nt_fail(who, "carousel shaping needs at least 2 stages");
     if (!(d_boards && d_after && d_scores && d_lengths && d_weights && d_scratch)) return nt_fail(who, "pointers");
     if (!(n_steps == 0 || d_subs)) return nt_fail(who, "pointers");
     if (tc && !(d_err_sum && d_abs_err_sum)) return nt_fail(who, "pointers");
@@ -522,9 +577,15 @@ int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t
         if (!(lam->horizon >= 1 && lam->horizon <= G2048_NTUPLE_MAX_HORIZON))
             return nt_fail(who, "horizon must be in [1, G2048_NTUPLE_MAX_HORIZON]");
         if (n * lam->horizon > (1ll << 20)) return nt_fail(who, "n * horizon must be <= 2^20");
-        if (!(lam->hist_after && lam->hist_delta)) return nt_fail(who, "pointers");
+        // the carousel forms run h = 1 without the window, so they take NULL rings there
+        if (!(lam->hist_after && lam->hist_delta) && !(car && lam->horizon == 1)) return nt_fail(who, "pointers");
         if (!(((uintptr_t)lam->hist_after & 7u) == 0 && ((uintptr_t)lam->hist_delta & 3u) == 0))
             return nt_fail(who, "d_hist_after must be 8-byte and d_hist_delta 4-byte aligned");
+    }
+    if (car) {
+        if (!(car->start_stage && car->stage_pool)) return nt_fail(who, "pointers");
+        if (!(((uintptr_t)car->start_stage & 3u) == 0 && ((uintptr_t)car->stage_pool & 7u) == 0))
+            return nt_fail(who, "d_start_stage must be 4-byte and d_stage_pool 8-byte aligned");
     }
     if (n_steps == 0) return G2048_OK;
     const NtScratch lay = nt_scratch_layout(lam ? n * lam->horizon : n, n_placements, n_weights, tc);
@@ -557,7 +618,16 @@ int nt_train(const char* who, bool tc, bool staged, uint64_t* d_boards, uint64_t
     args.horizon = lam ? (uint32_t)lam->horizon : 0u;
     args.hist_after = lam ? (u64*)lam->hist_after : nullptr;
     args.hist_delta = lam ? lam->hist_delta : nullptr;
+    args.start_stage = car ? car->start_stage : nullptr;
+    args.pool = car ? (u64*)car->stage_pool : nullptr;
+    args.pending = car ? (u64*)((uint8_t*)d_scratch + lay.bytes) : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
+    if (car) {  // h = 1 is the staged TD(0) / TC step, without the ring traffic
+        if (lam->horizon > 1) return tc ? nt_launch<true, true, true, true>(who, rng_mode, args, st)
+                                        : nt_launch<false, true, true, true>(who, rng_mode, args, st);
+        return tc ? nt_launch<true, true, false, true>(who, rng_mode, args, st)
+                  : nt_launch<false, true, false, true>(who, rng_mode, args, st);
+    }
     if (lam) {
         if (staged) return tc ? nt_launch<true, true, true>(who, rng_mode, args, st)
                               : nt_launch<false, true, true>(who, rng_mode, args, st);
@@ -643,4 +713,40 @@ extern "C" int g2048_ntuple_lambda_tc_train(uint64_t* d_boards, uint64_t* d_afte
     return nt_train("ntuple_lambda_tc_train", true, h_stages != nullptr, d_boards, d_after, d_scores, d_lengths, n,
                     h_placements, n_placements, h_stages, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha,
                     d_subs, n_steps, rng_mode, d_scratch, d_stats, stream, &lam);
+}
+
+extern "C" int64_t g2048_ntuple_carousel_scratch_bytes(int64_t n, int horizon, int n_placements, int64_t n_weights,
+                                                       int tc) {
+    if (!(horizon >= 1 && horizon <= G2048_NTUPLE_MAX_HORIZON) || n < 1 || n * horizon > (1ll << 20)) return -1;
+    const int64_t bytes = nt_scratch_bytes(n * horizon, n_placements, n_weights, tc != 0);
+    return bytes < 0 ? -1 : bytes + 8 * n;  // the pending words
+}
+
+extern "C" int g2048_ntuple_carousel_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                              uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                              int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                              int64_t n_weights, float alpha, float lambda, int horizon,
+                                              uint64_t* d_hist_after, float* d_hist_delta, uint32_t* d_start_stage,
+                                              uint64_t* d_stage_pool, const uint32_t* d_subs, int64_t n_steps,
+                                              int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream) {
+    const NtLambda lam{lambda, horizon, d_hist_after, d_hist_delta};
+    const NtCarousel car{d_start_stage, d_stage_pool};
+    return nt_train("ntuple_carousel_td_train", false, h_stages != nullptr, d_boards, d_after, d_scores, d_lengths, n,
+                    h_placements, n_placements, h_stages, d_weights, n_weights, nullptr, nullptr, alpha, d_subs,
+                    n_steps, rng_mode, d_scratch, d_stats, stream, &lam, &car);
+}
+
+extern "C" int g2048_ntuple_carousel_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores,
+                                              uint32_t* d_lengths, int64_t n, const G2048TuplePlacement* h_placements,
+                                              int n_placements, const G2048TupleStages* h_stages, float* d_weights,
+                                              int64_t n_weights, double* d_err_sum, double* d_abs_err_sum, float alpha,
+                                              float lambda, int horizon, uint64_t* d_hist_after, float* d_hist_delta,
+                                              uint32_t* d_start_stage, uint64_t* d_stage_pool, const uint32_t* d_subs,
+                                              int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats,
+                                              void* stream) {
+    const NtLambda lam{lambda, horizon, d_hist_after, d_hist_delta};
+    const NtCarousel car{d_start_stage, d_stage_pool};
+    return nt_train("ntuple_carousel_tc_train", true, h_stages != nullptr, d_boards, d_after, d_scores, d_lengths, n,
+                    h_placements, n_placements, h_stages, d_weights, n_weights, d_err_sum, d_abs_err_sum, alpha,
+                    d_subs, n_steps, rng_mode, d_scratch, d_stats, stream, &lam, &car);
 }

@@ -134,6 +134,11 @@ __device__ __forceinline__ uint32_t nt_stage_base(const NtStages& st, u64 b) {
     return (uint32_t)(st.stage_of >> (4 * max_exponent(b)) & 15u) * st.stride;
 }
 
+// stage(b)
+__device__ __forceinline__ uint32_t nt_stage(const NtStages& st, u64 b) {
+    return (uint32_t)(st.stage_of >> (4 * max_exponent(b)) & 15u);
+}
+
 // V_S(b) of a multi-stage network
 template <bool COHERENT>
 __device__ __forceinline__ float nt_value_staged(const NtNet& net, const NtStages& st, u64 b) {

@@ -85,7 +85,12 @@ _SIGNATURES = {
                                             _I64, _INT, _P, _P, _P]),
     "g2048_ntuple_lambda_tc_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _P, _P, _FLT, _FLT, _INT, _P, _P,
                                             _P, _I64, _INT, _P, _P, _P]),
-    "g2048_play_host": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),
+    "g2048_ntuple_carousel_scratch_bytes": (_I64, [_I64, _INT, _INT, _I64, _INT]),
+    "g2048_ntuple_carousel_td_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _FLT, _FLT, _INT, _P, _P, _P,
+                                              _P, _P, _I64, _INT, _P, _P, _P]),
+    "g2048_ntuple_carousel_tc_train": (_INT, [_P, _P, _P, _P, _I64, _P, _INT, _P, _P, _I64, _P, _P, _FLT, _FLT, _INT, _P,
+                                              _P, _P, _P, _P, _I64, _INT, _P, _P, _P]),
+    "g2048_play_host":(_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),
     "g2048_play_host_packed": (_INT, [_INT, _U64, _P, _I64, _I64, _I64, _INT, _P, _P]),
     "g2048_play_packed": (_INT, [_INT, _P, _I64, _I64, _I64, _I64, _INT, _P, _P, _P, _P]),
     "g2048_rollout_steps": (_INT, [_INT, _P, _P, _P, _I64, _I64, _I64, _I64, _I64, _INT, _P, _P, _P, _P, _P, _P]),

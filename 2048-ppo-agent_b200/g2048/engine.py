@@ -440,7 +440,8 @@ def ntuple_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Ten
 
 def _lambda_checks(who: str, boards: torch.Tensor, placements: np.ndarray, weights: torch.Tensor, lam: float,
                    hist_after: torch.Tensor, hist_delta: torch.Tensor, scratch: torch.Tensor, tc: bool) -> int:
-    """The checks of the lambda wrappers (ValueError); returns the horizon h = hist_after.shape[0]."""
+    """The checks of the lambda wrappers (ValueError); returns the horizon h = hist_after.shape[0].  ``scratch`` None
+    skips the scratch size (the carousel wrappers check their own)."""
     from .ntuple import MAX_HORIZON
 
     n = boards.shape[0]
@@ -461,6 +462,8 @@ def _lambda_checks(who: str, boards: torch.Tensor, placements: np.ndarray, weigh
             raise ValueError(f"{who}: the rings must be contiguous and on {boards.device}")
     if n * h > 1 << 20:
         raise ValueError(f"{who}: n * h must be <= 2^20, got {n} * {h}")
+    if scratch is None:
+        return h
     size_of = N.lib.g2048_ntuple_tc_scratch_bytes if tc else N.lib.g2048_ntuple_td_scratch_bytes
     need = int(size_of(n * h, placements.shape[0], weights.numel()))
     if need < 0 or scratch.numel() * scratch.element_size() < need:
@@ -511,6 +514,102 @@ def ntuple_lambda_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: to
     call("g2048_ntuple_lambda_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
          _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), ptr(err_sum),
          ptr(abs_err_sum), float(alpha), float(lam), h, ptr(hist_after), ptr(hist_delta), ptr(_i32(subs)),
+         subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
+
+
+def ntuple_carousel_scratch(n: int, horizon: int, placements: np.ndarray, n_weights: int, tc: bool,
+                            device) -> torch.Tensor:
+    """Zeroed scratch of g2048_ntuple_carousel_td_train (tc False) / _tc_train (tc True) for n envs, window h =
+    ``horizon`` and this network (every call leaves it zeroed)."""
+    size = int(N.lib.g2048_ntuple_carousel_scratch_bytes(n, int(horizon), placements.shape[0], n_weights, int(bool(tc))))
+    if size < 0:
+        raise ValueError("ntuple_carousel_scratch: invalid sizes")
+    return torch.zeros(size // 8, dtype=torch.int64, device=device)
+
+
+def _carousel_checks(who: str, boards: torch.Tensor, placements: np.ndarray, weights: torch.Tensor, lam: float,
+                     hist_after, hist_delta, start_stage: torch.Tensor, stage_pool: torch.Tensor, stages,
+                     scratch: torch.Tensor, tc: bool) -> tuple[int, int, int, np.ndarray, int]:
+    """The checks of the carousel wrappers (ValueError): the lambda wrappers' when h > 1, the stages (S >= 2) and the
+    carousel arrays.  Returns (h, hist_after pointer, hist_delta pointer, the stages' checked copy, its pointer);
+    ``hist_after`` / ``hist_delta`` None means h = 1 without rings."""
+    n = boards.shape[0]
+    if stages is None:
+        raise ValueError(f"{who}: carousel shaping needs a multi-stage network (stages with S >= 2)")
+    st, st_ptr = _stages_ptr(stages, placements, weights.numel())
+    if int(st["n_thresholds"][0]) < 1:
+        raise ValueError(f"{who}: carousel shaping needs a multi-stage network (stages with S >= 2), got one stage")
+    S = int(st["n_thresholds"][0]) + 1
+    if (hist_after is None) != (hist_delta is None):
+        raise ValueError(f"{who}: hist_after and hist_delta must both be given or both be None")
+    if hist_after is None:
+        lam = float(lam)
+        if not (math.isfinite(lam) and 0.0 <= lam <= 1.0):
+            raise ValueError(f"{who}: lambda must be finite and in [0, 1], got {lam}")
+        h, ha_ptr, hd_ptr = 1, None, None
+    else:
+        h = _lambda_checks(who, boards, placements, weights, lam, hist_after, hist_delta, None, tc)
+        ha_ptr, hd_ptr = ptr(hist_after), ptr(hist_delta)
+    if not (isinstance(start_stage, torch.Tensor) and start_stage.dtype == torch.int32
+            and tuple(start_stage.shape) == (n,)):
+        raise ValueError(f"{who}: start_stage must be an int32 tensor of shape ({n},)")
+    if not (isinstance(stage_pool, torch.Tensor) and stage_pool.dtype == torch.int64
+            and tuple(stage_pool.shape) == (S - 1, n)):
+        raise ValueError(f"{who}: stage_pool must be an int64 tensor of shape ({S - 1}, {n})")
+    for t in (start_stage, stage_pool):
+        if t.device != boards.device or not t.is_contiguous():
+            raise ValueError(f"{who}: start_stage and stage_pool must be contiguous and on {boards.device}")
+    need = int(N.lib.g2048_ntuple_carousel_scratch_bytes(n, h, placements.shape[0], weights.numel(), int(tc)))
+    if need < 0 or scratch.numel() * scratch.element_size() < need:
+        raise ValueError(f"{who}: scratch holds {scratch.numel() * scratch.element_size()} bytes, this batch, horizon "
+                         f"and network need {need} (ntuple_carousel_scratch)")
+    return h, ha_ptr, hd_ptr, st, st_ptr
+
+
+def ntuple_carousel_td_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                             placements: np.ndarray, weights: torch.Tensor, alpha: float, lam: float,
+                             hist_after: torch.Tensor | None, hist_delta: torch.Tensor | None,
+                             start_stage: torch.Tensor, stage_pool: torch.Tensor, subs: torch.Tensor, rng_mode: int,
+                             scratch: torch.Tensor, stats: torch.Tensor | None = None,
+                             stages: np.ndarray | None = None) -> None:
+    """``subs.shape[0]`` synchronous TD steps of a multi-stage network with carousel shaping
+    (g2048_ntuple_carousel_td_train): ``ntuple_lambda_td_train`` (``hist_after`` / ``hist_delta`` None: h = 1, TD(0)),
+    where an episode that ends restarts, in turn, at the opening or from a board at which an earlier episode entered
+    the next stage.  ``start_stage`` (int32, (n,)) and ``stage_pool`` (int64, (S - 1, n)) are updated in place (zeros
+    at the start of a run).  ``stages``: the network's G2048TupleStages record, S >= 2, required.  ``scratch``:
+    ``ntuple_carousel_scratch(n, h, ..., tc=False)``."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    h, ha, hd, st, st_ptr = _carousel_checks("ntuple_carousel_td_train", boards, placements, weights, lam, hist_after,
+                                             hist_delta, start_stage, stage_pool, stages, scratch, False)
+    call("g2048_ntuple_carousel_td_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+         _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), float(alpha),
+         float(lam), h, ha, hd, ptr(start_stage), ptr(stage_pool), ptr(_i32(subs)), subs.shape[0], rng_mode,
+         ptr(scratch), ptr(stats), stream_ptr())
+
+
+def ntuple_carousel_tc_train(boards: torch.Tensor, after: torch.Tensor, scores: torch.Tensor, lengths: torch.Tensor,
+                             placements: np.ndarray, weights: torch.Tensor, err_sum: torch.Tensor,
+                             abs_err_sum: torch.Tensor, alpha: float, lam: float, hist_after: torch.Tensor | None,
+                             hist_delta: torch.Tensor | None, start_stage: torch.Tensor, stage_pool: torch.Tensor,
+                             subs: torch.Tensor, rng_mode: int, scratch: torch.Tensor,
+                             stats: torch.Tensor | None = None, stages: np.ndarray | None = None) -> None:
+    """``subs.shape[0]`` synchronous TC steps with carousel shaping (g2048_ntuple_carousel_tc_train):
+    ``ntuple_lambda_tc_train``'s E / A update with ``ntuple_carousel_td_train``'s restarts.  ``scratch``:
+    ``ntuple_carousel_scratch(n, h, ..., tc=True)``."""
+    n = boards.shape[0]
+    assert boards.dtype == after.dtype == torch.int64 and scores.dtype == lengths.dtype == torch.int32
+    assert after.shape[0] == scores.shape[0] == lengths.shape[0] == n
+    assert weights.dtype == torch.float32 and weights.is_contiguous()
+    for s in (err_sum, abs_err_sum):
+        assert s.dtype == torch.float64 and s.is_contiguous() and s.numel() == weights.numel()
+    h, ha, hd, st, st_ptr = _carousel_checks("ntuple_carousel_tc_train", boards, placements, weights, lam, hist_after,
+                                             hist_delta, start_stage, stage_pool, stages, scratch, True)
+    call("g2048_ntuple_carousel_tc_train", ptr(boards), ptr(after), ptr(scores), ptr(lengths), n,
+         _placements_ptr(placements), placements.shape[0], st_ptr, ptr(weights), weights.numel(), ptr(err_sum),
+         ptr(abs_err_sum), float(alpha), float(lam), h, ha, hd, ptr(start_stage), ptr(stage_pool), ptr(_i32(subs)),
          subs.shape[0], rng_mode, ptr(scratch), ptr(stats), stream_ptr())
 
 

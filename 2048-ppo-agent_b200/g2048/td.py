@@ -26,6 +26,15 @@ network TC(lambda) learned better players than TC and TD(0), and TD(lambda) wors
 (profiles/README.md, round 11):
 
     learner = g2048.NTupleTCLearner(0, batch_size=1 << 16, lam=0.5, horizon=3)
+
+With ``carousel=True`` a multi-stage network is learned with carousel shaping (``g2048_ntuple_carousel_td_train`` /
+``_tc_train``, any horizon): an episode that ends restarts, in turn, at the opening or from a board at which an
+earlier episode entered stage 1, 2, ..., so that the later stages' tables see a fair share of the training.  The
+summary of ``train`` then also counts those shaped episodes (``shaped_episodes``, ``shaped_env_steps``); the other
+entries count only the episodes that began at the opening (profiles/README.md, round 12):
+
+    net = g2048.NTupleNetwork.staged(g2048.NTupleNetwork.four_six(), (13,))
+    learner = g2048.NTupleTCLearner(0, batch_size=1 << 16, network=net, lam=0.5, horizon=3, carousel=True)
 """
 from __future__ import annotations
 
@@ -93,6 +102,16 @@ def _check_ring(ring, shape, dtype, name) -> torch.Tensor:
     return ring
 
 
+def _check_start_stage(t, n: int, n_stages: int) -> torch.Tensor:
+    """A checkpoint's start_stage: an int32 (n,) tensor with values in [0, n_stages), or ValueError."""
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or tuple(t.shape) != (n,):
+        got = (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t).__name__
+        raise ValueError(f"start_stage must be a torch.int32 tensor of shape ({n},), got {got}")
+    if bool(((t < 0) | (t >= n_stages)).any()):
+        raise ValueError(f"start_stage values must lie in [0, {n_stages})")
+    return t
+
+
 def _resolved(device) -> torch.device:
     """``device`` with the current CUDA device filled in for a bare "cuda"."""
     device = torch.device(device)
@@ -142,6 +161,9 @@ class _BatchTDLearner:
             self._launch(subs, stats)
             self.chain.consume(n_steps)
             self.steps += n_steps
+        return self._summary(stats)
+
+    def _summary(self, stats: torch.Tensor) -> dict:
         return E.play_stats_dict(stats)
 
     # -- checkpointing: key chain, env state and the value function ----------------------------------------------
@@ -226,10 +248,16 @@ class NTupleTDLearner(_BatchTDLearner):
     and a load whose placements, n_weights or stages differ from the learner's network is rejected before anything
     changes (a checkpoint without stages is a single-stage network's).  With ``horizon > 1`` it also holds ``lam``,
     ``horizon`` and both rings; a load with another horizon or with rings of the wrong shape or dtype is rejected, and
-    a checkpoint without them is a ``horizon=1`` learner's."""
+    a checkpoint without them is a ``horizon=1`` learner's.
+    ``carousel``: carousel shaping of a multi-stage network (a single-stage one is a ValueError), through
+    ``g2048_ntuple_carousel_td_train`` for every horizon.  The learner then holds ``start_stage`` (int32 (batch_size,))
+    and ``stage_pool`` (int64 (S - 1, batch_size)), zeros at construction, and its checkpoint holds ``carousel`` and
+    both; a load with another carousel setting, arrays of the wrong shape or dtype, or a start stage outside [0, S)
+    is rejected before anything changes."""
 
     def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
-                 alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None, lam: float = 0.0, horizon: int = 1):
+                 alpha: float = DEFAULT_NTUPLE_ALPHA, rng_mode=None, device=None, lam: float = 0.0, horizon: int = 1,
+                 carousel: bool = False):
         self.batch_size, self.alpha = self._check_common(batch_size, alpha)
         self.lam = _check_lam(lam)
         self.horizon = _check_horizon(horizon)
@@ -237,6 +265,11 @@ class NTupleTDLearner(_BatchTDLearner):
             raise ValueError(f"batch_size * horizon must be <= 2^20, got {self.batch_size} * {self.horizon}")
         if network is not None and not isinstance(network, NTupleNetwork):
             raise ValueError("network must be an NTupleNetwork")
+        if not isinstance(carousel, (bool, np.bool_)):
+            raise ValueError(f"carousel must be a bool, got {carousel!r}")
+        self.carousel = bool(carousel)
+        if self.carousel and (network is None or network.n_stages < 2):
+            raise ValueError("carousel shaping needs a multi-stage network (NTupleNetwork.staged)")
         self._start(rng_mode, device)
         self.network = NTupleNetwork.four_six(device=self.device) if network is None else network
         if _resolved(self.network.weights.device) != _resolved(self.device):
@@ -246,11 +279,28 @@ class NTupleTDLearner(_BatchTDLearner):
             shape = (self.horizon, self.batch_size)
             self.hist_after = torch.zeros(shape, dtype=torch.int64, device=self.device)
             self.hist_delta = torch.zeros(shape, dtype=torch.float32, device=self.device)
+        if self.carousel:
+            self.start_stage = torch.zeros(self.batch_size, dtype=torch.int32, device=self.device)
+            self.stage_pool = torch.zeros((self.network.n_stages - 1, self.batch_size), dtype=torch.int64,
+                                          device=self.device)
         self._scratch = self._new_scratch()
 
     def _new_scratch(self) -> torch.Tensor:
+        if self.carousel:
+            return E.ntuple_carousel_scratch(self.batch_size, self.horizon, self.network.placements,
+                                             self.network.n_weights, False, self.device)
         return E.ntuple_td_scratch(self.batch_size * self.horizon, self.network.placements, self.network.n_weights,
                                    self.device)
+
+    def _rings(self) -> tuple:
+        return (self.hist_after, self.hist_delta) if self.horizon > 1 else (None, None)
+
+    def _summary(self, stats: torch.Tensor) -> dict:
+        out = E.play_stats_dict(stats)
+        if self.carousel:
+            words = stats.cpu()
+            out.update(shaped_episodes=int(words[12]), shaped_env_steps=int(words[13]))
+        return out
 
     @property
     def weights(self) -> torch.Tensor:
@@ -258,6 +308,11 @@ class NTupleTDLearner(_BatchTDLearner):
 
     def _launch(self, subs, stats) -> None:
         net = self.network
+        if self.carousel:
+            E.ntuple_carousel_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
+                                       self.alpha, self.lam, *self._rings(), self.start_stage, self.stage_pool, subs,
+                                       self.rng_mode, self._scratch, stats, stages=net.stages)
+            return
         if self.horizon > 1:
             E.ntuple_lambda_td_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
                                      self.alpha, self.lam, self.hist_after, self.hist_delta, subs, self.rng_mode,
@@ -274,7 +329,23 @@ class NTupleTDLearner(_BatchTDLearner):
         if self.horizon > 1:
             out.update({"lam": self.lam, "horizon": self.horizon, "hist_after": self.hist_after.cpu().clone(),
                         "hist_delta": self.hist_delta.cpu().clone()})
+        if self.carousel:
+            out.update({"carousel": True, "start_stage": self.start_stage.cpu().clone(),
+                        "stage_pool": self.stage_pool.cpu().clone()})
         return out
+
+    def _check_carousel_state(self, state):
+        """The checkpoint's carousel arrays: None without carousel, else (start_stage, stage_pool); ValueError if they
+        do not fit this learner."""
+        carousel = state.get("carousel", False)
+        if not isinstance(carousel, (bool, np.bool_)) or bool(carousel) != self.carousel:
+            raise ValueError(f"checkpoint was written with carousel={carousel!r}, this learner has "
+                             f"carousel={self.carousel}")
+        if not self.carousel:
+            return None
+        S = self.network.n_stages
+        start_stage = _check_start_stage(state.get("start_stage"), self.batch_size, S)
+        return start_stage, _check_ring(state.get("stage_pool"), (S - 1, self.batch_size), torch.int64, "stage_pool")
 
     def _check_window_state(self, state):
         """The checkpoint's window: None for horizon 1, else (lam, hist_after, hist_delta); ValueError if it does not
@@ -302,15 +373,19 @@ class NTupleTDLearner(_BatchTDLearner):
         if thresholds != net.stage_thresholds or int(state.get("stage_stride", 0)) != net.stage_stride:
             raise ValueError("checkpoint was written for a network with different stages")
         window = self._check_window_state(state)
-        return _check_weights(state["weights"], net.n_weights), window
+        carousel = self._check_carousel_state(state)
+        return _check_weights(state["weights"], net.n_weights), window, carousel
 
     def _load_values(self, values) -> None:
-        weights, window = values
+        weights, window, carousel = values
         self.network.weights.copy_(weights.to(self.device))
         if window is not None:
             self.lam = window[0]
             self.hist_after.copy_(window[1].to(self.device))
             self.hist_delta.copy_(window[2].to(self.device))
+        if carousel is not None:
+            self.start_stage.copy_(carousel[0].to(self.device))
+            self.stage_pool.copy_(carousel[1].to(self.device))
 
 
 def _check_sums(sums, n_weights: int, name: str) -> torch.Tensor:
@@ -333,24 +408,34 @@ class NTupleTCLearner(NTupleTDLearner):
     sign keep a large step, weights whose errors cancel stop moving (g2048_ntuple_tc_train, include/g2048.h).
 
     ``network`` may hold weights learned before (for example by ``NTupleTDLearner``): TC starts from them with
-    E = A = 0.  ``lam`` / ``horizon``: delayed TC(lambda), the window of ``NTupleTDLearner``.  ``state_dict`` /
+    E = A = 0.  ``lam`` / ``horizon``: delayed TC(lambda), the window of ``NTupleTDLearner``; ``carousel``: its carousel
+    shaping (``g2048_ntuple_carousel_tc_train``).  ``state_dict`` /
     ``load_state_dict`` resume a run bit for bit, E and A included."""
 
     def __init__(self, init_seed: int, batch_size: int, network: NTupleNetwork | None = None,
                  alpha: float = DEFAULT_NTUPLE_TC_ALPHA, rng_mode=None, device=None, lam: float = 0.0,
-                 horizon: int = 1):
+                 horizon: int = 1, carousel: bool = False):
         super().__init__(init_seed, batch_size, network=network, alpha=alpha, rng_mode=rng_mode, device=device,
-                         lam=lam, horizon=horizon)
+                         lam=lam, horizon=horizon, carousel=carousel)
         n_weights = self.network.n_weights
         self.err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
         self.abs_err_sum = torch.zeros(n_weights, dtype=torch.float64, device=self.device)
 
     def _new_scratch(self) -> torch.Tensor:
+        if self.carousel:
+            return E.ntuple_carousel_scratch(self.batch_size, self.horizon, self.network.placements,
+                                             self.network.n_weights, True, self.device)
         return E.ntuple_tc_scratch(self.batch_size * self.horizon, self.network.placements, self.network.n_weights,
                                    self.device)
 
     def _launch(self, subs, stats) -> None:
         net = self.network
+        if self.carousel:
+            E.ntuple_carousel_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
+                                       self.err_sum, self.abs_err_sum, self.alpha, self.lam, *self._rings(),
+                                       self.start_stage, self.stage_pool, subs, self.rng_mode, self._scratch, stats,
+                                       stages=net.stages)
+            return
         if self.horizon > 1:
             E.ntuple_lambda_tc_train(self.boards, self.after, self.scores, self.lengths, net.placements, net.weights,
                                      self.err_sum, self.abs_err_sum, self.alpha, self.lam, self.hist_after,

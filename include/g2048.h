@@ -417,6 +417,54 @@ int g2048_ntuple_lambda_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t
                                  uint64_t* d_hist_after, float* d_hist_delta, const uint32_t* d_subs, int64_t n_steps,
                                  int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream);
 
+/* ---- Carousel shaping of a multi-stage network (Jaskowski 2018): episodes take turns starting at the opening and
+ * from the boards at which earlier episodes entered stage 1, 2, ..., so that the later stages get a fair share of the
+ * training.  g2048_ntuple_lambda_td_train / _tc_train word for word (h = 1: TD(0) / TC), with d_hist_after and
+ * d_hist_delta allowed to be NULL when horizon == 1, h_stages required with S >= 2, and two caller-owned arrays:
+ *   d_start_stage: uint32[n], per env the stage its current episode began in (4-byte aligned).
+ *   d_stage_pool:  uint64[(S - 1) * n], stage-major (8-byte aligned): entry (l - 1, e) at (l - 1) * n + e is the board
+ *           at which env e most recently entered stage l; 0 is none.
+ * Zeroed arrays are a valid start: such a run is the staged learner's until the first stage entry.  Only step 3 and
+ * the statistics change:
+ *   Recording (an env that moves): s is the board at the start of the step, s' = spawn(best) its new board.  If
+ *           stage(s') > stage(s) (by 1: the thresholds are strictly increasing and the largest exponent grows by at
+ *           most 1 a move), s' is written to pool entry (stage(s') - 1, e).  The write is visible from step t + 1:
+ *           every draw of step t reads the pool as it was at the start of step t, which keeps the results bit-exact
+ *           and independent of the grid.
+ *   Restart (an env without a legal move): c = start_stage[e], l = c + 1 if c + 1 < S, else 0 (c >= S - 1 wraps to 0).
+ *           If l >= 1: split2(k, k1, k2) with the env's step key k, j = (uint32)(((uint64)bits_scalar(k1) * n) >> 32),
+ *           b = pool entry (l - 1, j) as it was at the start of the step; if b != 0 the env restarts from b with
+ *           start_stage[e] = l.  Otherwise (l = 0 or an empty entry) it restarts from init(k) as before, with
+ *           start_stage[e] = 0.  In both cases after, score and length go to 0.  Pool boards that hold a 2^15 tile are
+ *           outside the contract, as for d_boards.
+ *   Statistics: words [0..7] and [16 + e] count only the episodes that began at the opening (start_stage == 0), so
+ *           summaries stay comparable with the other learners'; the episodes that began from a pool board add 1 to
+ *           word [12] and their length to word [13].
+ * Equivalence: if no env enters a stage during a call, the pool stays as it was, and with an empty pool every restart
+ * takes init(k): the call then equals g2048_ntuple_staged_td_train / _tc_train (h = 1) or
+ * g2048_ntuple_lambda_td_train / _tc_train (h > 1) bit for bit -- W, E, A, the env state, the rings and the
+ * statistics.
+ *   d_scratch: g2048_ntuple_carousel_scratch_bytes(n, horizon, n_placements, n_weights, tc) bytes: the lambda form's
+ *           scratch for n * h envs, then one pending board per env (uint64[n]) that holds a stage entry until the
+ *           pool takes it after the step's draws.  Zeroed by the caller once; every call leaves it zeroed.  -1 for
+ *           invalid sizes.
+ * G2048_ERR_INVALID before any launch for everything the lambda entry points reject, NULL h_stages or S = 1, and NULL
+ * or misaligned d_start_stage / d_stage_pool. */
+int64_t g2048_ntuple_carousel_scratch_bytes(int64_t n, int horizon, int n_placements, int64_t n_weights, int tc);
+int g2048_ntuple_carousel_td_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                   int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                   const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights, float alpha,
+                                   float lambda, int horizon, uint64_t* d_hist_after, float* d_hist_delta,
+                                   uint32_t* d_start_stage, uint64_t* d_stage_pool, const uint32_t* d_subs,
+                                   int64_t n_steps, int rng_mode, void* d_scratch, uint64_t* d_stats, void* stream);
+int g2048_ntuple_carousel_tc_train(uint64_t* d_boards, uint64_t* d_after, uint32_t* d_scores, uint32_t* d_lengths,
+                                   int64_t n, const G2048TuplePlacement* h_placements, int n_placements,
+                                   const G2048TupleStages* h_stages, float* d_weights, int64_t n_weights,
+                                   double* d_err_sum, double* d_abs_err_sum, float alpha, float lambda, int horizon,
+                                   uint64_t* d_hist_after, float* d_hist_delta, uint32_t* d_start_stage,
+                                   uint64_t* d_stage_pool, const uint32_t* d_subs, int64_t n_steps, int rng_mode,
+                                   void* d_scratch, uint64_t* d_stats, void* stream);
+
 /* Host-buffer form of the same call (the reference-facing entry: run_actions_max_tile's inner
  * run).  seed -> jax.random.key(seed); h_key_io (2 words, may be NULL) overrides the seed with an
  * explicit chain key and receives the key the reference's runner would hold afterwards.

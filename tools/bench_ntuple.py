@@ -47,7 +47,21 @@ horizon) instead:
     evaluation continues the first): learning curve, training wall time, greedy and depth-2 players on the seed-7 games;
     then one staged (13,) run of the best setting at --long-steps, next to staged TD(0).
 
-    python tools/bench_ntuple.py [--tc | --stages | --lambda] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
+With --carousel, carousel shaping of multi-stage networks (g2048_ntuple_carousel_td_train / _tc_train, the learners'
+carousel) instead:
+  * speed of the mechanism: at n = 2^14, 2^16 and 2^18, the 4x6 network trained by TD for --carousel-pretrain-steps
+    untimed steps, then staged (14,) copies of it with and without the carousel (TD(0)), carrying on from the same envs,
+    their timed launches alternated; few envs reach a 16384 tile, so the pool stays (nearly) empty and the ratio
+    isolates the mechanism.  Each carousel row reports the non-zero pool entries after timing;
+  * speed with a real mix: the same after --pretrain-steps untimed steps with (13,) copies, with the time-averaged
+    share of envs per stage and (carousel) per start stage;
+  * quality from the zero 4x6 network at n = 2^16 (seed 0), TC(lambda = 0.5, h = 3) at alpha 0.02: unstaged, staged
+    (13,), staged (13,) with the carousel, and half of --sweep-steps unstaged then staged((13,)) with the carousel;
+    evaluated after --sweep-steps and, continuing the same runs, after --long-steps steps: greedy and depth-2 players
+    on the seed-7 games, the share of env-steps in stage 1 (of (13,), sampled after every block) and the stage-1
+    entries ever updated (A > 0).
+
+    python tools/bench_ntuple.py [--tc | --stages | --lambda | --carousel] [--long-steps 40000] [--steps 500] [--sweep-steps 4000] [--games 1024] [--deep-games 128] [--speed-only | --skip-speed] [--out FILE]
 """
 import argparse
 import json
@@ -312,15 +326,20 @@ def _staged_run(lr, subs):
                                      subs, MODE, lr._scratch, stages=net.stages)
 
 
-def _promoted(lr, thresholds):
-    """A learner of staged(lr.network, thresholds) that carries on from lr's env state and key chain: at the start it
-    has exactly lr's values, so it plays lr's games."""
-    promoted = g2048.NTupleTDLearner(0, lr.batch_size, network=NTupleNetwork.staged(lr.network, thresholds),
-                                     alpha=lr.alpha, rng_mode=lr.rng_mode)
+def _promoted(lr, thresholds, carousel=False):
+    """A learner of lr's class of staged(lr.network, thresholds) that carries on from lr's env state, window and key
+    chain: at the start it has exactly lr's values, so it plays lr's games.  A TC learner's E and A are copied into
+    every stage, as the weights are.  ``carousel``: the new learner shapes, from an empty pool."""
+    promoted = type(lr)(0, lr.batch_size, network=NTupleNetwork.staged(lr.network, thresholds), alpha=lr.alpha,
+                        rng_mode=lr.rng_mode, lam=lr.lam, horizon=lr.horizon, carousel=carousel)
     ckpt = lr.state_dict()
-    for k in ("placements", "n_weights", "weights", "stage_thresholds", "stage_stride"):
-        ckpt.pop(k)
-    ckpt.update(promoted._values_state())
+    for k in ("placements", "n_weights", "weights", "stage_thresholds", "stage_stride", "err_sum", "abs_err_sum"):
+        ckpt.pop(k, None)
+    for k, v in promoted._values_state().items():
+        ckpt.setdefault(k, v)  # lr's window stays
+    if isinstance(lr, g2048.NTupleTCLearner):
+        S = len(thresholds) + 1
+        ckpt["err_sum"], ckpt["abs_err_sum"] = lr.err_sum.cpu().repeat(S), lr.abs_err_sum.cpu().repeat(S)
     promoted.load_state_dict(ckpt)
     return promoted
 
@@ -612,6 +631,133 @@ def main_lambda(args) -> None:
     _emit(result, args.out)
 
 
+def _carousel_run(lr, subs):
+    net = lr.network
+    return lambda: E.ntuple_carousel_td_train(lr.boards, lr.after, lr.scores, lr.lengths, net.placements, net.weights,
+                                              lr.alpha, 0.0, None, None, lr.start_stage, lr.stage_pool, subs, MODE,
+                                              lr._scratch, stages=net.stages)
+
+
+def _start_shares(lr) -> list:
+    return [round(float((lr.start_stage == s).float().mean()), 4) for s in range(lr.network.n_stages)]
+
+
+def carousel_speed(steps: int, pretrain: int, thresholds, reps: int = 3) -> list:
+    """At each size, the 4x6 network trained by TD (alpha 0.02, seed 0) for `pretrain` untimed steps, then staged
+    copies at `thresholds` with and without the carousel, which carry on from the same envs; their timed launches
+    alternated.  The carousel row carries its rate over the staged one, the non-zero pool entries after timing, and
+    (both) the share of envs per stage and, for the carousel, per start stage, averaged over samples taken before and
+    after every timed launch."""
+    out = []
+    subs = E.chain_advance(E.words_tensor([0, 1], "cuda"), MODE, steps)
+    for n in SIZES:
+        flat = g2048.NTupleTDLearner(0, n, alpha=g2048.td.DEFAULT_NTUPLE_ALPHA, rng_mode=MODE)
+        flat.train(pretrain)
+        learners = {"staged": _promoted(flat, thresholds), "carousel": _promoted(flat, thresholds, carousel=True)}
+        del flat
+        torch.cuda.empty_cache()
+        runs = {"staged": _staged_run(learners["staged"], subs), "carousel": _carousel_run(learners["carousel"], subs)}
+        for run in runs.values():
+            run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in runs}
+        shares = {k: [] for k in runs}
+        starts = []
+        for _ in range(reps):
+            for k, run in runs.items():
+                sample = lambda lr=learners[k]: (shares[k].append(_stage_shares(lr.boards, thresholds)),  # noqa: E731
+                                                 lr.carousel and starts.append(_start_shares(lr)))
+                sample()
+                times[k].append(_timed_once(run))
+                sample()
+        rows = [_row(k, n, steps, times[k], pretrain_steps=pretrain, stage_thresholds=list(thresholds)) for k in runs]
+        for row in rows:
+            samples = shares[row["what"]]
+            row["mean_share_of_envs_per_stage"] = [round(sum(x[s] for x in samples) / len(samples), 4)
+                                                   for s in range(len(samples[0]))]
+        rows[1]["rate_over_staged"] = rows[1]["learning_steps_per_s"] / rows[0]["learning_steps_per_s"]
+        rows[1]["mean_share_of_envs_per_start_stage"] = [round(sum(x[s] for x in starts) / len(starts), 4)
+                                                         for s in range(len(starts[0]))]
+        rows[1]["pool_entries_nonzero"] = int((learners["carousel"].stage_pool != 0).sum())
+        for row in rows:
+            print(json.dumps(row), file=sys.stderr, flush=True)
+        out += rows
+        del learners, runs
+        torch.cuda.empty_cache()
+    return out
+
+
+def _train_sampled(lr, total, block, shares):
+    """_train, appending the share of envs in stage 1 of (13,) after every block to `shares`; also returns the shaped
+    episodes and env-steps of a carousel learner."""
+    curve, wall, shaped = [], 0.0, [0, 0]
+    for _ in range(total // block):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        s = lr.train(block)
+        torch.cuda.synchronize()
+        wall += time.perf_counter() - t0
+        curve.append(round(s["score_sum"] / max(s["episodes"], 1), 1))
+        shares.append(_stage_shares(lr.boards, (13,))[1])
+        shaped[0] += s.get("shaped_episodes", 0)
+        shaped[1] += s.get("shaped_env_steps", 0)
+    return curve, wall, shaped
+
+
+CAROUSEL_RUNS = ("unstaged", "staged_t13", "staged_t13_carousel", "half_unstaged_then_staged_t13_carousel")
+
+
+def carousel_quality(short: int, long: int, block: int, B: int, deep: int, runs=CAROUSEL_RUNS) -> list:
+    """TC(lambda = 0.5, h = 3) at alpha 0.02 from the zero 4x6 network at n = 2^16 (seed 0): unstaged, staged (13,),
+    staged (13,) with the carousel, and short / 2 steps unstaged then staged((13,)) with the carousel; each evaluated
+    after `short` steps and, continuing, after `long`."""
+    n, lam, h, alpha = 1 << 16, 0.5, 3, g2048.td.DEFAULT_NTUPLE_TC_ALPHA
+    out = []
+    for name in runs:
+        net = NTupleNetwork.four_six()
+        if name.startswith("staged"):
+            net = NTupleNetwork.staged(net, (13,))
+        lr = g2048.NTupleTCLearner(0, n, network=net, alpha=alpha, lam=lam, horizon=h,
+                                   carousel=name == "staged_t13_carousel")
+        row = {"run": name, "learner": "tc", "lam": lam, "horizon": h, "alpha": alpha, "n": n, "block": block}
+        shares, curve, wall, shaped, done = [], [], 0.0, [0, 0], 0
+        for upto in (short, long):
+            if name.startswith("half") and done == 0:
+                c, w, _ = _train_sampled(lr, short // 2, block, shares)
+                curve, wall, done = curve + c, wall + w, short // 2
+                promoted = _promoted(lr, (13,), carousel=True)
+                del lr
+                torch.cuda.empty_cache()
+                lr = promoted
+            c, w, sh = _train_sampled(lr, upto - done, block, shares)
+            curve, wall, done = curve + c, wall + w, upto
+            shaped = [shaped[0] + sh[0], shaped[1] + sh[1]]
+            stage1 = None
+            if lr.network.n_stages > 1:
+                stage1 = int((lr.abs_err_sum[lr.network.stage_stride:] > 0).sum())
+            row[f"steps{upto}"] = {"train_seconds": round(wall, 2), **_players(lr.network, B, deep),
+                                   "share_of_env_steps_in_stage1_of_t13": round(sum(shares) / len(shares), 4),
+                                   "stage1_entries_updated": stage1, "shaped_episodes": shaped[0],
+                                   "shaped_env_steps": shaped[1]}
+            print(json.dumps(row), file=sys.stderr, flush=True)
+        row["curve_mean_score"] = curve
+        out.append(row)
+        del lr
+        torch.cuda.empty_cache()
+    return out
+
+
+def main_carousel(args) -> None:
+    result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
+    if not args.skip_speed:
+        result["speed_mechanism"] = carousel_speed(args.steps, args.carousel_pretrain_steps, (14,))
+        result["speed_mix"] = carousel_speed(args.steps, args.pretrain_steps, (13,))
+    if not args.speed_only:
+        result["quality"] = carousel_quality(args.sweep_steps, args.long_steps, args.block, args.games, args.deep_games,
+                                             args.carousel_runs.split(","))
+    _emit(result, args.out)
+
+
 def main_tc(args) -> None:
     result = {"gpu": gpu_info(), "l2": "warm for learning (the touched weights stay resident)"}
     if not args.skip_speed:
@@ -640,8 +786,13 @@ def main():
     ap.add_argument("--stages", action="store_true", help="multi-stage networks against the unstaged one (see above)")
     ap.add_argument("--lambda", dest="lam", action="store_true",
                     help="delayed TD(lambda) / TC(lambda) against TD(0) and TC (see above)")
+    ap.add_argument("--carousel", action="store_true", help="carousel shaping of staged networks (see above)")
     ap.add_argument("--pretrain-steps", type=int, default=20000,
-                    help="untimed training before the --stages and --lambda speed runs")
+                    help="untimed training before the --stages, --lambda and --carousel (real mix) speed runs")
+    ap.add_argument("--carousel-runs", default=",".join(CAROUSEL_RUNS),
+                    help="comma-separated quality runs of --carousel (default: all four)")
+    ap.add_argument("--carousel-pretrain-steps", type=int, default=2000,
+                    help="untimed training before the --carousel speed run of the mechanism")
     ap.add_argument("--long-steps", type=int, default=40000,
                     help="the longer equal-steps comparison of --tc, and the runs of --stages")
     ap.add_argument("--phase-probe", action="store_true", help=argparse.SUPPRESS)
@@ -653,6 +804,9 @@ def main():
         return
     if args.lam:
         main_lambda(args)
+        return
+    if args.carousel:
+        main_carousel(args)
         return
     if args.tc:
         main_tc(args)
